@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ICM-scored Gbp/s of the B200 hot path, next to the CPU reference.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 Default workload ``reads100`` = BASELINE.json configs[4], the sharded read set north_star's scaling target names
 (SURVEY.md section 8(d) config 5): 16 synthetic genomes (GC 0.30..0.70) with their own ICMs trained on the device,
@@ -67,7 +67,74 @@ def parse_args():
     ap.add_argument("--scale", type=float, default=1.0,
                     help="shrink a non-default workload (fraction of its reads / training strings); 1.0 = BASELINE size")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="b200 arm only: after the timed steps, write what the last timed step of the workload computed "
+                         "(rank 0) as DIR/<name>.npy, float32 / float64, at most 64 MB in all, so that two builds can be "
+                         "compared")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm; the reference arm keeps none")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+DUMP_SEED = 20261020
+
+
+def dump_outputs(dirname, arrays):
+    """{name: array} -> dirname/<name>.npy; float32 stays float32, everything else is widened to float64 (exact for the
+    int16 / int32 / int64 fields written here)."""
+    import numpy as np
+    arrays = {name: np.ascontiguousarray(a) for name, a in arrays.items()}
+    arrays = {name: a if a.dtype == np.float32 else a.astype(np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:  # the whole-call tables are not sampled: only a workload far beyond BASELINE size gets here
+        raise SystemExit(f"bench.py: --dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte limit")
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
+def seeded_sample(n, fits):
+    """Indices of a fixed, seeded sample of n items: all of them if fits(all), else the first half, quarter, ... of one
+    seeded permutation until fits(sample), down to none -- the same sample on every run with the same n."""
+    import numpy as np
+    idx = np.arange(n)
+    if fits(idx):
+        return idx
+    perm = np.random.default_rng(DUMP_SEED).permutation(n)
+    m = n // 2
+    while m > 0 and not fits(np.sort(perm[:m])):
+        m //= 2
+    return np.sort(perm[:m])
+
+
+def scoring_outputs(orfs, ooff, starts, soff):
+    """What a caller of the scoring half receives (ORF table + per-ORF start lists) as float64 tables: every ORF and
+    start when they fit DUMP_BYTES, else a seeded sample of ORFs with their complete start lists.
+      counts        [sequences, ORFs, starts] of the whole call
+      orf_counts    ORFs per sequence; start_counts  starts per ORF (whole call)
+      orfs          sampled ORFs: index, sequence, frame, stop_position, orf_len, gene_len
+      starts        their starts: ORF index, j, pos, score, which, truncated, first, n_err, err_pos[2], err_type[2]"""
+    import numpy as np
+    ooff, soff = np.asarray(ooff, np.int64), np.asarray(soff, np.int64)
+    n_orfs = len(orfs)
+    per_orf = np.diff(soff)
+    fixed = 8 * (3 + len(ooff) - 1 + n_orfs)
+    pick = seeded_sample(n_orfs, lambda ids: fixed + 8 * (6 * len(ids) + 12 * int(per_orf[ids].sum())) <= DUMP_BYTES)
+    seq = np.searchsorted(ooff, pick, side="right") - 1
+    o = orfs[pick]
+    orf_tab = np.stack([pick, seq, o["frame"], o["stop_position"], o["orf_len"], o["gene_len"]], axis=1).astype(np.float64)
+    lens = per_orf[pick]
+    owner = np.repeat(pick, lens)
+    rows = np.repeat(soff[pick], lens) + np.arange(int(lens.sum())) - np.repeat(np.cumsum(lens) - lens, lens)
+    s = starts[rows]
+    start_tab = np.column_stack([owner, s["j"], s["pos"], s["score"], s["which"], s["truncated"], s["first"], s["n_err"],
+                                 s["err_pos"], s["err_type"]]).astype(np.float64)
+    return {"counts": np.array([len(ooff) - 1, n_orfs, len(starts)], np.float64), "orf_counts": np.diff(ooff),
+            "start_counts": per_orf, "orfs": orf_tab, "starts": start_tab}
 
 
 def measured_peak():
@@ -421,6 +488,8 @@ def run_b200(args, env):
         k1_ms, k1_n = ctx.profile_read("k1")
         k3_ms, k3_n = ctx.profile_read("k3")
         clk = clocks.stop(t_wall0, t_wall1) if clocks else None
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, scoring_outputs(*ss.get_orfs(), *ss.get_starts()))
 
         # ---- end to end: host ASCII in, ORFs + start lists out ----
         e2e_ms = 0.0
@@ -733,6 +802,9 @@ def run_b200_reads(args, env, kind):
         kms = {k: ctx.profile_read(k) for k in ("k1", "k2", "k3")}
         clk = clocks.stop(t_wall0, t_wall1) if clocks else None
         n_orfs_last, uncert = sets[(Wu + K - 1) % nb].n_orfs, sets[(Wu + K - 1) % nb].uncertified
+        if rank == 0 and args.dump_outputs:
+            last = sets[(Wu + K - 1) % nb]
+            dump_outputs(args.dump_outputs, scoring_outputs(*last.get_orfs(), *last.get_starts()))
 
         # ---- end to end: pinned host ASCII in, ORF table + start lists out (pinned) ----
         for s in sets:
@@ -1086,6 +1158,9 @@ def run_b200_train(args, env):
         ms = sum(x.elapsed_time(y) for x, y in zip(e0, e1))
         k4_ms, k4_n = ctx.profile_read("k4")
         clk = clocks.stop(t_wall0, t_wall1) if clocks else None
+        if rank == 0 and args.dump_outputs:
+            mip, prob = model.tables()
+            dump_outputs(args.dump_outputs, {"model_mip": mip.astype(np.float32), "model_prob": prob})
         ss.close()
         # ---- end to end: pinned host strings in, model tables out ----
         e2e_ms, d2h = 0.0, 0
@@ -1209,18 +1284,22 @@ def simple_desc(n_reads):
 
 
 def _simple_ref_worker(job):
-    """One reference process: Score_String (the unmodified ICM library through oracle/_ref's ctypes shim) of a slice
-    of reads under every model; returns seconds."""
-    model_paths, seqs = job
+    """One reference process: Score_String (the unmodified ICM library through oracle/_ref's ctypes shim, or the oracle
+    port where oracle/_ref is absent) of a slice of reads under every model; returns seconds."""
+    model_paths, seqs, use_ref = job
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import oracle_lib as O
-    R = O.ref()
-    hs = [R.ref_icm_read(p.encode()) for p in model_paths]
+    if use_ref:
+        R = O.ref()
+        read, score = R.ref_icm_read, R.ref_score_string
+    else:
+        read, score = O.lib().orc_icm_read, O.lib().orc_score_string
+    hs = [read(p.encode()) for p in model_paths]
     t0 = time.perf_counter()
     acc = 0.0
     for h in hs:
         for s in seqs:
-            acc += R.ref_score_string(h, s, len(s), 0)
+            acc += score(h, s, len(s), 0)
     return time.perf_counter() - t0
 
 
@@ -1237,24 +1316,31 @@ def run_reference_simple(args):
     tmp = tempfile.mkdtemp(prefix="gmg_ref_")
     try:
         exe = ref_bin("build-icm")
-        if exe is None or not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "lib", "libref_icm.so")):
-            print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref (reference build) missing"}), flush=True)
-            return
+        have = exe is not None and os.path.exists(os.path.join(ROOT, "oracle", "_ref", "lib", "libref_icm.so"))
+        if not have:
+            cores = 1
+            sys.path.insert(0, os.path.join(ROOT, "tests"))
+            import oracle_lib as O
         paths = []
-        for k in range(SIMPLE_MODELS):  # the reference's own build-icm trains the models (not timed)
+        for k in range(SIMPLE_MODELS):  # the reference's own build-icm (or the oracle port) trains the models (not timed)
             ts, toff = simple_training(k)
-            fa = os.path.join(tmp, f"train{k}.fa")
-            W.write_fasta(fa, ts, toff, prefix="g")
             mp = os.path.join(tmp, f"m{k}.icm")
-            with open(fa, "rb") as fin:
-                subprocess.run([exe, "-d", "7", "-w", "12", "-p", "1", mp], stdin=fin, check=True,
-                               stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            if have:
+                fa = os.path.join(tmp, f"train{k}.fa")
+                W.write_fasta(fa, ts, toff, prefix="g")
+                with open(fa, "rb") as fin:
+                    subprocess.run([exe, "-d", "7", "-w", "12", "-p", "1", mp], stdin=fin, check=True,
+                                   stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            else:
+                raw_t = ts.tobytes()
+                strs = O.cstr_array([raw_t[toff[i]:toff[i + 1]] for i in range(len(toff) - 1)])
+                O.lib().orc_icm_write(O.lib().orc_icm_train(strs, len(toff) - 1, 12, 7, 1), mp.encode())
             paths.append(mp)
         raw = a.tobytes()
         jobs = []
         for i in range(cores):
             lo = (i * n_sample) % max(1, n_avail - n_sample + 1)
-            jobs.append((paths, [raw[off[j]:off[j + 1]] for j in range(lo, lo + n_sample)]))
+            jobs.append((paths, [raw[off[j]:off[j + 1]] for j in range(lo, lo + n_sample)], have))
         times = []
         with ProcessPoolExecutor(max_workers=cores) as ex:
             for k in range(args.warmup + args.steps):
@@ -1268,9 +1354,11 @@ def run_reference_simple(args):
                 "warmup": args.warmup, "ms_per_step": 1e3 * sum(times) / len(times), "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic", "impl": "reference",
                 "config": {"workload": simple_desc(n_avail)},
-                "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "reference",
+                "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "reference" if have else "port",
                                  "sample": f"each step: {cores} processes, each ICM_t::Score_String of its own {n_sample} reads "
-                                           f"under all {SIMPLE_MODELS} models (the unmodified ICM library through a ctypes shim)"},
+                                           f"under all {SIMPLE_MODELS} models (" +
+                                           ("the unmodified ICM library through a ctypes shim)" if have else
+                                            "the oracle port, models trained by its Train_Model)")},
                 "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "gpu_launches": 0}
         print(json.dumps(line), flush=True)
     finally:
@@ -1321,6 +1409,9 @@ def run_b200_simple(args, env):
         ms = sum(x.elapsed_time(y) for x, y in zip(e0, e1))
         k_ms, k_n = ctx.profile_read("fs")
         clk = clocks.stop(t_wall0, t_wall1) if clocks else None
+        if rank == 0 and args.dump_outputs:  # reads (columns) sampled only when the matrix exceeds DUMP_BYTES
+            cols = seeded_sample(out.shape[1], lambda ids: out.shape[0] * len(ids) * 8 <= DUMP_BYTES)
+            dump_outputs(args.dump_outputs, {"scores": out[:, cols], "score_reads": cols})
         ss.close()
         e2e_ms = 0.0
         for k in range(Wu + K):
@@ -1429,6 +1520,7 @@ def main():
                 sub.workload = wl
                 sub.steps = min(args.steps, steps)
                 sub.warmup = min(max(args.warmup, 3), 5)
+                sub.dump_outputs = None  # the dump holds the headline workload's outputs only
                 sub_line = runners[wl](sub, env)
                 if sub_line is not None:
                     extra[wl] = sub_line
