@@ -234,6 +234,15 @@ class ICM_Training_t : public ICM_t {
   // the same with the options the device path adds: reverse on the device instead of on the host, and an
   // all-reduce callback summing each level's count slab across the GPUs of a box (include/gmg_icm.h)
   void Train_Strings(const std::vector<char*>& data, int reverse, gmg_allreduce_fn allreduce, void* user) {
+    gmg_seqset* ss = Seqset_Of(data);
+    gmg_icm* h = NULL;
+    GMG_OR_DIE(gmg_icm_train(Gmg_Context(), ss, model_len, model_depth, periodicity, reverse, allreduce, user, &h));
+    gmg_seqset_free(ss);
+    Adopt(h);
+  }
+
+  // the training strings as a device seqset
+  static gmg_seqset* Seqset_Of(const std::vector<char*>& data) {
     std::vector<int64_t> off(data.size() + 1, 0);
     for (size_t i = 0; i < data.size(); i++) off[i + 1] = off[i] + (int64_t)strlen(data[i]);
     char* cat = NULL;
@@ -241,11 +250,18 @@ class ICM_Training_t : public ICM_t {
     for (size_t i = 0; i < data.size(); i++) memcpy(cat + off[i], data[i], (size_t)(off[i + 1] - off[i]));
     gmg_seqset* ss = NULL;
     GMG_OR_DIE(gmg_seqset_create(Gmg_Context(), cat, off.data(), (int64_t)data.size(), NULL, &ss));
-    gmg_icm* h = NULL;
-    GMG_OR_DIE(gmg_icm_train(Gmg_Context(), ss, model_len, model_depth, periodicity, reverse, allreduce, user, &h));
-    gmg_seqset_free(ss);
+    GMG_OR_DIE(gmg_ctx_sync(Gmg_Context()));  // the upload has read `cat`
     gmg_host_free(cat);
-    Adopt(h);
+    return ss;
+  }
+
+  // Train_Model for many training sets in one device pass (gmg_icm_train_many): models[k] gets the model of sets[k];
+  // every model takes this object's shape
+  void Train_Many(const std::vector<gmg_seqset*>& sets, int reverse, const std::vector<ICM_Training_t*>& models) {
+    std::vector<gmg_icm*> h(sets.size(), NULL);
+    GMG_OR_DIE(gmg_icm_train_many(Gmg_Context(), sets.data(), (int)sets.size(), model_len, model_depth, periodicity, reverse,
+                                  h.data()));
+    for (size_t k = 0; k < sets.size(); k++) models[k]->Adopt(h[k]);
   }
 
   // Train straight from a multi-FASTA image (parsed, lower-cased and packed on the device -- no per-character

@@ -128,6 +128,7 @@ def lib():
         "gmg_icm_train": (i32, [vp, vp, i32, i32, i32, i32, ALLREDUCE_FN, vp, P(vp)]),
         "gmg_icm_train_sharded": (i32, [vp, vp, i32, i32, i32, i32, ALLREDUCE_FN, vp, i32, i32, i64, P(vp)]),
         "gmg_trainer_set_shard": (i32, [vp, i32, i32, i64, ALLREDUCE_FN, vp]),
+        "gmg_icm_train_many": (i32, [vp, P(vp), i32, i32, i32, i32, i32, P(vp)]),
         "gmg_ctx_train_flagged": (i64, [vp]),
     }
     for name, (res, args) in sig.items():
@@ -659,6 +660,17 @@ class ICMTraining:
                                            rank, world, global_bases, C.byref(h)))
         self.flagged_nodes = int(lib().gmg_ctx_train_flagged(self.ctx.h))
         return ICM(self.ctx, h)
+
+    def Train_Models(self, sets, reverse=False):
+        """Train_Model for many training sets in one call (gmg_icm_train_many): element k of the result is the model of
+        ``sets[k]`` (a SeqSet or a list of strings, as Train_Model takes), byte-identical to Train_Model on it alone.
+        ``flagged_nodes`` is summed over the batch."""
+        ss = [s if isinstance(s, SeqSet) else SeqSet(self.ctx, seqs=s) for s in sets]
+        arr = (C.c_void_p * len(ss))(*[s.h for s in ss])
+        hs = (C.c_void_p * len(ss))()
+        _check(lib().gmg_icm_train_many(self.ctx.h, arr, len(ss), self.w, self.d, self.p, 1 if reverse else 0, hs))
+        self.flagged_nodes = int(lib().gmg_ctx_train_flagged(self.ctx.h))
+        return [ICM(self.ctx, C.c_void_p(h)) for h in hs]
 
     # split form, for callers that want to drive the levels themselves
     def levels(self, data, reverse=False):

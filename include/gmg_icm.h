@@ -298,6 +298,11 @@ int gmg_icm_train(gmg_ctx* ctx, gmg_seqset* s, int w, int d, int p, int reverse,
  * every level's count slab across the ranks; every rank returns the identical model */
 int gmg_icm_train_sharded(gmg_ctx* ctx, gmg_seqset* s, int w, int d, int p, int reverse, gmg_allreduce_fn ar, void* user,
                           int rank, int world, int64_t global_bases, gmg_icm** out);
+/* Train_Model (icm.cc:1356) for n_models independent training sets in one call: out[k] is the model of sets[k], byte-identical
+ * (gmg_icm_write) to gmg_icm_train(ctx, sets[k], w, d, p, reverse, NULL, NULL, &m).  All models share (w, d, p, reverse).
+ * gmg_ctx_train_flagged afterwards returns the number of flagged nodes summed over the batch.  A set may appear more than
+ * once.  On failure no out[k] is left allocated (all are NULL). */
+int gmg_icm_train_many(gmg_ctx* ctx, gmg_seqset* const* sets, int n_models, int w, int d, int p, int reverse, gmg_icm** out);
 /* Position choice and interpolation of a level run on the device; nodes whose choice lies within the error bound of the
  * device's logarithm are recomputed on the host with the reference's own libm.  This returns how many nodes of the
  * last gmg_icm_train* call on the context took that path (diagnostic). */
