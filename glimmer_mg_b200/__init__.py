@@ -6,7 +6,7 @@ package is the thin Python mirror of the reference's operator surface (``ICM_t``
 library.  There is no CPU fallback: importing works without a GPU, creating a :class:`Context` does not.
 """
 from .icm import (Context, EventModel, ICM, ICMTraining, Params, SeqSet, GmgError, ORF_DTYPE, START_DTYPE, lib, lib_path,
-                  build_indep_wo_stops, parse_quality_fasta, score_strings_many)
+                  build_indep_wo_stops, parse_quality_fasta, regions_from_coords, score_strings_many)
 
 __all__ = ["Context", "EventModel", "ICM", "ICMTraining", "Params", "SeqSet", "GmgError", "ORF_DTYPE", "START_DTYPE", "lib",
-           "lib_path", "build_indep_wo_stops", "parse_quality_fasta", "score_strings_many"]
+           "lib_path", "build_indep_wo_stops", "parse_quality_fasta", "regions_from_coords", "score_strings_many"]

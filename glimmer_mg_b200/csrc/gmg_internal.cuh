@@ -139,7 +139,12 @@ struct gmg_seqset {
   uint64_t* d_words;         // 2-bit bases, base i at bits 2*(i%32) of word i/32
   int32_t* d_blk2seq;        // sequence holding base 32*b; bit 31 = interior block (see k_blk2seq)
   uint8_t* d_qual;           // per-base quality (input file values) or NULL
-  unsigned long long* d_gc;  // {gc count, ORFs of the last g3 scoring call that took the ordered-sum fallback}
+  unsigned long long* d_gc;  // {gc count, ORFs of the last g3 scoring call that took the ordered-sum fallback,
+                             //  4 x bases per code (k_bucket_finish), non-acgt bytes counted by the pack}
+  // every input byte that is not a / c / g / t in either case, position-sorted: (base index << 8) | tolower(byte).
+  // The 2-bit pack keeps only Filter(byte); extraction needs the raw IUPAC code to complement it before Filter.
+  uint64_t* d_nacgt;
+  int64_t n_nacgt;
   // base buckets (k_bucket_*): the K1 planes are stored bucketed by the base at each position (see gmg_plane_index)
   uint32_t* d_bktidx;        // [nblk][4] plane index of the first base-b position at or after 32-base block blk
   // walk-ready contexts in plane-index order (model independent; K1 shifts them down by 32 - 2 W, W <= 14):
@@ -243,4 +248,5 @@ __device__ __forceinline__ uint64_t gmg_reverse_bases(uint64_t v, int W) {
 
 int gmg_seqset_ensure_buckets(gmg_ctx* ctx, gmg_seqset* s);
 // kernel launchers implemented across the .cu files
-int gmg_launch_pack(gmg_ctx* ctx, const uint8_t* d_ascii, int64_t total, uint64_t* d_words, unsigned long long* d_gc);
+int gmg_launch_pack(gmg_ctx* ctx, const uint8_t* d_ascii, int64_t total, uint64_t* d_words, unsigned long long* d_gc,
+                    uint64_t* d_nacgt, int64_t cap_nacgt);

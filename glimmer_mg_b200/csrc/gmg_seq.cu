@@ -8,6 +8,7 @@
 #include <limits.h>
 #include <string.h>
 
+#include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
 #include "gmg_internal.cuh"
@@ -22,15 +23,36 @@ __device__ __forceinline__ unsigned filter_code(unsigned ch) {
   }
 }
 
+__device__ __forceinline__ bool is_acgt(unsigned ch) {
+  const unsigned c = ch | 0x20u;
+  return c == 'a' || c == 'c' || c == 'g' || c == 't';
+}
+
+// g + c among the 32 bases of a packed word (codes 1 and 2: exactly one of the two bits set; zero padding is 'a')
+__device__ __forceinline__ unsigned word_gc(uint64_t v) {
+  return (unsigned)__popcll((v ^ (v >> 1)) & 0x5555555555555555ull);
+}
+
+// sum of every thread's count into *gc: one atomic per warp; every thread of the warp must call it
+__device__ __forceinline__ void warp_add_gc(unsigned my_gc, unsigned long long* gc) {
+  for (int o = 16; o > 0; o >>= 1) my_gc += __shfl_down_sync(0xffffffffu, my_gc, o);
+  if ((threadIdx.x & 31) == 0 && my_gc) atomicAdd(gc, (unsigned long long)my_gc);
+}
+
 // one thread packs 32 bases (32 ASCII bytes = two 16-byte loads) into one 64-bit word and
 // counts its g/c; a warp therefore reads 1 KB contiguous and writes 256 B contiguous.
+// Bytes other than a / c / g / t (bit b of `odd`) go to the non-acgt list: one ballot per warp finds out whether any
+// lane has one, so acgt-only input never reaches the atomic.  *n_nacgt counts every such byte, also those past `cap`
+// (the caller sees the overflow and packs again with room for all of them).  The list comes out unordered.
 __global__ void __launch_bounds__(256) k_pack(const uint8_t* __restrict__ ascii, int64_t total,
-                                              uint64_t* __restrict__ words, unsigned long long* __restrict__ gc) {
+                                              uint64_t* __restrict__ words, unsigned long long* __restrict__ gc,
+                                              uint64_t* __restrict__ nacgt, int64_t cap,
+                                              unsigned long long* __restrict__ n_nacgt) {
   int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   int64_t nwords = (total + 31) >> 5;
-  unsigned my_gc = 0;
+  unsigned my_gc = 0, odd = 0;
+  const int64_t base = w << 5;
   if (w < nwords) {
-    int64_t base = w << 5;
     uint64_t v = 0;
     if (base + 32 <= total && ((reinterpret_cast<uintptr_t>(ascii + base) & 15) == 0)) {
       const uint4* src = reinterpret_cast<const uint4*>(ascii + base);
@@ -42,23 +64,40 @@ __global__ void __launch_bounds__(256) k_pack(const uint8_t* __restrict__ ascii,
         for (int k = 0; k < 4; k++)
 #pragma unroll
           for (int b = 0; b < 4; b++) {
-            unsigned code = filter_code((r[k] >> (8 * b)) & 0xFF);
-            my_gc += (code == 1 || code == 2);
-            v |= (uint64_t)code << (2 * (h * 16 + k * 4 + b));
+            const unsigned ch = (r[k] >> (8 * b)) & 0xFF;
+            v |= (uint64_t)filter_code(ch) << (2 * (h * 16 + k * 4 + b));
+            odd |= (is_acgt(ch) ? 0u : 1u) << (h * 16 + k * 4 + b);
           }
       }
     } else {
       for (int b = 0; b < 32 && base + b < total; b++) {
-        unsigned code = filter_code(ascii[base + b]);
-        my_gc += (code == 1 || code == 2);
-        v |= (uint64_t)code << (2 * b);
+        const unsigned ch = ascii[base + b];
+        v |= (uint64_t)filter_code(ch) << (2 * b);
+        odd |= (is_acgt(ch) ? 0u : 1u) << b;
       }
     }
     words[w] = v;
+    my_gc = word_gc(v);
   }
-  // block reduction of the GC count -> one atomic per warp
-  for (int o = 16; o > 0; o >>= 1) my_gc += __shfl_down_sync(0xffffffffu, my_gc, o);
-  if ((threadIdx.x & 31) == 0 && my_gc) atomicAdd(gc, (unsigned long long)my_gc);
+  if (__ballot_sync(0xffffffffu, odd != 0)) {
+    const int lane = threadIdx.x & 31;
+    const unsigned cnt = (unsigned)__popc(odd);
+    unsigned incl = cnt;  // inclusive warp prefix of the counts
+    for (int o = 1; o < 32; o <<= 1) {
+      const unsigned t = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += t;
+    }
+    unsigned long long first = 0;
+    if (lane == 31) first = atomicAdd(n_nacgt, (unsigned long long)incl);
+    unsigned long long e = __shfl_sync(0xffffffffu, first, 31) + (incl - cnt);
+    for (; odd; odd &= odd - 1, e++) {
+      const int b = __ffs(odd) - 1;
+      unsigned ch = ascii[base + b];
+      if (ch >= 'A' && ch <= 'Z') ch += 32;
+      if (e < (unsigned long long)cap) nacgt[e] = ((uint64_t)(base + b) << 8) | ch;
+    }
+  }
+  warp_add_gc(my_gc, gc);
 }
 
 __global__ void k_unpack(const uint64_t* __restrict__ words, int64_t total, char* __restrict__ out) {
@@ -227,22 +266,26 @@ int gmg_seqset_ensure_buckets(gmg_ctx* ctx, gmg_seqset* s) {
   return 0;
 }
 
-int gmg_launch_pack(gmg_ctx* ctx, const uint8_t* d_ascii, int64_t total, uint64_t* d_words, unsigned long long* d_gc) {
+// d_gc[6] counts the non-acgt bytes (d_nacgt holds the first cap_nacgt of them)
+int gmg_launch_pack(gmg_ctx* ctx, const uint8_t* d_ascii, int64_t total, uint64_t* d_words, unsigned long long* d_gc,
+                    uint64_t* d_nacgt, int64_t cap_nacgt) {
   int64_t nwords = (total + 31) >> 5;
   if (nwords == 0) return 0;
   if (gmg_prof_begin(ctx, GMG_PROF_PACK)) return 1;
-  k_pack<<<(unsigned)((nwords + 255) / 256), 256, 0, ctx->stream>>>(d_ascii, total, d_words, d_gc);
+  k_pack<<<(unsigned)((nwords + 255) / 256), 256, 0, ctx->stream>>>(d_ascii, total, d_words, d_gc, d_nacgt, cap_nacgt,
+                                                                    d_gc + 6);
   gmg_prof_end(ctx, GMG_PROF_PACK);
   ctx->launches++;
   GMG_CUDA(cudaGetLastError());
   return 0;
 }
 
+// An empty set of n sequences with offsets h_off: device offsets, zeroed words and counters, blk2seq.  The creation routes
+// pack bases into it, gmg_seqset_extract copies them from another set.
 // copy_off_from_caller: the device copy of the offsets is made straight from h_off (gmg_seqset_create synchronises before
 // it returns, so a page-locked caller buffer travels at PCIe rate and without the driver's staging copy); otherwise from
 // the set's own host copy.
-static int seqset_build(gmg_ctx* ctx, const void* d_ascii, const int64_t* h_off, int64_t n, const void* d_qual,
-                        gmg_seqset** out, bool copy_off_from_caller = false) {
+static int seqset_alloc(gmg_ctx* ctx, const int64_t* h_off, int64_t n, gmg_seqset** out, bool copy_off_from_caller) {
   GMG_CHECK(n >= 0 && n < (1ll << 31), "gmg_seqset_create: %lld sequences unsupported", (long long)n);
   int64_t max_len = 0;
   for (int64_t i = 0; i < n; i++) {
@@ -262,6 +305,7 @@ static int seqset_build(gmg_ctx* ctx, const void* d_ascii, const int64_t* h_off,
   s->n_orfs = 0; s->d_orfs = NULL; s->d_orf_off = NULL; s->d_orf_seq = NULL;
   s->n_starts = 0; s->d_starts = NULL; s->d_start_off = NULL; s->uncertified = 0;
   s->cap_orfs = s->cap_starts = 0;
+  s->d_nacgt = NULL; s->n_nacgt = 0;
   GMG_CUDA(cudaSetDevice(ctx->device));
   int64_t nwords = (s->total + 31) >> 5;
   int64_t nblk = nwords > 0 ? nwords : 1;
@@ -273,13 +317,35 @@ static int seqset_build(gmg_ctx* ctx, const void* d_ascii, const int64_t* h_off,
   GMG_CUDA(cudaMemcpyAsync(s->d_off, copy_off_from_caller && n > 0 ? h_off : s->off.data(), (size_t)(s->n + 1) * sizeof(int64_t),
                            cudaMemcpyHostToDevice, ctx->stream));
   GMG_CUDA(cudaMallocAsync(&s->d_blk2seq, (size_t)nblk * sizeof(int32_t), s->ctx->stream));
-  GMG_CUDA(cudaMallocAsync(&s->d_gc, 6 * sizeof(unsigned long long), s->ctx->stream));
-  GMG_CUDA(cudaMemsetAsync(s->d_gc, 0, 6 * sizeof(unsigned long long), ctx->stream));
+  GMG_CUDA(cudaMallocAsync(&s->d_gc, 7 * sizeof(unsigned long long), s->ctx->stream));
+  GMG_CUDA(cudaMemsetAsync(s->d_gc, 0, 7 * sizeof(unsigned long long), ctx->stream));
   if (s->total > 0) {
-    if (gmg_launch_pack(ctx, (const uint8_t*)d_ascii, s->total, s->d_words, s->d_gc)) return 1;
     k_blk2seq<<<(unsigned)((nblk + 255) / 256), 256, 0, ctx->stream>>>(s->d_off, s->n, nblk, s->d_blk2seq);
     ctx->launches++;
     GMG_CUDA(cudaGetLastError());
+  }
+  *out = s;
+  return 0;
+}
+
+// room for the pack's first pass at the non-acgt list (context scratch SCR_MISC): assembled genomes hold a few such bytes
+// per Mbp; input with more packs a second time at the exact size (seqset_finish_nacgt)
+static int64_t nacgt_cap(int64_t total) { return 4096 + total / 1024; }
+
+// Pack the ASCII at d_ascii into a new set.  The count of non-acgt bytes is on its way to ctx->h_scalars[15]: synchronise
+// the stream, then call seqset_finish_nacgt while d_ascii is still intact.
+static int seqset_build(gmg_ctx* ctx, const void* d_ascii, const int64_t* h_off, int64_t n, const void* d_qual,
+                        gmg_seqset** out, bool copy_off_from_caller = false) {
+  gmg_seqset* s;
+  if (seqset_alloc(ctx, h_off, n, &s, copy_off_from_caller)) return 1;
+  ctx->h_scalars[15] = 0;
+  if (s->total > 0) {
+    void* d_list;
+    if (gmg_scratch(ctx, SCR_MISC, (size_t)nacgt_cap(s->total) * sizeof(uint64_t), &d_list)) return 1;
+    if (gmg_launch_pack(ctx, (const uint8_t*)d_ascii, s->total, s->d_words, s->d_gc, (uint64_t*)d_list,
+                        nacgt_cap(s->total)))
+      return 1;
+    GMG_CUDA(cudaMemcpyAsync(ctx->h_scalars + 15, s->d_gc + 6, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
     if (d_qual) {
       GMG_CUDA(cudaMallocAsync(&s->d_qual, (size_t)s->total, s->ctx->stream));
       GMG_CUDA(cudaMemcpyAsync(s->d_qual, d_qual, (size_t)s->total, cudaMemcpyDeviceToDevice, ctx->stream));
@@ -289,10 +355,39 @@ static int seqset_build(gmg_ctx* ctx, const void* d_ascii, const int64_t* h_off,
   return 0;
 }
 
+// Sorts the pack's non-acgt list into the set (after the stream synchronisation that brought its count to the host).
+// A list that overflowed the first pass is recorded again, at its exact size, from the same ASCII.
+static int seqset_finish_nacgt(gmg_ctx* ctx, gmg_seqset* s, const void* d_ascii) {
+  const int64_t cnt = ctx->h_scalars[15];
+  if (cnt == 0) return 0;
+  GMG_CHECK(cnt < (1ll << 31), "gmg_seqset_create: %lld bytes other than a, c, g, t -- split the batch", (long long)cnt);
+  void *d_list, *d_tmp;
+  if (gmg_scratch(ctx, SCR_MISC, (size_t)(cnt > nacgt_cap(s->total) ? cnt : nacgt_cap(s->total)) * sizeof(uint64_t), &d_list))
+    return 1;
+  if (cnt > nacgt_cap(s->total)) {
+    GMG_CUDA(cudaMemsetAsync(s->d_gc, 0, 7 * sizeof(unsigned long long), ctx->stream));
+    if (gmg_launch_pack(ctx, (const uint8_t*)d_ascii, s->total, s->d_words, s->d_gc, (uint64_t*)d_list, cnt)) return 1;
+  }
+  GMG_CUDA(cudaMallocAsync(&s->d_nacgt, (size_t)cnt * sizeof(uint64_t), ctx->stream));
+  int end_bit = 8;
+  while (end_bit < 64 && (s->total >> (end_bit - 8)) != 0) end_bit++;
+  size_t tmp_bytes = 0;
+  GMG_CUDA(cub::DeviceRadixSort::SortKeys(NULL, tmp_bytes, (const uint64_t*)d_list, s->d_nacgt, (int)cnt, 8, end_bit,
+                                          ctx->stream));
+  if (gmg_scratch(ctx, SCR_TMP4, tmp_bytes, &d_tmp)) return 1;
+  GMG_CUDA(cub::DeviceRadixSort::SortKeys(d_tmp, tmp_bytes, (const uint64_t*)d_list, s->d_nacgt, (int)cnt, 8, end_bit,
+                                          ctx->stream));
+  ctx->launches++;
+  s->n_nacgt = cnt;
+  return 0;
+}
+
 extern "C" int gmg_seqset_create_device(gmg_ctx* ctx, const void* d_ascii, const int64_t* h_off, int64_t n,
                                         const void* d_qual, gmg_seqset** out) {
   GMG_CHECK(ctx && h_off && out, "gmg_seqset_create_device: NULL argument");
-  return seqset_build(ctx, d_ascii, h_off, n, d_qual, out);
+  if (seqset_build(ctx, d_ascii, h_off, n, d_qual, out)) return 1;
+  GMG_CUDA(cudaStreamSynchronize(ctx->stream));
+  return seqset_finish_nacgt(ctx, *out, d_ascii);
 }
 
 extern "C" int gmg_seqset_create(gmg_ctx* ctx, const char* h_ascii, const int64_t* h_off, int64_t n,
@@ -311,9 +406,9 @@ extern "C" int gmg_seqset_create(gmg_ctx* ctx, const char* h_ascii, const int64_
       GMG_CUDA(cudaMemcpyAsync(d_q, h_qual, (size_t)total, cudaMemcpyHostToDevice, ctx->stream));
     }
   }
-  int rc = seqset_build(ctx, d_ascii, h_off, n, d_q, out, true);
-  if (rc == 0) GMG_CUDA(cudaStreamSynchronize(ctx->stream));  // host buffers may be reused by the caller
-  return rc;
+  if (seqset_build(ctx, d_ascii, h_off, n, d_q, out, true)) return 1;
+  GMG_CUDA(cudaStreamSynchronize(ctx->stream));  // host buffers may be reused by the caller
+  return seqset_finish_nacgt(ctx, *out, d_ascii);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -465,6 +560,7 @@ extern "C" int gmg_seqset_from_fasta(gmg_ctx* ctx, const char* h_bytes, int64_t 
   s->hdr_off.assign(h_tab.begin() + (n_rec ? n_rec : 0), h_tab.begin() + (n_rec ? 2 * n_rec : 0));
   s->hdr_end.assign(h_tab.begin() + (n_rec ? 2 * n_rec : 0), h_tab.end());
   GMG_CUDA(cudaStreamSynchronize(ctx->stream));  // d_out (scratch) has been consumed by the pack kernel
+  if (seqset_finish_nacgt(ctx, s, d_out)) return 1;
   *out = s;
   if (n_records) *n_records = n_rec;
   return 0;
@@ -661,7 +757,8 @@ extern "C" void gmg_seqset_free(gmg_seqset* s) {
   if (!s) return;
   cudaSetDevice(s->ctx->device);
   void* ptrs[] = {s->d_off, s->d_words_base, s->d_blk2seq, s->d_qual, s->d_gc, s->d_orfs, s->d_orf_off,
-                  s->d_orf_seq, s->d_starts, s->d_start_off, s->d_cbits, s->d_bktidx, s->d_ctxf, s->d_ctxr};
+                  s->d_orf_seq, s->d_starts, s->d_start_off, s->d_cbits, s->d_bktidx, s->d_ctxf, s->d_ctxr,
+                  s->d_nacgt};
   for (void* p : ptrs)
     if (p) cudaFreeAsync(p, s->ctx->stream);
   delete s;
@@ -690,5 +787,210 @@ extern "C" int gmg_seqset_unpack(gmg_seqset* s, char* h_out) {
   GMG_CUDA(cudaGetLastError());
   GMG_CUDA(cudaMemcpyAsync(h_out, d, (size_t)s->total, cudaMemcpyDeviceToHost, ctx->stream));
   GMG_CUDA(cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// extract (Util/extract.cc) on a resident set.  Output sequence r is region r: bases [from[r], from[r] + len_r) of the
+// source (global base indices), read upwards on strand +1; on strand -1 read downwards and complemented.  The reference
+// complements the raw IUPAC code (Complement, Common/delcher.cc) and build-icm applies Filter afterwards; the 2-bit
+// complement 3 - code equals that for a / c / g / t only, so the positions of the source's non-acgt list that fall into
+// minus regions are patched with Filter(Complement(raw)).
+
+// Complement of a lower-case IUPAC code; every other byte becomes 'n', so the complement of a non-acgt byte is again
+// non-acgt and the output list has one entry per source entry inside a region.
+__device__ __forceinline__ unsigned iupac_complement(unsigned ch) {
+  switch (ch) {
+    case 'a': return 't';
+    case 'c': return 'g';
+    case 'g': return 'c';
+    case 't': return 'a';
+    case 'r': return 'y';
+    case 'y': return 'r';
+    case 'm': return 'k';
+    case 'k': return 'm';
+    case 'b': return 'v';
+    case 'v': return 'b';
+    case 'd': return 'h';
+    case 'h': return 'd';
+    case 's': return 's';
+    case 'w': return 'w';
+    default: return 'n';
+  }
+}
+
+// first index of the (position-sorted) list whose position is >= p
+__device__ __forceinline__ int64_t nacgt_lower_bound(const uint64_t* __restrict__ list, int64_t n, int64_t p) {
+  int64_t lo = 0, hi = n;
+  const uint64_t key = (uint64_t)p << 8;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (__ldg(list + mid) < key) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo;
+}
+
+// largest r < n with key[r] <= x (key ascending, key[0] <= x): the region of an output position (off) or of an output
+// list entry (list_base).  Empty regions share their key with the next one, so the search lands on a non-empty one.
+__device__ __forceinline__ int64_t last_at_or_below(const int64_t* __restrict__ key, int64_t n, int64_t x) {
+  int64_t lo = 0, hi = n;
+  while (hi - lo > 1) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (__ldg(key + mid) <= x) lo = mid;
+    else hi = mid;
+  }
+  return lo;
+}
+
+// per region: the source list entries inside it, [first[r], first[r] + cnt[r])
+__global__ void __launch_bounds__(256) k_extract_count(const uint64_t* __restrict__ list, int64_t n_list,
+                                                       const int64_t* __restrict__ off, const int64_t* __restrict__ from,
+                                                       int64_t n, int64_t* __restrict__ first, int64_t* __restrict__ cnt) {
+  const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  const int64_t a = nacgt_lower_bound(list, n_list, from[r]);
+  const int64_t b = nacgt_lower_bound(list, n_list, from[r] + (off[r + 1] - off[r]));
+  first[r] = a;
+  cnt[r] = b - a;
+}
+
+// one thread per output word: each region piece inside the word is a two-word funnel shift of the source (plus, on
+// strand -1, base reversal, complement and the non-acgt patch); then the word's g + c count
+__global__ void __launch_bounds__(256) k_extract_words(const uint64_t* __restrict__ src, const uint64_t* __restrict__ list,
+                                                       int64_t n_list, const int64_t* __restrict__ off,
+                                                       const int64_t* __restrict__ from, const int8_t* __restrict__ strand,
+                                                       int64_t n, int64_t total, uint64_t* __restrict__ words,
+                                                       unsigned long long* __restrict__ gc) {
+  const int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  unsigned my_gc = 0;
+  if (w < ((total + 31) >> 5)) {
+    const int64_t w0 = w << 5, end = w0 + 32 < total ? w0 + 32 : total;
+    uint64_t v = 0;
+    for (int64_t p = w0; p < end;) {
+      const int64_t r = last_at_or_below(off, n, p);
+      const int64_t a = __ldg(off + r), e = __ldg(off + r + 1);
+      const int64_t q = e < end ? e : end;
+      const int m = (int)(q - p);
+      const int64_t k = p - a;  // offset of the piece in its region
+      uint64_t x;
+      if (__ldg(strand + r) > 0) {
+        x = gmg_extract32(src, __ldg(from + r) + k);
+      } else {
+        const int64_t s0 = __ldg(from + r) + (e - a) - k - m;  // lowest source base of the piece
+        x = ~gmg_reverse_bases(gmg_extract32(src, s0), m);  // 3 - code = code ^ 3
+        for (int64_t i = n_list ? nacgt_lower_bound(list, n_list, s0) : 0; i < n_list; i++) {
+          const uint64_t ent = __ldg(list + i);
+          const int64_t ps = (int64_t)(ent >> 8);
+          if (ps >= s0 + m) break;
+          const int j = (int)(s0 + m - 1 - ps);  // its place in the piece
+          x = (x & ~(3ull << (2 * j))) | ((uint64_t)filter_code(iupac_complement((unsigned)(ent & 0xFF))) << (2 * j));
+        }
+      }
+      if (m < 32) x &= (1ull << (2 * m)) - 1ull;
+      v |= x << (2 * (p - w0));
+      p = q;
+    }
+    words[w] = v;
+    my_gc = word_gc(v);
+  }
+  warp_add_gc(my_gc, gc);
+}
+
+// one thread per output list entry: its region (by the exclusive sum `base` of cnt), the source entry, the new position
+// and, on strand -1, the complemented code; regions are in output order and a minus region takes its entries in reverse,
+// so the output list is position-sorted
+__global__ void __launch_bounds__(256) k_extract_list(const uint64_t* __restrict__ list, const int64_t* __restrict__ off,
+                                                      const int64_t* __restrict__ from, const int8_t* __restrict__ strand,
+                                                      int64_t n, const int64_t* __restrict__ first,
+                                                      const int64_t* __restrict__ cnt, const int64_t* __restrict__ base,
+                                                      int64_t n_out, uint64_t* __restrict__ out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_out) return;
+  const int64_t r = last_at_or_below(base, n, i);
+  const int64_t k = i - base[r];
+  const int64_t a = off[r], len = off[r + 1] - a;
+  uint64_t ent;
+  int64_t pos;
+  unsigned ch;
+  if (strand[r] > 0) {
+    ent = list[first[r] + k];
+    pos = a + ((int64_t)(ent >> 8) - from[r]);
+    ch = (unsigned)(ent & 0xFF);
+  } else {
+    ent = list[first[r] + cnt[r] - 1 - k];
+    pos = a + (from[r] + len - 1 - (int64_t)(ent >> 8));
+    ch = iupac_complement((unsigned)(ent & 0xFF));
+  }
+  out[i] = ((uint64_t)pos << 8) | ch;
+}
+
+extern "C" int gmg_seqset_extract(gmg_ctx* ctx, gmg_seqset* src, int64_t n, const int32_t* h_seq, const int32_t* h_lo,
+                                  const int32_t* h_len, const int8_t* h_strand, gmg_seqset** out) {
+  GMG_CHECK(ctx && src && out && (n == 0 || (h_seq && h_lo && h_len && h_strand)), "gmg_seqset_extract: NULL argument");
+  GMG_CHECK(n >= 0 && n < (1ll << 31), "gmg_seqset_extract: %lld regions unsupported", (long long)n);
+  std::vector<int64_t> off((size_t)n + 1, 0), from((size_t)n);
+  for (int64_t i = 0; i < n; i++) {
+    GMG_CHECK(h_seq[i] >= 0 && h_seq[i] < src->n, "gmg_seqset_extract: region %lld: sequence %d out of range (the set "
+              "holds %lld)", (long long)i, h_seq[i], (long long)src->n);
+    const int64_t L = src->off[(size_t)h_seq[i] + 1] - src->off[(size_t)h_seq[i]];
+    GMG_CHECK(h_lo[i] >= 0, "gmg_seqset_extract: region %lld: start %d is negative", (long long)i, h_lo[i]);
+    GMG_CHECK(h_len[i] >= 0 && (int64_t)h_lo[i] + h_len[i] <= L, "gmg_seqset_extract: region %lld: [%d, %lld) is not "
+              "inside its %lld bp sequence %d", (long long)i, h_lo[i], (long long)h_lo[i] + h_len[i], (long long)L, h_seq[i]);
+    GMG_CHECK(h_strand[i] == 1 || h_strand[i] == -1, "gmg_seqset_extract: region %lld: strand %d is not +1 or -1",
+              (long long)i, (int)h_strand[i]);
+    off[(size_t)i + 1] = off[(size_t)i] + h_len[i];
+    from[(size_t)i] = src->off[(size_t)h_seq[i]] + h_lo[i];
+  }
+  GMG_CUDA(cudaSetDevice(ctx->device));
+  gmg_seqset* s;
+  if (seqset_alloc(ctx, off.data(), n, &s, false)) return 1;
+  if (s->total == 0) {
+    *out = s;
+    return 0;
+  }
+  // region table: from | first | cnt | base (int64 [n] each) | strand (int8 [n])
+  void* d_tab;
+  if (gmg_scratch(ctx, SCR_MISC, (size_t)n * (4 * sizeof(int64_t) + 1) + 64, &d_tab)) return 1;
+  int64_t* d_from = (int64_t*)d_tab;
+  int64_t* d_first = d_from + n;
+  int64_t* d_cnt = d_first + n;
+  int64_t* d_base = d_cnt + n;
+  int8_t* d_strand = (int8_t*)(d_base + n);
+  GMG_CUDA(cudaMemcpyAsync(d_from, from.data(), (size_t)n * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+  GMG_CUDA(cudaMemcpyAsync(d_strand, h_strand, (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+  const unsigned grid_r = (unsigned)((n + 255) / 256);
+  if (src->n_nacgt > 0) {
+    k_extract_count<<<grid_r, 256, 0, ctx->stream>>>(src->d_nacgt, src->n_nacgt, s->d_off, d_from, n, d_first, d_cnt);
+    size_t tmp_bytes = 0;
+    void* d_tmp;
+    GMG_CUDA(cub::DeviceScan::ExclusiveSum(NULL, tmp_bytes, d_cnt, d_base, n, ctx->stream));
+    if (gmg_scratch(ctx, SCR_TMP4, tmp_bytes, &d_tmp)) return 1;
+    GMG_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, d_cnt, d_base, n, ctx->stream));
+    ctx->launches += 2;
+    ctx->h_scalars[15] = ctx->h_scalars[14] = 0;
+    GMG_CUDA(cudaMemcpyAsync(ctx->h_scalars + 14, d_base + n - 1, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    GMG_CUDA(cudaMemcpyAsync(ctx->h_scalars + 15, d_cnt + n - 1, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  const int64_t nwords = (s->total + 31) >> 5;
+  k_extract_words<<<(unsigned)((nwords + 255) / 256), 256, 0, ctx->stream>>>(src->d_words, src->d_nacgt, src->n_nacgt,
+                                                                             s->d_off, d_from, d_strand, n, s->total,
+                                                                             s->d_words, s->d_gc);
+  ctx->launches++;
+  GMG_CUDA(cudaGetLastError());
+  GMG_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (src->n_nacgt > 0) {
+    const int64_t n_out = ctx->h_scalars[14] + ctx->h_scalars[15];
+    if (n_out > 0) {
+      GMG_CUDA(cudaMallocAsync(&s->d_nacgt, (size_t)n_out * sizeof(uint64_t), ctx->stream));
+      k_extract_list<<<(unsigned)((n_out + 255) / 256), 256, 0, ctx->stream>>>(src->d_nacgt, s->d_off, d_from, d_strand, n,
+                                                                               d_first, d_cnt, d_base, n_out, s->d_nacgt);
+      ctx->launches++;
+      GMG_CUDA(cudaGetLastError());
+      s->n_nacgt = n_out;
+      GMG_CUDA(cudaStreamSynchronize(ctx->stream));
+    }
+  }
+  *out = s;
   return 0;
 }

@@ -12,6 +12,7 @@ Errors: the reference prints to stderr and exits (icm.cc:635-657); here every fa
 """
 import ctypes as C
 import os
+import re
 
 import numpy as np
 
@@ -100,6 +101,7 @@ def lib():
         "gmg_seqset_total_bases": (i64, [vp]),
         "gmg_seqset_gc_fraction": (i32, [vp, P(C.c_double)]),
         "gmg_seqset_unpack": (i32, [vp, vp]),
+        "gmg_seqset_extract": (i32, [vp, vp, i64, vp, vp, vp, vp, P(vp)]),
         "gmg_icm_score_strings": (i32, [vp, vp, vp, i32, vp]),
         "gmg_icm_score_strings_many": (i32, [vp, P(vp), i32, vp, i32, vp]),
         "gmg_icm_cumulative_score": (i32, [vp, vp, vp, i32, vp]),
@@ -312,24 +314,44 @@ class SeqSet:
         The returned set has ``headers``: the header text of every record."""
         buf = np.frombuffer(image, np.uint8) if isinstance(image, (bytes, bytearray, memoryview)) else \
             np.ascontiguousarray(image, np.uint8)
-        self = cls.__new__(cls)
-        self.ctx = ctx
-        self.h = C.c_void_p()
-        n = C.c_int64()
-        _check(lib().gmg_seqset_from_fasta(ctx.h, buf.ctypes.data if len(buf) else None, len(buf), C.byref(self.h),
-                                           C.byref(n)))
-        self.n = n.value
-        self.off = np.zeros(self.n + 1, np.int64)
-        _check(lib().gmg_seqset_offsets(self.h, self.off.ctypes.data))
-        self.total = int(self.off[-1])
-        self.n_orfs = 0
-        self.n_starts = 0
+        h, n = C.c_void_p(), C.c_int64()
+        _check(lib().gmg_seqset_from_fasta(ctx.h, buf.ctypes.data if len(buf) else None, len(buf), C.byref(h), C.byref(n)))
+        self = cls._adopt(ctx, h)
         ho, he = np.zeros(self.n, np.int64), np.zeros(self.n, np.int64)
         if self.n:
             _check(lib().gmg_seqset_fasta_headers(self.h, ho.ctypes.data, he.ctypes.data))
         raw = buf.tobytes()
         self.headers = [raw[a:b].decode(errors="replace") for a, b in zip(ho.tolist(), he.tolist())]
         return self
+
+    @classmethod
+    def _adopt(cls, ctx, h):
+        """Wrap a set the library has just created."""
+        self = cls.__new__(cls)
+        self.ctx = ctx
+        self.h = h
+        self.n = int(lib().gmg_seqset_count(h))
+        self.off = np.zeros(self.n + 1, np.int64)
+        _check(lib().gmg_seqset_offsets(self.h, self.off.ctypes.data))
+        self.total = int(self.off[-1])
+        self.n_orfs = 0
+        self.n_starts = 0
+        return self
+
+    def extract(self, seq, lo, length, strand):
+        """extract (Glimmer's Util/extract.cc) on the device: region i, bases [lo[i], lo[i] + length[i]) of sequence
+        seq[i] (0-based), becomes sequence i of the returned set; strand[i] = -1 takes its reverse complement, with raw
+        IUPAC codes complemented before Filter as extract + build-icm do.  Regions must lie inside their sequence.  The
+        result has no qualities and no headers.  ``regions_from_coords`` turns coordinate files into these arrays."""
+        seq, lo, length = (np.ascontiguousarray(x, np.int32).reshape(-1) for x in (seq, lo, length))
+        strand = np.ascontiguousarray(strand, np.int8).reshape(-1)
+        if not len(seq) == len(lo) == len(length) == len(strand):
+            raise GmgError(f"extract: {len(seq)} sequences, {len(lo)} starts, {len(length)} lengths and {len(strand)} "
+                           "strands given")
+        h = C.c_void_p()
+        _check(lib().gmg_seqset_extract(self.ctx.h, self.h, len(seq), seq.ctypes.data, lo.ctypes.data, length.ctypes.data,
+                                        strand.ctypes.data, C.byref(h)))
+        return SeqSet._adopt(self.ctx, h)
 
     def set_quality_fasta(self, image):
         """Per-base qualities from the image of a quality file (Fasta_Qual_Vec_Read, Common/fasta.cc:115), parsed on the
@@ -611,6 +633,70 @@ def parse_quality_fasta(ctx, image):
     _check(lib().gmg_quality_parse_fasta(ctx.h, ptr, len(buf), C.byref(nr), C.byref(nv), off.ctypes.data, vals.ctypes.data,
                                          nr.value, nv.value))
     return off, vals
+
+
+_FRAME = re.compile(r"[+-][0-9]+")
+
+
+def regions_from_coords(lines, headers=None, trim_stop=True):
+    """Coordinate text -> (seq, lo, length, strand) arrays for ``SeqSet.extract``, as extract (Util/extract.cc) reads a
+    coordinate file.  A line is ``id start end ...``: 1-based inclusive positions, start > end for the minus strand.  That
+    covers long-orfs output, the headers of a ``.train`` file and the body of a ``.predict`` file.
+
+    ``headers`` (e.g. ``SeqSet.from_fasta(...).headers``): the ``>`` lines of a ``.predict`` file select the sequence of
+    the lines that follow, by whole header or by its first word.  Without it every region is on sequence 0 and a ``>``
+    line is an error.  ``trim_stop`` drops the last codon (the stop), as ``extract -t`` does.
+
+    A fourth field that is a signed frame (``+2``, ``-1``) must agree with the orientation; where it does not, the gene
+    wraps around the end of a circular sequence, which the device path does not support."""
+    if isinstance(lines, (str, bytes)):
+        lines = lines.splitlines()
+    index = None
+    if headers is not None:
+        index = {}
+        for i, h in enumerate(headers):
+            index.setdefault(h.strip(), i)
+        for i, h in enumerate(headers):
+            if h.split():
+                index.setdefault(h.split()[0], i)
+    cur = 0 if headers is None else None
+    seq, lo, length, strand = [], [], [], []
+    for k, line in enumerate(lines, 1):
+        if isinstance(line, bytes):
+            line = line.decode()
+        t = line.split()
+        if not t:
+            continue
+        if line.startswith(">"):
+            if index is None:
+                raise GmgError(f"coordinates line {k}: a '>' line selects a sequence; pass headers= to say which")
+            name = line[1:].strip()
+            cur = index.get(name, index.get(name.split()[0] if name.split() else name))
+            if cur is None:
+                raise GmgError(f"coordinates line {k}: no sequence with header {name!r}")
+            continue
+        if cur is None:
+            raise GmgError(f"coordinates line {k}: coordinates before the first '>' line")
+        if len(t) < 3:
+            raise GmgError(f"coordinates line {k}: expected `id start end`, got {line.strip()!r}")
+        start, end = int(t[1]), int(t[2])
+        fwd = start <= end
+        if len(t) > 3 and _FRAME.fullmatch(t[3]) and (t[3][0] == "+") != fwd:
+            raise GmgError(f"coordinates line {k}: {t[0]} runs from {start} to {end} in frame {t[3]}: it wraps around "
+                           "the end of its sequence, which extraction does not support")
+        a, b = (start - 1, end) if fwd else (end - 1, start)  # 0-based [a, b)
+        if trim_stop:
+            if fwd:
+                b -= 3
+            else:
+                a += 3
+        if b < a:
+            raise GmgError(f"coordinates line {k}: {t[0]} is shorter than its stop codon")
+        seq.append(cur)
+        lo.append(a)
+        length.append(b - a)
+        strand.append(1 if fwd else -1)
+    return (np.array(seq, np.int32), np.array(lo, np.int32), np.array(length, np.int32), np.array(strand, np.int8))
 
 
 def score_strings_many(ctx, models, strings, frame=0, pinned=False):

@@ -136,7 +136,7 @@ void gmg_icm_free(gmg_icm* m);
  * one Phred value per base (Fasta_Qual_Vec_Read, fasta.cc:115). */
 int gmg_seqset_create(gmg_ctx* ctx, const char* h_ascii, const int64_t* h_off, int64_t n,
                       const uint8_t* h_qual, gmg_seqset** out);
-/* same, ASCII already resident in HBM (d_ascii); offsets still from the host. async. */
+/* same, ASCII already resident in HBM (d_ascii); offsets still from the host.  Returns once d_ascii has been read. */
 int gmg_seqset_create_device(gmg_ctx* ctx, const void* d_ascii, const int64_t* h_off, int64_t n,
                              const void* d_qual, gmg_seqset** out);
 void gmg_seqset_free(gmg_seqset* s);
@@ -168,6 +168,14 @@ int64_t gmg_seqset_total_bases(const gmg_seqset* s);
 int gmg_seqset_gc_fraction(gmg_seqset* s, double* gc);
 /* unpack to lower-case acgt (what the drivers hold in `Sequence`) */
 int gmg_seqset_unpack(gmg_seqset* s, char* h_out);
+/* extract (Util/extract.cc) on a resident set: n regions [lo[i], lo[i] + len[i]) of sequence seq[i] (0-based) become the
+ * n sequences of a new set; strand[i] = -1 takes the reverse complement of the region, complementing raw IUPAC codes before
+ * Filter as extract + build-icm do.  Regions must lie inside their sequence (no wrap-around).  The new set is an ordinary
+ * set (score, find ORFs, train, unpack, extract again); it carries no qualities and no headers.  Every set keeps the
+ * position and raw code of each input byte other than a / c / g / t for this; a minus region's output holds the
+ * complemented code, so extracting from an extracted set equals extracting from the source directly. */
+int gmg_seqset_extract(gmg_ctx* ctx, gmg_seqset* src, int64_t n, const int32_t* h_seq, const int32_t* h_lo,
+                       const int32_t* h_len, const int8_t* h_strand, gmg_seqset** out);
 
 /* ---- scalar operator surface (each call = device work over one string) -------------- */
 /* ICM_t::Score_String (icm.cc:864-903) for n strings of a seqset; frame = first base's period */
