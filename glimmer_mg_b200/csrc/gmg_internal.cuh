@@ -185,6 +185,8 @@ enum { SCR_PLANES = 0, SCR_CUM = 1, SCR_TMP = 2, SCR_TMP2 = 3, SCR_FLAGS = 4, SC
        SCR_MG_GATE = 8, SCR_MG_ROOT = 9, SCR_MG_L0 = 10, SCR_MG_CALL1 = 11, SCR_MG_L1 = 12, SCR_MG_L2 = 13, SCR_RED = 14,
        SCR_MISC = 15 };
 int gmg_scratch(gmg_ctx* ctx, int slot, size_t bytes, void** out);
+// ctx->h_stage holds at least `bytes` (grown to max(bytes, want)); its contents are not kept when it grows
+int gmg_host_stage(gmg_ctx* ctx, size_t bytes, size_t want);
 
 // ---- device helpers ---------------------------------------------------------------------
 

@@ -10,6 +10,7 @@
 
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+#include <thrust/iterator/transform_iterator.h>
 
 #include "gmg_internal.cuh"
 
@@ -734,6 +735,294 @@ extern "C" int gmg_seqset_quality_from_fasta(gmg_ctx* ctx, gmg_seqset* s, const 
     GMG_CUDA(cudaGetLastError());
     GMG_CUDA(cudaStreamSynchronize(ctx->stream));  // the values live in context scratch
   }
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// FASTQ ingest on the device: four-line records (header '@', sequence, '+' [header], qualities).  One scan over the
+// '\n' marks gives every byte its line; record r is lines 4r .. 4r+3.  The records end at the line of the last
+// non-white-space byte, so blank lines may follow the last record.  The first failure is the smallest (line, reason,
+// byte) key of any check; it travels to the host with the record count in one stream synchronisation.
+enum { FQ_NO_AT = 0, FQ_NO_PLUS = 1, FQ_PLUS_TEXT = 2, FQ_TRUNCATED = 3, FQ_QUAL_LEN = 4, FQ_QUAL_BYTE = 5 };
+
+// line < 2^31, reason < 8, byte position < 2^30 (images are < 1 GiB)
+__device__ __forceinline__ unsigned long long fq_key(int64_t line, unsigned reason, int64_t pos) {
+  return ((unsigned long long)line << 33) | ((unsigned long long)reason << 30) | (unsigned long long)pos;
+}
+
+struct FqIsNewline {
+  __host__ __device__ __forceinline__ uint32_t operator()(uint8_t c) const { return c == '\n' ? 1u : 0u; }
+};
+
+struct FqCtl {
+  unsigned long long err;  // first failure (fq_key), ~0 = none
+  int32_t last_nb;         // line of the last non-white-space byte, -1 = none
+  uint32_t last_line;      // index of the last line (the text after a final '\n' is an empty last line)
+};
+
+// One thread per byte, line[i] = '\n' bytes before byte i.  starts[j] = first byte of line j, starts[last + 1] = n + 1,
+// so line j ends (at its '\n' or at the image end) at starts[j + 1] - 1.  Also the range check of every quality byte
+// (lines 4r+3 without their '\n' and one trailing '\r'): lines past the last record are blank, and a key on one of them
+// sorts after every failure inside the records, so the host drops it.
+__global__ void __launch_bounds__(256) k_fastq_lines(const uint8_t* __restrict__ in, int64_t n,
+                                                     const uint32_t* __restrict__ line, unsigned lo,
+                                                     uint32_t* __restrict__ starts, FqCtl* __restrict__ ctl) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  int nb = -1;
+  unsigned long long bad = ~0ull;
+  if (i < n) {
+    const unsigned ch = in[i];
+    const uint32_t j = line[i];
+    if (ch == '\n') starts[j + 1] = (uint32_t)(i + 1);
+    if (i == 0) starts[0] = 0;
+    if (i == n - 1) {
+      const uint32_t last = j + (ch == '\n' ? 1u : 0u);
+      starts[last + 1] = (uint32_t)(n + 1);
+      ctl->last_line = last;
+    }
+    if (!fasta_is_space(ch)) nb = (int)j;
+    if ((j & 3u) == 3u && ch != '\n' && !(ch == '\r' && (i + 1 == n || in[i + 1] == '\n')) && (ch < lo || ch > '~'))
+      bad = fq_key(j, FQ_QUAL_BYTE, i);
+  }
+  nb = __reduce_max_sync(0xffffffffu, nb);
+  if ((threadIdx.x & 31) == 0 && nb >= 0) atomicMax(&ctl->last_nb, nb);
+  if (__any_sync(0xffffffffu, bad != ~0ull)) {
+    for (int o = 16; o > 0; o >>= 1) {
+      const unsigned long long t = __shfl_xor_sync(0xffffffffu, bad, o);
+      bad = t < bad ? t : bad;
+    }
+    if ((threadIdx.x & 31) == 0) atomicMin(&ctl->err, bad);
+  }
+}
+
+// One warp per record (grid-stride; the record count is on the device): the '@' and '+' lines, the '+' text against the
+// header, the sequence characters (non-white-space bytes of line 4r+1) and the quality line's length.  Writes the
+// sequence length and the header span; seq_len[n_rec] = 0 so that an exclusive sum over n_rec + 1 entries ends in the total.
+__global__ void __launch_bounds__(256) k_fastq_records(const uint8_t* __restrict__ in, const uint32_t* __restrict__ starts,
+                                                       FqCtl* __restrict__ ctl, uint32_t* __restrict__ seq_len,
+                                                       uint32_t* __restrict__ hdr_off, uint32_t* __restrict__ hdr_end) {
+  const int lane = threadIdx.x & 31;
+  const int64_t last_nb = ctl->last_nb, last_line = ctl->last_line;
+  const int64_t n_rec = last_nb < 0 ? 0 : last_nb / 4 + 1;
+  if (blockIdx.x == 0 && threadIdx.x == 0) seq_len[n_rec] = 0;
+  const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < n_rec; r += warps) {
+    const int64_t l0 = 4 * r;
+    const int64_t have = last_line - l0 + 1;  // lines of the record in the image (>= 1)
+    unsigned long long err = have < 4 ? fq_key(last_line + 1, FQ_TRUNCATED, 0) : ~0ull;
+    // header: '@', then the text after the blanks, to the line end
+    const int64_t h0 = starts[l0], h1 = (int64_t)starts[l0 + 1] - 1;
+    int64_t ho = h1;
+    if (h1 > h0 && in[h0] == '@') {
+      ho = h0 + 1;
+      while (ho < h1 && in[ho] == ' ') ho++;
+    } else {
+      err = min(err, fq_key(l0, FQ_NO_AT, h0));
+    }
+    unsigned cnt = 0;
+    if (have >= 2) {
+      const int64_t s0 = starts[l0 + 1], s1 = (int64_t)starts[l0 + 2] - 1;
+      for (int64_t p = s0 + lane; p < s1; p += 32) cnt += fasta_is_space(in[p]) ? 0u : 1u;
+      cnt = __reduce_add_sync(0xffffffffu, cnt);
+    }
+    if (have >= 3) {
+      const int64_t p0 = starts[l0 + 2], p1 = (int64_t)starts[l0 + 3] - 1;
+      if (p1 > p0 && in[p0] == '+') {
+        int64_t pt = p0 + 1, pe = p1, he = h1;  // one trailing '\r' of either line does not count
+        while (pt < pe && in[pt] == ' ') pt++;
+        if (pe > pt && in[pe - 1] == '\r') pe--;
+        if (he > ho && in[he - 1] == '\r') he--;
+        if (pe > pt) {
+          bool differ = pe - pt != he - ho;
+          if (!differ) {
+            bool d = false;
+            for (int64_t k = lane; k < pe - pt; k += 32) d |= in[pt + k] != in[ho + k];
+            differ = __any_sync(0xffffffffu, d);
+          }
+          if (differ) err = min(err, fq_key(l0 + 2, FQ_PLUS_TEXT, p0));
+        }
+      } else {
+        err = min(err, fq_key(l0 + 2, FQ_NO_PLUS, p0));
+      }
+    }
+    if (have >= 4) {
+      const int64_t q0 = starts[l0 + 3];
+      int64_t q1 = (int64_t)starts[l0 + 4] - 1;
+      if (q1 > q0 && in[q1 - 1] == '\r') q1--;
+      if (q1 - q0 != (int64_t)cnt) err = min(err, fq_key(l0 + 3, FQ_QUAL_LEN, q0));
+    }
+    if (lane == 0) {
+      seq_len[r] = cnt;
+      hdr_off[r] = (uint32_t)ho;
+      hdr_end[r] = (uint32_t)h1;
+      if (err != ~0ull) atomicMin(&ctl->err, err);
+    }
+  }
+}
+
+// One warp per record of a checked image: the sequence characters to seq[off[r] ..) (a ballot keeps their order past
+// white space) and the quality bytes minus the Phred offset to qual[off[r] ..)
+__global__ void __launch_bounds__(256) k_fastq_copy(const uint8_t* __restrict__ in, const uint32_t* __restrict__ starts,
+                                                    const int64_t* __restrict__ off, int64_t n_rec, unsigned lo,
+                                                    uint8_t* __restrict__ seq, uint8_t* __restrict__ qual) {
+  const int lane = threadIdx.x & 31;
+  const int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (r >= n_rec) return;  // warp-uniform
+  const int64_t s0 = starts[4 * r + 1], s1 = (int64_t)starts[4 * r + 2] - 1, q0 = starts[4 * r + 3];
+  const int64_t o = off[r], len = off[r + 1] - o;
+  int64_t k = o;
+  for (int64_t p = s0; p < s1; p += 32) {
+    const unsigned ch = p + lane < s1 ? in[p + lane] : ' ';
+    const bool keep = !fasta_is_space(ch);
+    const unsigned m = __ballot_sync(0xffffffffu, keep);
+    if (keep) seq[k + __popc(m & ((1u << lane) - 1u))] = (uint8_t)ch;
+    k += __popc(m);
+  }
+  for (int64_t t = lane; t < len; t += 32) qual[o + t] = (uint8_t)(in[q0 + t] - lo);
+}
+
+// the message of the first failure (key from k_fastq_lines / k_fastq_records)
+static int fastq_error(gmg_ctx* ctx, const char* h_bytes, int64_t n, int phred_offset, unsigned long long key,
+                       const uint32_t* d_seq_len) {
+  const int64_t line = (int64_t)(key >> 33), pos = (int64_t)(key & ((1ull << 30) - 1));
+  const int reason = (int)((key >> 30) & 7);
+  const long long rec = line / 4 + 1, ln = line + 1;
+  switch (reason) {
+    case FQ_NO_AT:
+      gmg_set_error("gmg_seqset_from_fastq: record %lld (line %lld): the header line does not start with '@' "
+                    "(multi-line FASTQ records are not supported)", rec, ln);
+      break;
+    case FQ_NO_PLUS:
+      gmg_set_error("gmg_seqset_from_fastq: record %lld (line %lld): the separator line does not start with '+' "
+                    "(multi-line FASTQ records are not supported)", rec, ln);
+      break;
+    case FQ_PLUS_TEXT:
+      gmg_set_error("gmg_seqset_from_fastq: record %lld (line %lld): the text after '+' differs from the header", rec, ln);
+      break;
+    case FQ_TRUNCATED: {
+      static const char* role[4] = {"header", "sequence", "'+'", "quality"};
+      gmg_set_error("gmg_seqset_from_fastq: record %lld (line %lld): truncated last record: the image ends before its %s "
+                    "line", rec, ln, role[line & 3]);
+      break;
+    }
+    case FQ_QUAL_LEN: {
+      uint32_t cnt = 0;
+      GMG_CUDA(cudaMemcpyAsync(&cnt, d_seq_len + (rec - 1), sizeof cnt, cudaMemcpyDeviceToHost, ctx->stream));
+      GMG_CUDA(cudaStreamSynchronize(ctx->stream));
+      const char* nl = (const char*)memchr(h_bytes + pos, '\n', (size_t)(n - pos));
+      int64_t q1 = nl ? nl - h_bytes : n;
+      if (q1 > pos && h_bytes[q1 - 1] == '\r') q1--;
+      gmg_set_error("gmg_seqset_from_fastq: record %lld (line %lld): the quality line holds %lld characters, the sequence "
+                    "%lld", rec, ln, (long long)(q1 - pos), (long long)cnt);
+      break;
+    }
+    default: {
+      int64_t a = pos;
+      while (a > 0 && h_bytes[a - 1] != '\n') a--;
+      gmg_set_error("gmg_seqset_from_fastq: record %lld (line %lld): quality byte %d at column %lld is outside [%d, 126] "
+                    "(phred offset %d)", rec, ln, (int)(uint8_t)h_bytes[pos], (long long)(pos - a + 1), phred_offset,
+                    phred_offset);
+      break;
+    }
+  }
+  return 1;
+}
+
+extern "C" int gmg_seqset_from_fastq(gmg_ctx* ctx, const char* h_bytes, int64_t n_bytes, int phred_offset,
+                                     gmg_seqset** out, int64_t* n_records) {
+  GMG_CHECK(ctx && out && n_bytes >= 0 && (h_bytes || n_bytes == 0), "gmg_seqset_from_fastq: bad argument");
+  *out = NULL;
+  if (n_records) *n_records = 0;
+  GMG_CHECK(phred_offset == 33 || phred_offset == 64, "gmg_seqset_from_fastq: phred_offset must be 33 or 64 (got %d)",
+            phred_offset);
+  GMG_CHECK(n_bytes < (1ll << 30), "gmg_seqset_from_fastq: images of 1 GiB or more must be split at record boundaries "
+            "(got %lld bytes)", (long long)n_bytes);
+  GMG_CUDA(cudaSetDevice(ctx->device));
+  const int64_t n = n_bytes;
+  const unsigned lo = (unsigned)phred_offset;
+  int64_t n_rec = 0;
+  std::vector<int64_t> off(1, 0), hdr_off, hdr_end;
+  void *d_seq = NULL, *d_qual = NULL;
+  if (n > 0) {
+    void *d_in, *d_work, *d_tab, *d_tmp;
+    if (gmg_scratch(ctx, SCR_TMP, (size_t)n + 64, &d_in)) return 1;
+    GMG_CUDA(cudaMemcpyAsync(d_in, h_bytes, (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    // line of every byte | line starts (at most n + 1 lines, plus the end sentinel) | control block
+    if (gmg_scratch(ctx, SCR_CUM, (size_t)(2 * n + 2) * sizeof(uint32_t) + 64, &d_work)) return 1;
+    uint32_t* d_line = (uint32_t*)d_work;
+    uint32_t* d_starts = d_line + n;
+    FqCtl* d_ctl = (FqCtl*)(((uintptr_t)(d_starts + n + 2) + 15) & ~(uintptr_t)15);
+    // per record (at most (n + 1) / 4 + 1 of them): offsets (int64) | sequence length | header start | header end
+    const int64_t cap = n / 4 + 2;
+    if (gmg_scratch(ctx, SCR_TMP3, (size_t)cap * (sizeof(int64_t) + 3 * sizeof(uint32_t)), &d_tab)) return 1;
+    int64_t* d_off = (int64_t*)d_tab;
+    uint32_t* d_len = (uint32_t*)(d_off + cap);
+    uint32_t* d_hoff = d_len + cap;
+    uint32_t* d_hend = d_hoff + cap;
+    GMG_CUDA(cudaMemsetAsync(d_ctl, 0xFF, sizeof(FqCtl), ctx->stream));  // err = ~0, last_nb = -1
+    const auto nl = thrust::make_transform_iterator((const uint8_t*)d_in, FqIsNewline());
+    size_t tb = 0;
+    GMG_CUDA(cub::DeviceScan::ExclusiveSum(NULL, tb, nl, d_line, n, ctx->stream));
+    if (gmg_scratch(ctx, SCR_TMP4, tb, &d_tmp)) return 1;
+    GMG_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp, tb, nl, d_line, n, ctx->stream));
+    k_fastq_lines<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>((const uint8_t*)d_in, n, d_line, lo, d_starts,
+                                                                        d_ctl);
+    const int64_t rblk = (cap + 7) / 8;  // eight warps a block
+    k_fastq_records<<<(unsigned)(rblk < 16 * ctx->sm_count ? rblk : 16 * ctx->sm_count), 256, 0, ctx->stream>>>(
+        (const uint8_t*)d_in, d_starts, d_ctl, d_len, d_hoff, d_hend);
+    ctx->launches += 3;
+    GMG_CUDA(cudaGetLastError());
+    GMG_CUDA(cudaMemcpyAsync(ctx->h_scalars + 4, d_ctl, sizeof(FqCtl), cudaMemcpyDeviceToHost, ctx->stream));
+    GMG_CUDA(cudaStreamSynchronize(ctx->stream));
+    FqCtl c;
+    memcpy(&c, ctx->h_scalars + 4, sizeof c);
+    n_rec = c.last_nb < 0 ? 0 : (int64_t)c.last_nb / 4 + 1;
+    if (c.err != ~0ull && (int64_t)(c.err >> 33) < 4 * n_rec) return fastq_error(ctx, h_bytes, n, phred_offset, c.err, d_len);
+    if (n_rec > 0) {
+      GMG_CUDA(cub::DeviceScan::ExclusiveSum(NULL, tb, d_len, d_off, n_rec + 1, ctx->stream));
+      if (gmg_scratch(ctx, SCR_TMP4, tb, &d_tmp)) return 1;
+      GMG_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp, tb, d_len, d_off, n_rec + 1, ctx->stream));
+      // at most n sequence characters
+      if (gmg_scratch(ctx, SCR_TMP2, (size_t)n + 64, &d_seq)) return 1;
+      if (gmg_scratch(ctx, SCR_QUAL, (size_t)n + 64, &d_qual)) return 1;
+      k_fastq_copy<<<(unsigned)((n_rec + 7) / 8), 256, 0, ctx->stream>>>((const uint8_t*)d_in, d_starts, d_off, n_rec, lo,
+                                                                         (uint8_t*)d_seq, (uint8_t*)d_qual);
+      ctx->launches += 2;
+      GMG_CUDA(cudaGetLastError());
+      // offsets | header starts | header ends through the context's page-locked staging
+      const size_t ob = (size_t)(n_rec + 1) * sizeof(int64_t), hb = (size_t)n_rec * sizeof(uint32_t);
+      if (gmg_host_stage(ctx, ob + 2 * hb, 0)) return 1;
+      char* st = (char*)ctx->h_stage;
+      GMG_CUDA(cudaMemcpyAsync(st, d_off, ob, cudaMemcpyDeviceToHost, ctx->stream));
+      GMG_CUDA(cudaMemcpyAsync(st + ob, d_hoff, hb, cudaMemcpyDeviceToHost, ctx->stream));
+      GMG_CUDA(cudaMemcpyAsync(st + ob + hb, d_hend, hb, cudaMemcpyDeviceToHost, ctx->stream));
+      GMG_CUDA(cudaStreamSynchronize(ctx->stream));
+      off.assign((const int64_t*)st, (const int64_t*)st + n_rec + 1);
+      hdr_off.assign((const uint32_t*)(st + ob), (const uint32_t*)(st + ob) + n_rec);
+      hdr_end.assign((const uint32_t*)(st + ob + hb), (const uint32_t*)(st + ob + hb) + n_rec);
+    }
+  }
+  gmg_seqset* s = NULL;
+  if (seqset_build(ctx, d_seq, off.data(), n_rec, d_qual, &s)) return 1;
+  s->hdr_off.swap(hdr_off);
+  s->hdr_end.swap(hdr_end);
+  GMG_CUDA(cudaStreamSynchronize(ctx->stream));  // d_seq / d_qual (scratch) have been consumed
+  if (seqset_finish_nacgt(ctx, s, d_seq)) {
+    gmg_seqset_free(s);
+    return 1;
+  }
+  *out = s;
+  if (n_records) *n_records = n_rec;
+  return 0;
+}
+
+extern "C" int gmg_seqset_qualities(const gmg_seqset* s, uint8_t* h_out) {
+  GMG_CHECK(s, "gmg_seqset_qualities: NULL set");
+  GMG_CHECK(s->d_qual, "gmg_seqset_qualities: the set has no qualities");
+  if (!h_out) return 0;
+  GMG_CUDA(cudaSetDevice(s->ctx->device));
+  GMG_CUDA(cudaMemcpyAsync(h_out, s->d_qual, (size_t)s->total, cudaMemcpyDeviceToHost, s->ctx->stream));
+  GMG_CUDA(cudaStreamSynchronize(s->ctx->stream));
   return 0;
 }
 

@@ -785,7 +785,7 @@ static void finish_node_host(gmg_trainer* t, int level, int f, int sub, const in
   }
 }
 
-static int ensure_stage(gmg_ctx* ctx, size_t bytes, size_t want) {
+int gmg_host_stage(gmg_ctx* ctx, size_t bytes, size_t want) {
   if (ctx->h_stage_bytes >= bytes) return 0;
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
   ctx->h_stage = NULL;
@@ -822,7 +822,7 @@ extern "C" int gmg_trainer_finish_level(gmg_trainer* t, int level) {
     gmg_prof_end(ctx, GMG_PROF_K4);
     ctx->launches++;
     GMG_CUDA(cudaGetLastError());
-    if (ensure_stage(ctx, out_bytes, (size_t)rows * level_nodes(t->D) * 24 + 256)) return 1;
+    if (gmg_host_stage(ctx, out_bytes, (size_t)rows * level_nodes(t->D) * 24 + 256)) return 1;
     GMG_CUDA(cudaMemcpyAsync(ctx->h_stage, t->d_lvl, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     GMG_CUDA(cudaStreamSynchronize(ctx->stream));
     const int8_t* h_mip = (const int8_t*)ctx->h_stage;
@@ -856,7 +856,7 @@ extern "C" int gmg_trainer_finish_level(gmg_trainer* t, int level) {
       const int g_apply = (int)((nf + 255) / 256 < cap ? (nf + 255) / 256 : cap);
       // the same layout in the page-locked staging buffer, whose level results have been read above; the next writer
       // of the buffer is the next level's D2H, ordered on the stream after the H2D of the fixes
-      if (ensure_stage(ctx, fix_off + (size_t)nf * sizeof(K4Fix), 0)) {
+      if (gmg_host_stage(ctx, fix_off + (size_t)nf * sizeof(K4Fix), 0)) {
         cudaFreeAsync(d_buf, ctx->stream);
         return 1;
       }
@@ -894,7 +894,7 @@ extern "C" int gmg_trainer_finish_level(gmg_trainer* t, int level) {
     return 0;
   }
   // ---- host: the slab comes back through the context's page-locked staging buffer ----
-  if (ensure_stage(ctx, slab_bytes, (size_t)rows * level_nodes(t->D) * per * sizeof(int32_t))) return 1;
+  if (gmg_host_stage(ctx, slab_bytes, (size_t)rows * level_nodes(t->D) * per * sizeof(int32_t))) return 1;
   GMG_CUDA(cudaMemcpyAsync(ctx->h_stage, t->d_counts, slab_bytes, cudaMemcpyDeviceToHost, ctx->stream));
   GMG_CUDA(cudaStreamSynchronize(ctx->stream));
   const int32_t* C = (const int32_t*)ctx->h_stage;

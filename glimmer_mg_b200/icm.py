@@ -98,6 +98,8 @@ def lib():
         "gmg_seqset_fasta_headers": (i32, [vp, vp, vp]),
         "gmg_quality_parse_fasta": (i32, [vp, vp, i64, P(i64), P(i64), vp, vp, i64, i64]),
         "gmg_seqset_quality_from_fasta": (i32, [vp, vp, vp, i64]),
+        "gmg_seqset_from_fastq": (i32, [vp, vp, i64, i32, P(vp), P(i64)]),
+        "gmg_seqset_qualities": (i32, [vp, vp]),
         "gmg_seqset_total_bases": (i64, [vp]),
         "gmg_seqset_gc_fraction": (i32, [vp, P(C.c_double)]),
         "gmg_seqset_unpack": (i32, [vp, vp]),
@@ -316,7 +318,23 @@ class SeqSet:
             np.ascontiguousarray(image, np.uint8)
         h, n = C.c_void_p(), C.c_int64()
         _check(lib().gmg_seqset_from_fasta(ctx.h, buf.ctypes.data if len(buf) else None, len(buf), C.byref(h), C.byref(n)))
-        self = cls._adopt(ctx, h)
+        return cls._adopt(ctx, h)._read_headers(buf)
+
+    @classmethod
+    def from_fastq(cls, ctx, image, phred_offset=33):
+        """Parse a FASTQ image (bytes / uint8 array; four-line records) on the device: sequences, ``headers`` (as
+        ``from_fasta`` reports the same lines with '>' for '@') and per-base qualities (byte - ``phred_offset``, 33 or
+        64), attached as ``set_quality_fasta`` attaches them.  Malformed input raises GmgError naming the record and
+        line."""
+        buf = np.frombuffer(image, np.uint8) if isinstance(image, (bytes, bytearray, memoryview)) else \
+            np.ascontiguousarray(image, np.uint8)
+        h, n = C.c_void_p(), C.c_int64()
+        _check(lib().gmg_seqset_from_fastq(ctx.h, buf.ctypes.data if len(buf) else None, len(buf), int(phred_offset),
+                                           C.byref(h), C.byref(n)))
+        return cls._adopt(ctx, h)._read_headers(buf)
+
+    def _read_headers(self, buf):
+        """``headers``: the header text of every record, from the offsets into the image ``buf``."""
         ho, he = np.zeros(self.n, np.int64), np.zeros(self.n, np.int64)
         if self.n:
             _check(lib().gmg_seqset_fasta_headers(self.h, ho.ctypes.data, he.ctypes.data))
@@ -359,6 +377,14 @@ class SeqSet:
         buf = np.frombuffer(image, np.uint8) if isinstance(image, (bytes, bytearray, memoryview)) else \
             np.ascontiguousarray(image, np.uint8)
         _check(lib().gmg_seqset_quality_from_fasta(self.ctx.h, self.h, buf.ctypes.data if len(buf) else None, len(buf)))
+
+    def qualities(self):
+        """Per-base qualities as attached (uint8 [total]), or None when the set has none."""
+        if lib().gmg_seqset_qualities(self.h, None) != 0:
+            return None
+        out = np.zeros(self.total, np.uint8)
+        _check(lib().gmg_seqset_qualities(self.h, out.ctypes.data))
+        return out
 
     def close(self):
         if self.h:

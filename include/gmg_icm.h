@@ -163,6 +163,32 @@ int gmg_seqset_fasta_headers(const gmg_seqset* s, int64_t* h_hdr_off, int64_t* h
 int gmg_quality_parse_fasta(gmg_ctx* ctx, const char* h_bytes, int64_t n_bytes, int64_t* n_records, int64_t* n_values,
                             int64_t* h_off, int32_t* h_values, int64_t cap_records, int64_t cap_values);
 int gmg_seqset_quality_from_fasta(gmg_ctx* ctx, gmg_seqset* s, const char* h_bytes, int64_t n_bytes);
+/* FASTQ ingest on the device: the sequences and Phred qualities of a FASTQ image in host memory (page-locked memory from
+ * gmg_host_alloc makes the copy run at PCIe rate).  Four-line records, LF or CRLF line ends:
+ *   line 1  '@' and the header.  Its text is what gmg_seqset_fasta_headers reports for the same line with '>' in place of
+ *           '@' (blanks after the marker skipped, the text runs to the line end), so FASTQ converted to FASTA keeps its
+ *           headers.  gmg_seqset_fasta_headers returns it as offsets into the FASTQ image.
+ *   line 2  the sequence: every non-white-space byte is a sequence character (Filter + lower-case + 2-bit pack as in
+ *           gmg_seqset_create, and the set keeps its non-acgt list, so gmg_seqset_extract works on it).
+ *   line 3  '+', optionally followed by the header text again (blanks after the '+' skipped; one trailing '\r' of either
+ *           line does not count).  Any other text is an error.
+ *   line 4  the qualities: as many bytes as line 2 has sequence characters (one trailing '\r' does not count), each in
+ *           [phred_offset, '~']; the value is byte - phred_offset.  phred_offset is 33 or 64.
+ * An empty sequence with an empty quality line is a record of length 0.  The last line may lack its '\n' (the text after
+ * a final '\n' is an empty last line).  Blank lines may follow the last record, nowhere else: the records end at the line
+ * of the last non-white-space byte.  Multi-line records are not supported (they fail the '@' / '+' checks).  Images must
+ * be < 1 GiB (split larger files at record boundaries).
+ * Every violation fails the call, with a message (gmg_last_error) naming the first bad record and its line (1-based) and
+ * the reason: no '@' / '+', '+' text other than the header, quality length other than the sequence length, a quality
+ * byte out of range, or a truncated last record.  Nothing is allocated for a rejected image (*out = NULL) and the
+ * context stays usable.
+ * The set carries its qualities exactly as gmg_seqset_quality_from_fasta attaches them, so gmg_score_orfs_mg with
+ * have_quality_file = 1 runs on it directly. */
+int gmg_seqset_from_fastq(gmg_ctx* ctx, const char* h_bytes, int64_t n_bytes, int phred_offset, gmg_seqset** out,
+                          int64_t* n_records);
+/* per-base qualities of any set (0..255, as attached: total_bases bytes to h_out); returns non-zero if the set has none
+ * (a set without bases has none).  h_out = NULL only asks whether it has them. */
+int gmg_seqset_qualities(const gmg_seqset* s, uint8_t* h_out);
 int64_t gmg_seqset_total_bases(const gmg_seqset* s);
 /* Set_GC_Fraction (glimmer_base.cc:2564-2595): (#c + #g after Filter) / total */
 int gmg_seqset_gc_fraction(gmg_seqset* s, double* gc);
