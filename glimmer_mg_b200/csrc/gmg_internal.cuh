@@ -16,7 +16,7 @@
 #define GMG_CTX_PAD 16384
 #define GMG_PAD_WORDS 8   // 64-bit words of zero padding before/after the packed bases
 #define GMG_NPROF 8
-#define GMG_NSCRATCH 16
+#define GMG_NSCRATCH 20
 #define GMG_PROF_RING 64
 
 void gmg_set_error(const char* fmt, ...);
@@ -87,6 +87,9 @@ struct gmg_ctx {
   cudaEvent_t ev_fork, ev_join;
   double mg_rate[4];   // start records per base seen by the last gmg_score_orfs_mg call, by (indels, subs) mode
   int64_t train_flagged;  // nodes of the last gmg_icm_train* call that the host recomputed (gmg_ctx_train_flagged)
+  int64_t indep_flagged;  // model entries of the last gmg_score_orfs_mg_gc call that the host recomputed (gmg_ctx_indep_flagged)
+  struct gmg_icm* indep_tpl;  // Build_Indep_WO_Stops topology (gmg_indep_build): walk tables shared by every GC's model
+  uint8_t* d_indep_src;       // [GMG_INDEP_REC] compact slot of every record entry (gmg_indep_build)
   void* h_stage;       // pinned staging for larger device -> host results (training count slabs), grown on demand
   size_t h_stage_bytes;
   // per-kernel device timing (gmg_ctx_profile): event pairs around the launches of each kernel class
@@ -183,7 +186,10 @@ struct gmg_seqset {
 enum { SCR_PLANES = 0, SCR_CUM = 1, SCR_TMP = 2, SCR_TMP2 = 3, SCR_FLAGS = 4, SCR_TMP3 = 5, SCR_QUAL = 6, SCR_TMP4 = 7,
        // flat glimmer-mg start enumeration (gmg_mg_flat.cuh): gates, root calls, per-level work arrays; reduction output
        SCR_MG_GATE = 8, SCR_MG_ROOT = 9, SCR_MG_L0 = 10, SCR_MG_CALL1 = 11, SCR_MG_L1 = 12, SCR_MG_L2 = 13, SCR_RED = 14,
-       SCR_MISC = 15 };
+       SCR_MISC = 15,
+       // gmg_score_orfs_mg_gc: per-GC model records, the call's inputs (GC values, sequence -> record, ignore lengths),
+       // the flagged-model list and the host's corrections
+       SCR_INDEP = 16, SCR_INDEP_IN = 17, SCR_INDEP_AUX = 18, SCR_INDEP_FIX = 19 };
 int gmg_scratch(gmg_ctx* ctx, int slot, size_t bytes, void** out);
 // ctx->h_stage holds at least `bytes` (grown to max(bytes, want)); its contents are not kept when it grows
 int gmg_host_stage(gmg_ctx* ctx, size_t bytes, size_t want);
@@ -247,6 +253,28 @@ __device__ __forceinline__ uint64_t gmg_reverse_bases(uint64_t v, int W) {
   v = (v >> 32) | (v << 32);
   return v >> (2 * (32 - W));
 }
+
+// ---- per-sequence independent models (gmg_score_orfs_mg_gc) ----------------------------------------------------
+// Build_Indep_WO_Stops (icm.cc:65-216) on the host: mip [3][21], prob [3][21][4] of the ICM_t(3,2,3)
+void gmg_indep_tables(double gc, const char* const* stops, int n_stops, int16_t* mip, float* prob);
+// Subscript(Filter(ch)) (icm.cc:2008-2027)
+int gmg_base_code(char ch);
+// the entries of the device view's prob table ((period * N + node) * 4 + base) that the full-window table
+// lut3 [384] and the partial-window table lutp [768] of a W == 3, P == 3 model take (icm_upload)
+void gmg_w3_lut_index(const int16_t* mip, int N, int D, int* idx3, int* idxp);
+// One record per GC value: the device view's prob [3][21][4], lut3 [384] and lutp [768] floats, in this order.  A kernel
+// scores a sequence with its record by pointing a copy of the shared DevIcm (W, D, P, N, mip) at it.
+#define GMG_INDEP_REC (252 + 384 + 768)
+struct IndepSeqs {
+  const float* rec;        // [n_models][GMG_INDEP_REC]
+  const int32_t* model;    // [n_seq] record of every sequence
+  const int32_t* isl;      // [n_seq] Ignore_Score_Len of every sequence
+  const int32_t* orf_seq;  // [n_orfs] sequence of every ORF (for kernels that otherwise see only ORF descriptors)
+};
+// the n_models records for the GC values d_gc (device) / h_gc (host, the same values) with p's stop codons into the
+// context's SCR_INDEP scratch; *base = the shared part of the device view
+int gmg_indep_build(gmg_ctx* ctx, const double* d_gc, const double* h_gc, int64_t n_models, const gmg_params* p,
+                    float** d_rec, DevIcm* base);
 
 int gmg_seqset_ensure_buckets(gmg_ctx* ctx, gmg_seqset* s);
 // kernel launchers implemented across the .cu files

@@ -83,6 +83,8 @@ extern "C" void gmg_host_free(void* p) {
 extern "C" void gmg_ctx_destroy(gmg_ctx* c) {
   if (!c) return;
   cudaSetDevice(c->device);
+  gmg_icm_free(c->indep_tpl);
+  if (c->d_indep_src) cudaFree(c->d_indep_src);
   for (int i = 0; i < GMG_NSCRATCH; i++)
     if (c->scratch[i]) cudaFree(c->scratch[i]);
   if (c->h_penalty) cudaFreeHost(c->h_penalty);
@@ -221,7 +223,7 @@ extern "C" int gmg_ignore_score_len(double gc, const gmg_params* p) {
 
 // ------------------------------------------------------------------------------------------
 
-static int base_code(char ch) {
+int gmg_base_code(char ch) {
   // Subscript(Filter(ch)) (icm.cc:2008-2027, gene.cc:1139-1175)
   switch (ch | 0x20) {
     case 'a': return 0;
@@ -259,6 +261,30 @@ static int num_nodes_for(int d) {
     n += pw;
   }
   return (int)n;
+}
+
+// Entries of the device view's prob table (cut nodes resolved to their parent's row) that the W == 3 lookup tables
+// take.  lut3: full-window value of every base triple, [strand][period][raw]; lutp: the same for the partial windows at
+// a sequence's ends
+// (Partial_Window_Prob, icm.cc:807-842), [strand][lim - 1][period][raw] -- window positions below lim are not available,
+// the walk stops at the first node that asks for one, so the entry does not depend on the raw code's bits at those
+// positions and the caller may index with whatever bases lie there.
+void gmg_w3_lut_index(const int16_t* mip, int N, int D, int* idx3, int* idxp) {
+  for (int i = 0; i < 384 + 768; i++) {
+    const bool full = i < 384;
+    const int k = full ? i : i - 384;
+    const int raw = k & 63, f = (k >> 6) % 3, lim = full ? 0 : 1 + (k / 192) % 2, strand = full ? k / 192 : k / 384;
+    // forward strand: window position k <-> base q0 + 2 - k; reverse strand: complement of base q0 + k
+    const unsigned ctx = strand == 0 ? (unsigned)(((raw >> 4) & 3) | (((raw >> 2) & 3) << 2) | ((raw & 3) << 4))
+                                     : (unsigned)((~raw) & 63);
+    int node = 0;
+    for (int l = 0; l < D; l++) {
+      const int pos = mip[(size_t)f * N + node];
+      if (pos < lim) break;
+      node = 4 * node + (int)((ctx >> (2 * pos)) & 3) + 1;
+    }
+    (full ? idx3[k] : idxp[k]) = (f * N + node) * 4 + (int)((ctx >> 4) & 3);
+  }
 }
 
 static int icm_upload(gmg_icm* m) {
@@ -364,36 +390,11 @@ static int icm_upload(gmg_icm* m) {
   m->dev.lut3 = NULL;
   m->dev.lutp = NULL;
   if (m->W == 3 && P == 3) {
-    std::vector<float> lut(384);
-    for (int i = 0; i < 384; i++) {
-      const int raw = i & 63, f = (i >> 6) % 3, strand = i / 192;
-      // forward strand: window position k <-> base q0 + 2 - k; reverse strand: complement of base q0 + k
-      const unsigned ctx = strand == 0 ? (unsigned)(((raw >> 4) & 3) | (((raw >> 2) & 3) << 2) | ((raw & 3) << 4))
-                                       : (unsigned)((~raw) & 63);
-      int node = 0;
-      for (int l = 0; l < D; l++) {
-        const int pos = m->mip[(size_t)f * N + node];
-        if (pos < 0) break;
-        node = 4 * node + (int)((ctx >> (2 * pos)) & 3) + 1;
-      }
-      lut[i] = eff[((size_t)f * N + node) * 4 + ((ctx >> 4) & 3)];
-    }
-    // the same for the partial windows at a sequence's ends (Partial_Window_Prob, icm.cc:807-842): window positions
-    // below lim are not available, the walk stops at the first node that asks for one -- so the entry does not depend
-    // on the raw code's bits at those positions and the caller may index with whatever bases lie there
-    std::vector<float> lutp(768);
-    for (int i = 0; i < 768; i++) {
-      const int raw = i & 63, f = (i >> 6) % 3, lim = 1 + (i / 192) % 2, strand = i / 384;
-      const unsigned ctx = strand == 0 ? (unsigned)(((raw >> 4) & 3) | (((raw >> 2) & 3) << 2) | ((raw & 3) << 4))
-                                       : (unsigned)((~raw) & 63);
-      int node = 0;
-      for (int l = 0; l < D; l++) {
-        const int pos = m->mip[(size_t)f * N + node];
-        if (pos < lim) break;
-        node = 4 * node + (int)((ctx >> (2 * pos)) & 3) + 1;
-      }
-      lutp[i] = eff[((size_t)f * N + node) * 4 + ((ctx >> 4) & 3)];
-    }
+    std::vector<int> idx3(384), idxp(768);
+    gmg_w3_lut_index(m->mip.data(), N, D, idx3.data(), idxp.data());
+    std::vector<float> lut(384), lutp(768);
+    for (int i = 0; i < 384; i++) lut[i] = eff[idx3[i]];
+    for (int i = 0; i < 768; i++) lutp[i] = eff[idxp[i]];
     GMG_CUDA(cudaMallocAsync(&m->d_lut3, 384 * sizeof(float), ctx->stream));
     GMG_CUDA(cudaMemcpyAsync(m->d_lut3, lut.data(), 384 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     GMG_CUDA(cudaMallocAsync(&m->d_lutp, 768 * sizeof(float), ctx->stream));
@@ -588,15 +589,14 @@ extern "C" void gmg_icm_free(gmg_icm* m) {
 // ICM in the reversed orientation the gene models use (icm.cc:65-216).  The table is tiny
 // (63 nodes) and is built once per run on the host in FP64 exactly like the reference
 // (its float accumulators round at every += ; glibc log), then uploaded.
-extern "C" int gmg_icm_build_indep(gmg_ctx* ctx, double gc, const char* const* stops, int n_stops, gmg_icm** out) {
-  GMG_CHECK(ctx && out, "gmg_icm_build_indep: NULL argument");
+void gmg_indep_tables(double gc, const char* const* stops, int n_stops, int16_t* mip, float* prob) {
   double base_prob[4], codon_prob[64];
   base_prob[1] = base_prob[2] = gc / 2.0;
   base_prob[0] = base_prob[3] = 0.5 - base_prob[1];
   for (int c = 0; c < 64; c++) codon_prob[c] = base_prob[(c >> 4) & 3] * base_prob[(c >> 2) & 3] * base_prob[c & 3];
   for (int i = 0; i < n_stops; i++) {
     // the model runs 3'->5', so the stop codon enters reversed
-    int j = base_code(stops[i][0]) + 4 * base_code(stops[i][1]) + 16 * base_code(stops[i][2]);
+    int j = gmg_base_code(stops[i][0]) + 4 * gmg_base_code(stops[i][1]) + 16 * gmg_base_code(stops[i][2]);
     codon_prob[j] = 1e-20;
   }
   double sum = 0.0;
@@ -604,9 +604,9 @@ extern "C" int gmg_icm_build_indep(gmg_ctx* ctx, double gc, const char* const* s
   for (int c = 0; c < 64; c++) codon_prob[c] /= sum;
 
   const int N = 21;
-  std::vector<int16_t> mip(3 * N, 0);
   std::vector<float> acc(3 * N * 4, 0.0f);
   static const int pw[3] = {1, 4, 16};
+  for (int i = 0; i < 3 * N; i++) mip[i] = 0;
   for (int f = 0; f < 3; f++) {
     const int d1 = pw[(3 - f) % 3], d2 = pw[(4 - f) % 3], d3 = pw[(5 - f) % 3];
     mip[f * N] = (f == 1) ? -1 : 1;
@@ -619,11 +619,17 @@ extern "C" int gmg_icm_build_indep(gmg_ctx* ctx, double gc, const char* const* s
       for (int c = 0; c < 64; c++) acc[(f * N + 5 + 4 * ((c / d2) % 4) + (c / d3) % 4) * 4 + (c / d1) % 4] += codon_prob[c];
     }
   }
-  std::vector<float> prob(3 * N * 4);
   for (int i = 0; i < 3 * N; i++) {
     double s = 0.0;
     for (int k = 0; k < 4; k++) s += acc[i * 4 + k];
     for (int k = 0; k < 4; k++) prob[i * 4 + k] = (float)(s == 0.0 ? 0.0 : log(acc[i * 4 + k] / s));
   }
-  return gmg_icm_from_tables(ctx, 3, 2, 3, mip.data(), prob.data(), out);
+}
+
+extern "C" int gmg_icm_build_indep(gmg_ctx* ctx, double gc, const char* const* stops, int n_stops, gmg_icm** out) {
+  GMG_CHECK(ctx && out, "gmg_icm_build_indep: NULL argument");
+  int16_t mip[3 * 21];
+  float prob[3 * 21 * 4];
+  gmg_indep_tables(gc, stops, n_stops, mip, prob);
+  return gmg_icm_from_tables(ctx, 3, 2, 3, mip, prob, out);
 }

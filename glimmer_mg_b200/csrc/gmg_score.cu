@@ -89,6 +89,15 @@ __device__ __forceinline__ float icm_str(const DevIcm& m, const uint64_t* __rest
                   lim > 0 ? lim : 0);
 }
 
+// gmg_score_orfs_mg_gc: the independent model of sequence s -- the shared view pointed at the sequence's record
+__device__ __forceinline__ DevIcm indep_of(const DevIcm& base, const IndepSeqs& X, int64_t s) {
+  DevIcm m = base;
+  m.prob = X.rec + (size_t)__ldg(X.model + s) * GMG_INDEP_REC;
+  m.lut3 = m.prob + 252;
+  m.lutp = m.prob + 636;
+  return m;
+}
+
 // 6-bit code (b0*16 + b1*4 + b2) of the forward-strand codon whose three bases start at global index g
 __device__ __forceinline__ int codon6_at(const uint64_t* __restrict__ words, int64_t g) {
   const int raw = (int)(gmg_extract32(words, g) & 63);  // b(g) | b(g+1) << 2 | b(g+2) << 4
@@ -1980,7 +1989,8 @@ __device__ __forceinline__ int low_bit_exp(double x) {
   return e - 1075 + (__ffsll((long long)mant) - 1);
 }
 
-__global__ void __launch_bounds__(128) k2_prefix(DevIcm indep, const uint64_t* __restrict__ words,
+template <bool kPS>
+__global__ void __launch_bounds__(128) k2_prefix(DevIcm indep_, IndepSeqs X, const uint64_t* __restrict__ words,
                                                  const int64_t* __restrict__ off, int64_t n_seq, int64_t total,
                                                  const float* __restrict__ planes, const uint32_t* __restrict__ bktidx,
                                                  CodonSets cs, DevParams P,
@@ -1990,6 +2000,9 @@ __global__ void __launch_bounds__(128) k2_prefix(DevIcm indep, const uint64_t* _
   const int64_t s = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (s >= n_seq) return;
+  DevIcm own;  // kPS: the sequence's own model; the single-model form reads the kernel parameter
+  if constexpr (kPS) own = indep_of(indep_, X, s);
+  const DevIcm& indep = kPS ? own : indep_;
   const int64_t a = off[s];
   const int L = (int)(off[s + 1] - a);
   if (L == 0) {
@@ -2162,7 +2175,8 @@ __device__ __forceinline__ void k2_cert_term(float v, unsigned& umin, float& asu
   asum += fabsf(v);
 }
 
-__global__ void __launch_bounds__(128) k2_prefix_lanes(DevIcm indep, const uint64_t* __restrict__ words,
+template <bool kPS>
+__global__ void __launch_bounds__(128) k2_prefix_lanes(DevIcm indep_, IndepSeqs X, const uint64_t* __restrict__ words,
                                                        const int64_t* __restrict__ off, int64_t n_seq, int64_t total,
                                                        const float* __restrict__ planes, const uint32_t* __restrict__ bktidx,
                                                        CodonSets cs, DevParams P, const uint8_t* __restrict__ qual_in,
@@ -2171,14 +2185,19 @@ __global__ void __launch_bounds__(128) k2_prefix_lanes(DevIcm indep, const uint6
                                                        uint8_t* __restrict__ cert) {
   constexpr unsigned FULL = 0xffffffffu;
   constexpr int NONE_LO = -0x40000000, NONE_HI = 0x40000000;
-  __shared__ float s_lut[384];
-  const bool have_lut = indep.lut3 != NULL;
-  if (have_lut)
-    for (int i = threadIdx.x; i < 384; i += blockDim.x) s_lut[i] = indep.lut3[i];
+  __shared__ float s_lut_sh[384];
+  const bool have_lut = indep_.lut3 != NULL;
+  if (!kPS && have_lut)
+    for (int i = threadIdx.x; i < 384; i += blockDim.x) s_lut_sh[i] = indep_.lut3[i];
   __syncthreads();
   const int64_t s = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (s >= n_seq) return;
+  // per-sequence models (gmg_score_orfs_mg_gc): the sequence's own table, read through L1
+  DevIcm own;  // kPS: the sequence's own model; the single-model form reads the kernel parameter
+  if constexpr (kPS) own = indep_of(indep_, X, s);
+  const DevIcm& indep = kPS ? own : indep_;
+  const float* const s_lut = kPS ? indep.lut3 : s_lut_sh;
   const int64_t a = off[s];
   const int L = (int)(off[s + 1] - a);
   if (L == 0) {
@@ -2767,11 +2786,11 @@ __device__ void mg_orf_starts(const MgSeq& S, const DevParams& P, const CodonSet
 // One thread per ORF: the recursion as the reference runs it (explicit stack).  Used for read sets without error
 // branches (plain glimmer-mg: one short linear walk per ORF) and, with kOnlyUncert, as the ORDERED path of the
 // sequences whose FP64 exactness certificate failed in K2 (their sums are re-formed in the reference's own order).
-template <bool kWrite>
+template <bool kWrite, bool kPS>
 __global__ void __launch_bounds__(128) k3_mg_starts(MgfBatch B, int64_t n_orfs, const gmg_orf* __restrict__ orfs,
                                                     const int32_t* __restrict__ orf_seq, CodonSets cs, DevParams P,
                                                     int only_uncert, const float* __restrict__ planes,
-                                                    const uint32_t* __restrict__ bktidx, DevIcm indep,
+                                                    const uint32_t* __restrict__ bktidx, DevIcm indep, IndepSeqs X,
                                                     int64_t* __restrict__ counts, const int64_t* __restrict__ start_off,
                                                     gmg_start* __restrict__ starts) {
   const int64_t oi = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -2795,11 +2814,17 @@ __global__ void __launch_bounds__(128) k3_mg_starts(MgfBatch B, int64_t n_orfs, 
   S.ordered = uncert ? 1 : 0;
   S.planes = planes;
   S.bktidx = bktidx;
-  S.indep = indep;
+  S.indep = kPS ? indep_of(indep, X, s) : indep;
   Emit e;
   e.out = kWrite ? starts + start_off[oi] : NULL;
   e.n = 0;
-  mg_orf_starts(S, P, cs, orfs[oi], oi, e);
+  if constexpr (kPS) {  // the sequence's own Ignore_Score_Len
+    DevParams Ps = P;
+    Ps.ignore_score_len = __ldg(X.isl + s);
+    mg_orf_starts(S, Ps, cs, orfs[oi], oi, e);
+  } else {
+    mg_orf_starts(S, P, cs, orfs[oi], oi, e);
+  }
   if (!kWrite) counts[oi] = e.n;
 }
 
@@ -2878,17 +2903,36 @@ __global__ void __launch_bounds__(256) k_mgf_e(MgfWork W) {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < W.n_orfs) mgf_pass_e(W, i);
 }
-__global__ void __launch_bounds__(128) k_mgf_w0(MgfBatch B, DevParams P, CodonSets cs, MgfWork W) {
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < W.n_orfs) mgf_write_0(B, P, cs, W, i);
+// the write passes set the records' long-ORF boost: with per-sequence ignore lengths (kPS) each thread takes its own
+__device__ __forceinline__ DevParams mgf_params_of(const DevParams& P, const IndepSeqs& X, int32_t s) {
+  DevParams Ps = P;
+  Ps.ignore_score_len = __ldg(X.isl + s);
+  return Ps;
 }
-__global__ void __launch_bounds__(128) k_mgf_w1(MgfBatch B, DevParams P, CodonSets cs, MgfWork W) {
+template <bool kPS>
+__global__ void __launch_bounds__(128) k_mgf_w0(MgfBatch B, DevParams P, CodonSets cs, MgfWork W, IndepSeqs X) {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < W.c1) mgf_write_1(B, P, cs, W, i);
+  if (i >= W.n_orfs) return;
+  if constexpr (kPS) mgf_write_0(B, mgf_params_of(P, X, W.orf_seq[i]), cs, W, i);
+  else mgf_write_0(B, P, cs, W, i);
 }
-__global__ void __launch_bounds__(128) k_mgf_w2(MgfBatch B, DevParams P, CodonSets cs, MgfWork W) {
+template <bool kPS>
+__global__ void __launch_bounds__(128) k_mgf_w1(MgfBatch B, DevParams P, CodonSets cs, MgfWork W, IndepSeqs X) {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < W.c2) mgf_write_2(B, P, cs, W, i);
+  if (i >= W.c1) return;
+  if constexpr (kPS) {
+    if (!W.call1[i].ok) return;  // (mgf_write_1's own test) the ORF of a call that does not exist is not set
+    mgf_write_1(B, mgf_params_of(P, X, W.orf_seq[W.call1[i].orf]), cs, W, i);
+  } else {
+    mgf_write_1(B, P, cs, W, i);
+  }
+}
+template <bool kPS>
+__global__ void __launch_bounds__(128) k_mgf_w2(MgfBatch B, DevParams P, CodonSets cs, MgfWork W, IndepSeqs X) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= W.c2) return;
+  if constexpr (kPS) mgf_write_2(B, mgf_params_of(P, X, W.orf_seq[W.call1[W.par2[i]].orf]), cs, W, i);
+  else mgf_write_2(B, P, cs, W, i);
 }
 
 // test hook (GMG_MG_FORCE_UNCERT=k): withdraw the certificate of every k-th sequence so that the ordered path runs
@@ -2976,17 +3020,18 @@ __global__ void __launch_bounds__(128) k3_mg_plain_count(MgfBatch B, DevParams P
   desc[o] = d;
 }
 
-__global__ void __launch_bounds__(128) k3_mg_plain(DevIcm indep, const float* __restrict__ planes,
-                                                   const uint32_t* __restrict__ bktidx, MgfBatch B, DevParams P, CodonSets cs,
+template <bool kPS>
+__global__ void __launch_bounds__(128) k3_mg_plain(DevIcm indep_, IndepSeqs X, const float* __restrict__ planes,
+                                                   const uint32_t* __restrict__ bktidx, MgfBatch B, DevParams P_, CodonSets cs,
                                                    const gmg_orf* __restrict__ orfs, const int32_t* __restrict__ orf_seq,
                                                    int64_t n_orfs, const int64_t* __restrict__ start_off,
                                                    gmg_start* __restrict__ starts, int exact_len,
                                                    unsigned long long* __restrict__ n_ordered, int slots, int lanes) {
   constexpr unsigned FULL = 0xffffffffu;
   extern __shared__ double s_pref_all[];  // [4 warps][slots]: sized for the batch's longest sequence (occupancy on short reads)
-  __shared__ float s_lut[384];
-  if (indep.lut3 != NULL)
-    for (int i = threadIdx.x; i < 384; i += blockDim.x) s_lut[i] = indep.lut3[i];
+  __shared__ float s_lut_sh[384];
+  if (!kPS && indep_.lut3 != NULL)
+    for (int i = threadIdx.x; i < 384; i += blockDim.x) s_lut_sh[i] = indep_.lut3[i];
   __syncthreads();
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int64_t o = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -2994,6 +3039,12 @@ __global__ void __launch_bounds__(128) k3_mg_plain(DevIcm indep, const float* __
   const int64_t so = start_off[o];
   if (start_off[o + 1] == so) return;
   const MgfSeq S = mgf_seq_of(B, orf_seq[o]);
+  // per-sequence models (gmg_score_orfs_mg_gc): the sequence's own table (read through L1) and ignore length
+  DevIcm own;  // kPS: the sequence's own model; the single-model form reads the kernel parameter
+  if constexpr (kPS) own = indep_of(indep_, X, orf_seq[o]);
+  const DevIcm& indep = kPS ? own : indep_;
+  const float* const s_lut = kPS ? indep.lut3 : s_lut_sh;
+  const DevParams P = kPS ? mgf_params_of(P_, X, orf_seq[o]) : P_;
   const gmg_orf orf = orfs[o];
   const bool fwd = orf.frame > 0;
   const int hi = fwd ? orf.stop_position - 1 : orf.stop_position + 3 + orf.orf_len;
@@ -3128,18 +3179,17 @@ __device__ __forceinline__ double mgl_codon_sum(const DevIcm& indep, const float
 // utilisation at 32 warps per SM): more ORFs in flight per warp at the same register count is what raises the throughput
 // on short reads (0.61 -> 0.49 ms per 31 Mbp with two; four: 0.50 -- the lane's serial share grows and its prefix
 // registers spill).
-template <int G, int K>
-__global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep, const float* __restrict__ planes,
+template <int G, int K, bool kPS>
+__global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep_, const float* __restrict__ planes,
                                                          const uint32_t* __restrict__ bktidx, MgfBatch B, DevParams P, Which4 which,
                                                          int64_t n_orfs, const int64_t* __restrict__ start_off,
                                                          gmg_start* __restrict__ starts, int exact_len,
                                                          unsigned long long* __restrict__ n_ordered,
-                                                         const PlainDesc* __restrict__ desc, int need_lo) {
+                                                         const PlainDesc* __restrict__ desc, int need_lo, IndepSeqs X) {
   constexpr unsigned FULL = 0xffffffffu;
   constexpr int HPW = 32 / G;                                       // ORFs per warp
   constexpr unsigned GMASK = G == 32 ? 0xffffffffu : ((1u << (G & 31)) - 1u);
   __shared__ double s_serial[4][HPW][G * K];  // codon-boundary prefixes of an ORF summed in serial order (rare)
-  const float* s_lut = indep.lut3;                // 1.5 KB: read through L1 (staging it cost 8 % of the kernel's instructions)
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int sub = lane % G, grp = lane / G, gshift = grp * G;
   // Persistent warps: a warp's life used to be five dependent load rounds (CSR -> ORF -> sequence offsets -> packed bases ->
@@ -3184,6 +3234,14 @@ __global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep, const 
   const int need = f.j_hi;  // terms j = 0 .. need - 1: score[j - 1] of the highest record position j_hi
   // this group's ORF is worked on here iff it has records and its length is this instance's
   const bool act = have && so1 != so && f.j_lo >= 3 && need > need_lo && need <= 3 * G * K;
+  // per-sequence models (gmg_score_orfs_mg_gc): the ORF's own table and ignore length
+  const int32_t xs = kPS && have ? __ldg(X.orf_seq + o) : 0;
+  DevIcm own;  // kPS: the sequence's own model; the single-model form reads the kernel parameter
+  if constexpr (kPS) own = indep_of(indep_, X, xs);
+  const DevIcm& indep = kPS ? own : indep_;
+  const float* s_lut = indep.lut3;  // 1.5 KB: read through L1 (staging it cost 8 % of the kernel's instructions)
+  DevParams Ps;  // kPS: the records' parameters with the sequence's ignore length (the single-model form reads P)
+  if constexpr (kPS) Ps = mgf_params_of(P, X, xs);
   MgfPlan pl;  // as mgf_plan leaves it
   pl.nT = (int)(d1.w >> 4);
   pl.state_after = (int)((d1.w >> 2) & 1u);
@@ -3270,11 +3328,11 @@ __global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep, const 
         const double sum = exact ? incl[k] : s_serial[wid][grp][c];
         const double sc = (sum - 0.0) + 0.0;
         if (trunc_rec) {
-          mgf_put(out + idx, P, j + 2, kp, sc, -1, 1, 1, 0, ep, et);
-          if (nr == 2) mgf_put(out + idx + 1, P, j + 2, kp, sc, which4_of(which, mgf_codon_at(B, S, f, fwd, j)), 0, 0, 0, ep, et);
+          mgf_put(out + idx, kPS ? Ps : P, j + 2, kp, sc, -1, 1, 1, 0, ep, et);
+          if (nr == 2) mgf_put(out + idx + 1, kPS ? Ps : P, j + 2, kp, sc, which4_of(which, mgf_codon_at(B, S, f, fwd, j)), 0, 0, 0, ep, et);
         } else {
           const int first = (pl.state_after && !seen_nonzero && (mnz & higher) == 0u) ? 1 : 0;
-          mgf_put(out + idx, P, j + 2, kp, sc, which4_of(which, mgf_codon_at(B, S, f, fwd, j)), 0, first, 0, ep, et);
+          mgf_put(out + idx, kPS ? Ps : P, j + 2, kp, sc, which4_of(which, mgf_codon_at(B, S, f, fwd, j)), 0, first, 0, ep, et);
         }
       }
       placed += __popc(m1) + __popc(m2);
@@ -3290,14 +3348,15 @@ __global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep, const 
 // gene - indep serially in the reference's own order (glimmer-mg.cc:577-586) and dropping each running sum into the
 // record that asks for it.  No scan, no certificate -- the order IS the reference's.  Measured slower than the warp form
 // on 100 bp reads (0.76 against 0.63 ms per 31 Mbp): kept as the simplest exact statement of the pass and for A/B runs.
-__global__ void __launch_bounds__(128) k3_mg_plain_serial(DevIcm indep, const float* __restrict__ planes,
-                                                          const uint32_t* __restrict__ bktidx, MgfBatch B, DevParams P,
+template <bool kPS>
+__global__ void __launch_bounds__(128) k3_mg_plain_serial(DevIcm indep_, IndepSeqs X, const float* __restrict__ planes,
+                                                          const uint32_t* __restrict__ bktidx, MgfBatch B, DevParams P_,
                                                           CodonSets cs, const gmg_orf* __restrict__ orfs,
                                                           const int32_t* __restrict__ orf_seq, int64_t n_orfs,
                                                           const int64_t* __restrict__ start_off, gmg_start* __restrict__ starts) {
-  __shared__ float s_lut[384];
-  if (indep.lut3 != NULL)
-    for (int i = threadIdx.x; i < 384; i += blockDim.x) s_lut[i] = indep.lut3[i];
+  __shared__ float s_lut_sh[384];
+  if (!kPS && indep_.lut3 != NULL)
+    for (int i = threadIdx.x; i < 384; i += blockDim.x) s_lut_sh[i] = indep_.lut3[i];
   __syncthreads();
   const int64_t o = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (o >= n_orfs) return;
@@ -3305,6 +3364,12 @@ __global__ void __launch_bounds__(128) k3_mg_plain_serial(DevIcm indep, const fl
   const int cnt = (int)(start_off[o + 1] - so);
   if (cnt == 0) return;
   const MgfSeq S = mgf_seq_of(B, orf_seq[o]);
+  // per-sequence models (gmg_score_orfs_mg_gc): the sequence's own table (read through L1) and ignore length
+  DevIcm own;  // kPS: the sequence's own model; the single-model form reads the kernel parameter
+  if constexpr (kPS) own = indep_of(indep_, X, orf_seq[o]);
+  const DevIcm& indep = kPS ? own : indep_;
+  const float* const s_lut = kPS ? indep.lut3 : s_lut_sh;
+  const DevParams P = kPS ? mgf_params_of(P_, X, orf_seq[o]) : P_;
   const gmg_orf orf = orfs[o];
   const bool fwd = orf.frame > 0;
   const int hi = fwd ? orf.stop_position - 1 : orf.stop_position + 3 + orf.orf_len;
@@ -3859,11 +3924,11 @@ extern "C" int gmg_score_orfs_g3(gmg_ctx* ctx, const gmg_icm* gene, const gmg_ic
   return 0;
 }
 
-extern "C" int gmg_score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const gmg_icm* indep, gmg_seqset* s,
-                                 const gmg_params* p, int64_t* n_starts) {
-  GMG_CHECK(ctx && gene && indep && s && p, "gmg_score_orfs_mg: NULL argument");
-  GMG_CHECK(gene->P == 3 && indep->P == 3, "glimmer-mg scoring needs periodicity-3 models");
-  if (gmg_icm_ready(gene) || gmg_icm_ready(indep)) return 1;
+// gmg_score_orfs_mg (kPS = false: one independent model) and gmg_score_orfs_mg_gc (kPS: the model and ignore length of
+// every sequence from X); the kernels take the same switch, so the single-model call compiles to the work it always did
+template <bool kPS>
+static int score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& indep, const IndepSeqs& X, gmg_seqset* s,
+                         const gmg_params* p, int64_t* n_starts) {
   CodonSets cs;
   DevParams dp;
   if (make_codon_sets(p, &cs, &dp)) return 1;
@@ -3928,8 +3993,8 @@ extern "C" int gmg_score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const gmg_ic
     const int plain_serial = getenv("GMG_PLAIN_SERIAL") ? atoi(getenv("GMG_PLAIN_SERIAL")) : 0;
     if (total_starts > 0 && plain_serial && exact_len >= 0) {
       if (gmg_prof_begin(ctx, GMG_PROF_K3)) return 1;
-      k3_mg_plain_serial<<<(unsigned)((s->n_orfs + 127) / 128), 128, 0, ctx->stream>>>(
-          indep->dev, planes, s->d_bktidx, B, dp, cs, s->d_orfs, s->d_orf_seq, s->n_orfs, s->d_start_off, s->d_starts);
+      k3_mg_plain_serial<kPS><<<(unsigned)((s->n_orfs + 127) / 128), 128, 0, ctx->stream>>>(
+          indep, X, planes, s->d_bktidx, B, dp, cs, s->d_orfs, s->d_orf_seq, s->n_orfs, s->d_start_off, s->d_starts);
       gmg_prof_end(ctx, GMG_PROF_K3);
       ctx->launches++;
       GMG_CUDA(cudaGetLastError());
@@ -3951,22 +4016,22 @@ extern "C" int gmg_score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const gmg_ic
         int done_to = -1;  // ORFs with need <= done_to are taken by an instance launched so far
         if (plain_lanes >= 3) {
           const int64_t need_ctas = (s->n_orfs * 8 + 127) / 128;
-          k3_mg_plain_lanes<8, 6><<<(unsigned)(need_ctas < lanes_cap ? need_ctas : lanes_cap), 128, 0, ctx->stream>>>(
-              indep->dev, planes, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to);
+          k3_mg_plain_lanes<8, 6, kPS><<<(unsigned)(need_ctas < lanes_cap ? need_ctas : lanes_cap), 128, 0, ctx->stream>>>(
+              indep, planes, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to, X);
           ctx->launches++;
           done_to = 3 * 8 * 6;
         }
         if (plain_lanes >= 2 && s->max_len > done_to) {
           const int64_t need_ctas = (s->n_orfs * 16 + 127) / 128;
-          k3_mg_plain_lanes<16, 4><<<(unsigned)(need_ctas < lanes_cap ? need_ctas : lanes_cap), 128, 0, ctx->stream>>>(
-              indep->dev, planes, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to);
+          k3_mg_plain_lanes<16, 4, kPS><<<(unsigned)(need_ctas < lanes_cap ? need_ctas : lanes_cap), 128, 0, ctx->stream>>>(
+              indep, planes, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to, X);
           ctx->launches++;
           done_to = 3 * 16 * 4;
         }
         if (s->max_len > done_to) {
           const int64_t need_ctas = (s->n_orfs * 32 + 127) / 128;
-          k3_mg_plain_lanes<32, 4><<<(unsigned)(need_ctas < lanes_cap ? need_ctas : lanes_cap), 128, 0, ctx->stream>>>(
-              indep->dev, planes, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to);
+          k3_mg_plain_lanes<32, 4, kPS><<<(unsigned)(need_ctas < lanes_cap ? need_ctas : lanes_cap), 128, 0, ctx->stream>>>(
+              indep, planes, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to, X);
           ctx->launches++;
         }
       }
@@ -3974,8 +4039,8 @@ extern "C" int gmg_score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const gmg_ic
       const bool all_taken = plain_lanes && s->max_len <= 96 * 4 && p->min_gene_len >= 6;
       if (!all_taken) {
         const int slots = (int)(s->max_len / 3 + 4);
-        k3_mg_plain<<<(unsigned)((s->n_orfs * 32 + 127) / 128), 128, (size_t)4 * slots * sizeof(double), ctx->stream>>>(
-            indep->dev, planes, s->d_bktidx, B, dp, cs, s->d_orfs, s->d_orf_seq, s->n_orfs, s->d_start_off, s->d_starts, exact_len,
+        k3_mg_plain<kPS><<<(unsigned)((s->n_orfs * 32 + 127) / 128), 128, (size_t)4 * slots * sizeof(double), ctx->stream>>>(
+            indep, X, planes, s->d_bktidx, B, dp, cs, s->d_orfs, s->d_orf_seq, s->n_orfs, s->d_start_off, s->d_starts, exact_len,
             (unsigned long long*)(counts + s->n_orfs + 1), slots, plain_lanes);
         ctx->launches++;
       }
@@ -4019,11 +4084,11 @@ extern "C" int gmg_score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const gmg_ic
   if (gmg_prof_begin(ctx, GMG_PROF_K2)) return 1;
   static const int k2_mode = getenv("GMG_K2_MODE") ? atoi(getenv("GMG_K2_MODE")) : 0;  // 0 lane-serial tiles, 1 one position per lane
   if (k2_mode == 0)
-    k2_prefix_lanes<<<g2, 128, 0, ctx->stream>>>(indep->dev, s->d_words, s->d_off, s->n, s->total, planes, s->d_bktidx, cs,
+    k2_prefix_lanes<kPS><<<g2, 128, 0, ctx->stream>>>(indep, X, s->d_words, s->d_off, s->n, s->total, planes, s->d_bktidx, cs,
                                                  dp, p->have_quality_file ? s->d_qual : NULL, (double*)d_cum, fwd_prev,
                                                  rev_next, need_qual ? (uint8_t*)d_qual : NULL, cert);
   else
-    k2_prefix<<<g2, 128, 0, ctx->stream>>>(indep->dev, s->d_words, s->d_off, s->n, s->total, planes, s->d_bktidx, cs, dp,
+    k2_prefix<kPS><<<g2, 128, 0, ctx->stream>>>(indep, X, s->d_words, s->d_off, s->n, s->total, planes, s->d_bktidx, cs, dp,
                                            p->have_quality_file ? s->d_qual : NULL, (double*)d_cum, fwd_prev, rev_next,
                                            need_qual ? (uint8_t*)d_qual : NULL, cert);
   gmg_prof_end(ctx, GMG_PROF_K2);
@@ -4158,12 +4223,12 @@ extern "C" int gmg_score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const gmg_ic
     k_mgf_e<<<(no + 255) / 256, 256, 0, ctx->stream>>>(W);
     ctx->launches++;
     // sequences without a certificate: counted (and later written) in the reference's serial order
-    k3_mg_starts<false><<<g3, 128, 0, ctx->stream>>>(B, s->n_orfs, s->d_orfs, s->d_orf_seq, cs, dp, 1, planes, s->d_bktidx,
-                                                     indep->dev, counts, NULL, NULL);
+    k3_mg_starts<false, kPS><<<g3, 128, 0, ctx->stream>>>(B, s->n_orfs, s->d_orfs, s->d_orf_seq, cs, dp, 1, planes, s->d_bktidx,
+                                                     indep, X, counts, NULL, NULL);
     ctx->launches++;
   } else {
-    k3_mg_starts<false><<<g3, 128, 0, ctx->stream>>>(B, s->n_orfs, s->d_orfs, s->d_orf_seq, cs, dp, 0, planes, s->d_bktidx,
-                                                     indep->dev, counts, NULL, NULL);
+    k3_mg_starts<false, kPS><<<g3, 128, 0, ctx->stream>>>(B, s->n_orfs, s->d_orfs, s->d_orf_seq, cs, dp, 0, planes, s->d_bktidx,
+                                                     indep, X, counts, NULL, NULL);
     ctx->launches++;
   }
   gmg_prof_end(ctx, GMG_PROF_K3);
@@ -4186,24 +4251,24 @@ extern "C" int gmg_score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const gmg_ic
     if (k3mg_mode == 0) {
       W.start_off = s->d_start_off;
       W.starts = s->d_starts;
-      k_mgf_w0<<<g3, 128, 0, ctx->stream>>>(B, dp, cs, W);
+      k_mgf_w0<kPS><<<g3, 128, 0, ctx->stream>>>(B, dp, cs, W, X);
       ctx->launches++;
       if (W.c1) {
-        k_mgf_w1<<<(W.c1 + 127) / 128, 128, 0, ctx->stream>>>(B, dp, cs, W);
+        k_mgf_w1<kPS><<<(W.c1 + 127) / 128, 128, 0, ctx->stream>>>(B, dp, cs, W, X);
         ctx->launches++;
       }
       if (W.c2) {
-        k_mgf_w2<<<(W.c2 + 127) / 128, 128, 0, ctx->stream>>>(B, dp, cs, W);
+        k_mgf_w2<kPS><<<(W.c2 + 127) / 128, 128, 0, ctx->stream>>>(B, dp, cs, W, X);
         ctx->launches++;
       }
       if (bad > 0) {
-        k3_mg_starts<true><<<g3, 128, 0, ctx->stream>>>(B, s->n_orfs, s->d_orfs, s->d_orf_seq, cs, dp, 1, planes, s->d_bktidx,
-                                                        indep->dev, NULL, s->d_start_off, s->d_starts);
+        k3_mg_starts<true, kPS><<<g3, 128, 0, ctx->stream>>>(B, s->n_orfs, s->d_orfs, s->d_orf_seq, cs, dp, 1, planes, s->d_bktidx,
+                                                        indep, X, NULL, s->d_start_off, s->d_starts);
         ctx->launches++;
       }
     } else {
-      k3_mg_starts<true><<<g3, 128, 0, ctx->stream>>>(B, s->n_orfs, s->d_orfs, s->d_orf_seq, cs, dp, 0, planes, s->d_bktidx,
-                                                      indep->dev, NULL, s->d_start_off, s->d_starts);
+      k3_mg_starts<true, kPS><<<g3, 128, 0, ctx->stream>>>(B, s->n_orfs, s->d_orfs, s->d_orf_seq, cs, dp, 0, planes, s->d_bktidx,
+                                                      indep, X, NULL, s->d_start_off, s->d_starts);
       ctx->launches++;
     }
   }
@@ -4212,6 +4277,82 @@ extern "C" int gmg_score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const gmg_ic
   s->n_starts = total_starts;
   if (n_starts) *n_starts = total_starts;
   return 0;
+}
+
+extern "C" int gmg_score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const gmg_icm* indep, gmg_seqset* s,
+                                 const gmg_params* p, int64_t* n_starts) {
+  GMG_CHECK(ctx && gene && indep && s && p, "gmg_score_orfs_mg: NULL argument");
+  GMG_CHECK(gene->P == 3 && indep->P == 3, "glimmer-mg scoring needs periodicity-3 models");
+  if (gmg_icm_ready(gene) || gmg_icm_ready(indep)) return 1;
+  IndepSeqs none;
+  memset(&none, 0, sizeof none);
+  return score_orfs_mg<false>(ctx, gene, indep->dev, none, s, p, n_starts);
+}
+
+// glimmer-mg -c: every read scored with the independent model of its own GC fraction (and, optionally, its own
+// Ignore_Score_Len).  The GC values are deduplicated by bit pattern in one host pass, one model record per distinct value
+// is built on the device (gmg_indep_build), and the kernels of gmg_score_orfs_mg look up the record of each ORF's sequence.
+extern "C" int gmg_score_orfs_mg_gc(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqset* s, const double* h_gc,
+                                    const int32_t* h_isl, const gmg_params* p, int64_t* n_starts) {
+  GMG_CHECK(ctx && gene && s && p && (h_gc || s->n == 0), "gmg_score_orfs_mg_gc: NULL argument");
+  GMG_CHECK(gene->P == 3, "glimmer-mg scoring needs periodicity-3 models");
+  GMG_CHECK(p->n_stop >= 0 && p->n_stop <= 8, "gmg_score_orfs_mg_gc: %d stop codons", p->n_stop);
+  const int64_t n = s->n;
+  for (int64_t i = 0; i < n; i++) {
+    GMG_CHECK(h_gc[i] >= 0.0 && h_gc[i] <= 1.0, "gmg_score_orfs_mg_gc: sequence %lld: GC fraction %g is not in [0, 1]",
+              (long long)i, h_gc[i]);
+    GMG_CHECK(!h_isl || h_isl[i] >= 0, "gmg_score_orfs_mg_gc: sequence %lld: negative ignore_score_len %d", (long long)i,
+              h_isl ? h_isl[i] : 0);
+  }
+  if (gmg_icm_ready(gene)) return 1;
+  // inputs in one page-locked block: [distinct GC values][model of every sequence][ignore length of every sequence]
+  const size_t gc_bytes = (size_t)(n > 0 ? n : 1) * sizeof(double), seq_bytes = (size_t)(n > 0 ? n : 1) * sizeof(int32_t);
+  if (gmg_host_stage(ctx, gc_bytes + 2 * seq_bytes, 0)) return 1;
+  double* h_uniq = (double*)ctx->h_stage;
+  int32_t* h_model = (int32_t*)((char*)ctx->h_stage + gc_bytes);
+  int32_t* h_isl_all = h_model + (n > 0 ? n : 1);
+  // dedupe by bit pattern: open addressing, table of at least 2 n slots
+  int64_t n_models = 0;
+  {
+    int bits = 4;
+    while ((int64_t(1) << bits) < 2 * n) bits++;
+    const uint64_t mask = (uint64_t(1) << bits) - 1;
+    std::vector<int32_t> slot((size_t)mask + 1, -1);
+    for (int64_t i = 0; i < n; i++) {
+      uint64_t key;
+      memcpy(&key, &h_gc[i], sizeof key);
+      uint64_t h = (key * 0x9E3779B97F4A7C15ull) >> (64 - bits);
+      for (;; h = (h + 1) & mask) {
+        const int32_t m = slot[h];
+        if (m < 0) {
+          slot[h] = (int32_t)n_models;
+          h_uniq[n_models] = h_gc[i];
+          h_model[i] = (int32_t)n_models++;
+          break;
+        }
+        uint64_t km;
+        memcpy(&km, &h_uniq[m], sizeof km);
+        if (km == key) {
+          h_model[i] = m;
+          break;
+        }
+      }
+      h_isl_all[i] = h_isl ? h_isl[i] : p->ignore_score_len;
+    }
+  }
+  void* d_in;
+  if (gmg_scratch(ctx, SCR_INDEP_IN, gc_bytes + 2 * seq_bytes, &d_in)) return 1;
+  GMG_CUDA(cudaMemcpyAsync(d_in, ctx->h_stage, (size_t)n_models * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  GMG_CUDA(cudaMemcpyAsync((char*)d_in + gc_bytes, h_model, 2 * seq_bytes, cudaMemcpyHostToDevice, ctx->stream));
+  float* d_rec;
+  DevIcm base;
+  if (gmg_indep_build(ctx, (const double*)d_in, h_uniq, n_models, p, &d_rec, &base)) return 1;
+  IndepSeqs X;
+  X.rec = d_rec;
+  X.model = (const int32_t*)((char*)d_in + gc_bytes);
+  X.isl = X.model + (n > 0 ? n : 1);
+  X.orf_seq = s->d_orf_seq;
+  return score_orfs_mg<true>(ctx, gene, base, X, s, p, n_starts);
 }
 
 extern "C" int gmg_reduce_starts_mg(gmg_ctx* ctx, gmg_seqset* s, const gmg_params* p, const gmg_event_model* em,

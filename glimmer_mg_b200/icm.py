@@ -117,6 +117,8 @@ def lib():
         "gmg_set_orfs": (i32, [vp, vp, vp, vp]),
         "gmg_score_orfs_g3": (i32, [vp, vp, vp, vp, P(_Params), P(i64)]),
         "gmg_score_orfs_mg": (i32, [vp, vp, vp, vp, P(_Params), P(i64)]),
+        "gmg_score_orfs_mg_gc": (i32, [vp, vp, vp, vp, vp, P(_Params), P(i64)]),
+        "gmg_ctx_indep_flagged": (i64, [vp]),
         "gmg_get_starts": (i32, [vp, vp, vp, vp]),
         "gmg_all_frame_scores": (i32, [vp, vp, vp, i64, vp, vp, vp, vp]),
         "gmg_reduce_starts_mg": (i32, [vp, vp, P(_Params), P(_EventModel), P(i64), P(i64)]),
@@ -229,6 +231,11 @@ class Context:
     @property
     def launches(self):
         return int(lib().gmg_ctx_launch_count(self.h))
+
+    @property
+    def indep_flagged(self):
+        """model entries of the last score_orfs_mg_gc call whose logarithm the host recomputed (diagnostic)"""
+        return int(lib().gmg_ctx_indep_flagged(self.h))
 
     PROF = {"k1": 0, "k2": 1, "k3": 2, "k4": 3, "orf": 4, "pack": 5, "fs": 6}
 
@@ -457,6 +464,24 @@ class SeqSet:
     def score_orfs_mg(self, gene, indep, params):
         n = C.c_int64()
         _check(lib().gmg_score_orfs_mg(self.ctx.h, gene.h, indep.h, self.h, C.byref(params.c), C.byref(n)))
+        self.n_starts = n.value
+        return self.n_starts
+
+    def score_orfs_mg_gc(self, gene, gc, params, ignore_score_len=None):
+        """score_orfs_mg with the independent model of every sequence's own GC fraction (glimmer-mg -c): sequence i is
+        scored with Build_Indep_WO_Stops(gc[i], params' stop codons) and, when given, ignore_score_len[i] in place of
+        params.ignore_score_len.  Bit-identical to scoring each sequence alone that way."""
+        gc = np.ascontiguousarray(gc, np.float64)
+        if gc.shape != (self.n,):
+            raise GmgError(f"score_orfs_mg_gc: {gc.size} GC values for {self.n} sequences")
+        isl = None
+        if ignore_score_len is not None:
+            isl = np.ascontiguousarray(ignore_score_len, np.int32)
+            if isl.shape != (self.n,):
+                raise GmgError(f"score_orfs_mg_gc: {isl.size} ignore lengths for {self.n} sequences")
+        n = C.c_int64()
+        _check(lib().gmg_score_orfs_mg_gc(self.ctx.h, gene.h, self.h, gc.ctypes.data,
+                                          isl.ctypes.data if isl is not None else None, C.byref(params.c), C.byref(n)))
         self.n_starts = n.value
         return self.n_starts
 

@@ -258,6 +258,20 @@ int gmg_all_frame_scores(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqset* s, int64
  * Score_Orf_Starts / Score_Indels / Pass_Stop_Penalty recursion for every ORF. */
 int gmg_score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const gmg_icm* indep, gmg_seqset* s,
                       const gmg_params* p, int64_t* n_starts);
+/* gmg_score_orfs_mg with a per-sequence independent model (glimmer-mg -c, which builds the model from each read's GC
+ * fraction): sequence i is scored as gmg_score_orfs_mg scores it in a set of its own with
+ * indep = Build_Indep_WO_Stops(h_gc[i], p's stop codons) and p->ignore_score_len replaced by h_isl[i] (h_isl = NULL:
+ * p->ignore_score_len for all).  Results (raw start lists, gmg_get_starts / gmg_get_orf_starts / gmg_reduce_starts_mg
+ * afterwards) are bit-identical to that.  Needs ORFs (gmg_find_orfs / gmg_set_orfs); every mode of gmg_score_orfs_mg.
+ * The models are built on the device, one per distinct GC value (exact bit pattern); the launch count does not depend
+ * on the number of sequences or of distinct values.  Rejected before any device work, with a message naming the first
+ * bad sequence: a GC value that is NaN or outside [0, 1], a negative ignore length; the context stays usable. */
+int gmg_score_orfs_mg_gc(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqset* s, const double* h_gc, const int32_t* h_isl,
+                         const gmg_params* p, int64_t* n_starts);
+/* The models of gmg_score_orfs_mg_gc take their logarithms on the device where the result provably rounds to the float
+ * that glibc's log gives; the other entries are recomputed on the host.  This returns how many entries the last
+ * gmg_score_orfs_mg_gc call on the context recomputed (diagnostic; results are exact either way). */
+int64_t gmg_ctx_indep_flagged(const gmg_ctx* ctx);
 /* ---- start-list reduction (the consumer side of Score_Orfs_Errors, glimmer-mg.cc:1656-1684, and the per-position
  * arg-max of Add_Events_Fwd / Add_Events_Rev, glimmer_base.cc:65-128, 175-235) ------------------------------------
  * With -i nearly every raw start record is dominated by another candidate at the same start position; the
