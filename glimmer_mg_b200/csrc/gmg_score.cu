@@ -162,6 +162,10 @@ static int make_codon_sets(const gmg_params* p, CodonSets* cs, DevParams* dp) {
     if (cs->stop_mask >> rc & 1) cs->raw_mask[3] |= 1ull << raw;
   }
   GMG_CHECK(p->indel_max >= 0 && p->indel_max <= 2, "indel_max %d unsupported (0..2)", p->indel_max);
+  // qualities live in a uint8 plane (file values clamped to 255): Clean_Quality_454's threshold + 1 must fit it, and a
+  // gate test q <= threshold must not open for values the clamp brought down to 255
+  GMG_CHECK(p->indel_quality_threshold <= 254, "indel_quality_threshold %d unsupported (at most 254)",
+            p->indel_quality_threshold);
   dp->min_gene_len = p->min_gene_len;
   dp->allow_truncated = p->allow_truncated;
   dp->allow_indels = p->allow_indels;
@@ -2065,17 +2069,20 @@ __global__ void __launch_bounds__(128) k2_prefix(DevIcm indep_, IndepSeqs X, con
         int nv = __shfl_sync(0xffffffffu, prevv, l < 0 ? 0 : l);
         if (l >= 0) last_stop[c] = nv;
       }
-      // Set_Quality_454 (glimmer-mg.cc:1865-1906): last base of a homopolymer run of length r gets
-      // 31 - 5*min(r,5), every other base 31.  Clean_Quality_454 (:519-546) when a quality file is given.
+      // Without a quality file, Set_Quality_454 (glimmer-mg.cc:1865-1906): last base of a homopolymer run of length r
+      // gets 31 - 5*min(r,5), every other base 31.  With one, the file's values (already clamped to 0..255), cleaned by
+      // Clean_Quality_454 (:519-546) under -i only, as main() does (:385-392): under -s alone they reach
+      // Pass_Stop_Penalty as read.
       if (in && qual) {
         const int b = gmg_base_at(words, a + q);
         const bool last_of_run = (q == L - 1) || (gmg_base_at(words, a + q + 1) != b);
         int qv;
         if (qual_in) {
           qv = qual_in[a + q];
-          if (qv <= 0) qv = 1;
-          if (!last_of_run && qv < P.indel_q_thresh + 1) qv = P.indel_q_thresh + 1;
-          qv = min(qv, 255);
+          if (P.allow_indels) {
+            if (qv <= 0) qv = 1;
+            if (!last_of_run && qv < P.indel_q_thresh + 1) qv = P.indel_q_thresh + 1;
+          }
         } else if (!last_of_run) {
           qv = 31;
         } else {
@@ -2280,11 +2287,12 @@ __global__ void __launch_bounds__(128) k2_prefix_lanes(DevIcm indep_, IndepSeqs 
             const int b = (int)bs;
             const bool last_of_run = (q == L - 1) || ((int)((win >> (2 * (i + 5))) & 3) != b);
             int qv;
-            if (qual_in) {
+            if (qual_in) {  // the file's values; Clean_Quality_454 under -i only (see k2_prefix)
               qv = qual_in[a + q];
-              if (qv <= 0) qv = 1;
-              if (!last_of_run && qv < P.indel_q_thresh + 1) qv = P.indel_q_thresh + 1;
-              qv = min(qv, 255);
+              if (P.allow_indels) {
+                if (qv <= 0) qv = 1;
+                if (!last_of_run && qv < P.indel_q_thresh + 1) qv = P.indel_q_thresh + 1;
+              }
             } else if (!last_of_run) {
               qv = 31;
             } else {

@@ -63,11 +63,12 @@ typedef struct {
   int32_t allow_indels;            /* glimmer-mg -i */
   int32_t allow_subs;              /* glimmer-mg -s */
   int32_t min_indel_orf_len;       /* Min_Indel_ORF_Len, 15 */
-  int32_t indel_quality_threshold; /* 18 */
+  int32_t indel_quality_threshold; /* 18 (<= 254 supported: threshold + 1 must fit the uint8 quality plane) */
   int32_t indel_max;               /* 2 (<= 2 supported) */
   int32_t ignore_score_len;        /* Ignore_Score_Len; INT32_MAX = off */
   double indel_suffix_score_threshold; /* -12 */
-  int32_t have_quality_file;       /* Quality_File_Name != NULL (changes Pass_Stop_Penalty) */
+  int32_t have_quality_file;       /* Quality_File_Name != NULL (changes Pass_Stop_Penalty); the set's qualities are
+                                      cleaned (Clean_Quality_454) under allow_indels only, as glimmer-mg does */
   int32_t n_start, n_stop;
   char start_codon[8][4];          /* lower-case, e.g. "atg" */
   char stop_codon[8][4];

@@ -5,7 +5,11 @@
 // plain loops with std exclusive scans, and the start lists must equal orc_mg_score_orfs byte for byte.
 // This is a debugging aid for kernel logic in a container without a GPU; the product never runs this way.
 //
-//   mgflat_check <model.icm> <reads.fa> <n_reads> <allow_indels> <allow_subs> <indel_max> [truncate_len]
+// With a quality seed the reads carry seeded Phred values as from a quality file (have_quality_file = 1): the oracle
+// gets them as they are, the quality plane is built by glimmer-mg's rule (Clean_Quality_454 under -i only) and the
+// Pass_Stop_Penalty of every root call is filled in as k_mg_sub_pstop + the host log fill it.
+//
+//   mgflat_check <model.icm> <reads.fa> <n_reads> <allow_indels> <allow_subs> <indel_max> [truncate_len [qual_seed]]
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -50,6 +54,21 @@ static void make_sets(const orc_params& p, CodonSets* cs) {
   }
 }
 
+// seeded Phred values: half of them from the edges of the quality tables (0, the indel threshold 18 and its
+// neighbours, 1 - 10^(-q/10) rounding to 1 from 163 on, 255), the rest uniform in 0..40 (splitmix64)
+static std::vector<int> seeded_quality(uint64_t& st, int L) {
+  static const int edge[12] = {0, 1, 2, 17, 18, 19, 20, 40, 93, 162, 163, 255};
+  std::vector<int> q((size_t)L);
+  for (int i = 0; i < L; i++) {
+    uint64_t z = (st += 0x9E3779B97F4A7C15ull);
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    z ^= z >> 31;
+    q[i] = (z & 1) ? edge[(z >> 8) % 12] : (int)((z >> 8) % 41);
+  }
+  return q;
+}
+
 static std::vector<std::string> read_fasta(const char* path, int n_max) {
   std::vector<std::string> out;
   FILE* fp = fopen(path, "r");
@@ -85,6 +104,8 @@ int main(int argc, char** argv) {
   }
   orc_icm* gene = orc_icm_read(argv[1]);
   const int trunc_len = argc > 7 ? atoi(argv[7]) : 0;
+  const bool have_qual = argc > 8;
+  uint64_t qual_state = have_qual ? strtoull(argv[8], NULL, 10) : 0;
   std::vector<std::string> reads = read_fasta(argv[2], atoi(argv[3]));
   if (trunc_len > 0)
     for (auto& r : reads)
@@ -126,7 +147,8 @@ int main(int argc, char** argv) {
   P.indel_q_thresh = op.indel_quality_threshold;
   P.indel_max = op.indel_max;
   P.ignore_score_len = op.ignore_score_len;
-  P.have_quality_file = 0;
+  P.have_quality_file = have_qual ? 1 : 0;
+  op.have_quality_file = P.have_quality_file;
   P.indel_suffix_thresh = op.indel_suffix_score_threshold;
 
   // codon bitmaps
@@ -149,6 +171,8 @@ int main(int argc, char** argv) {
   std::vector<double> cum((size_t)6 * total, 0.0);
   std::vector<int32_t> fwd_prev(total), rev_next(total);
   std::vector<uint8_t> qual(total, 31);
+  std::vector<std::vector<int>> raw_qual((size_t)n);
+  long n_zero = 0, n_high = 0;
   for (int64_t i = 0; i < n; i++) {
     const int L = (int)reads[i].size();
     if (L == 0) continue;
@@ -169,7 +193,17 @@ int main(int argc, char** argv) {
     }
     orc_save_prev_stops(s, L, &op, fwd_prev.data() + off[i], rev_next.data() + off[i]);
     std::vector<int> qv(L);
-    orc_set_quality_454(s, L, qv.data());
+    if (have_qual) {
+      raw_qual[i] = seeded_quality(qual_state, L);
+      qv = raw_qual[i];
+      if (op.allow_indels) orc_clean_quality_454(s, L, qv.data(), op.indel_quality_threshold);
+      for (int q = 0; q < L; q++) {
+        n_zero += qv[q] == 0;
+        n_high += qv[q] >= 163;
+      }
+    } else {
+      orc_set_quality_454(s, L, qv.data());
+    }
     for (int q = 0; q < L; q++) qual[off[i] + q] = (uint8_t)qv[q];
   }
   const int64_t nblk = total / 32 + 2;
@@ -207,7 +241,8 @@ int main(int argc, char** argv) {
     const int no = orc_find_orfs(reads[i].c_str(), L, &op, &o);
     std::vector<int> so(no + 1, 0);
     orc_start* st = NULL;
-    const int ns = orc_mg_score_orfs(gene, indep, reads[i].c_str(), L, NULL, &op, o, no, so.data(), &st);
+    const int ns = orc_mg_score_orfs(gene, indep, reads[i].c_str(), L, have_qual ? raw_qual[i].data() : NULL, &op, o, no, so.data(),
+                                     &st);
     for (int k = 0; k < no; k++) {
       gmg_orf g;
       g.frame = o[k].frame;
@@ -240,6 +275,20 @@ int main(int argc, char** argv) {
   B.gate_pos = gate_pos.data();
   B.tables = tables.data();
   B.sub_pen = NULL;
+  // Pass_Stop_Penalty of every root call with a quality file: p_stop as k_mg_sub_pstop forms it, the log as the host takes it
+  std::vector<double> sub_pen;
+  if (have_qual && op.allow_subs) {
+    sub_pen.resize(n_orfs);
+    for (uint32_t o = 0; o < n_orfs; o++) {
+      const MgfSeq S = mgf_seq_of(B, orf_seq[o]);
+      const bool fwd = orfs[o].frame > 0;
+      int lo, hi;
+      mgf_open(B, S, fwd, fwd ? orfs[o].stop_position - 1 : orfs[o].stop_position + 3, &lo, &hi);
+      const double ps = mgf_stop_pstop(B, S, fwd, lo, hi);
+      sub_pen[o] = log(1.0 - ps) - log(ps);
+    }
+    B.sub_pen = sub_pen.data();
+  }
 
   MgfWork W;
   memset(&W, 0, sizeof W);
@@ -382,7 +431,13 @@ int main(int argc, char** argv) {
       }
     }
   }
-  printf("%s: %lld reads, %u ORFs, %u level-1 candidates, %u level-2 candidates, %lld starts (oracle %zu)\n", bad ? "MISMATCH" : "OK",
-         (long long)n, n_orfs, W.c1, W.c2, (long long)n_starts, want.size());
+  long n_inf = 0, n_ninf = 0;
+  for (const orc_start& w : want) {
+    n_inf += isinf(w.score) && w.score > 0;
+    n_ninf += isinf(w.score) && w.score < 0;
+  }
+  printf("%s: %lld reads, %u ORFs, %u level-1 candidates, %u level-2 candidates, %lld starts (oracle %zu); qualities 0: %ld, "
+         ">= 163: %ld; scores +inf: %ld, -inf: %ld\n",
+         bad ? "MISMATCH" : "OK", (long long)n, n_orfs, W.c1, W.c2, (long long)n_starts, want.size(), n_zero, n_high, n_inf, n_ninf);
   return bad ? 1 : 0;
 }

@@ -165,10 +165,6 @@ def test_golden_reads(gm, ctx, gene, phred_offset, eol):
         (w_orfs, w_ooff), (w_st, w_so), _, _ = raw_starts(gm, want, gene, flags)
         assert orfs.tobytes() == w_orfs.tobytes() and (ooff == w_ooff).all()
         assert st.tobytes() == w_st.tobytes() and (so == w_so).all()
-        if flags.get("allow_subs"):
-            # -s with a quality file: the oracle port's start scores differ from the device's for some ORFs of these
-            # reads on the FASTA + quality-file route as well, so the comparison above is this mode's check
-            continue
         # the first 200 reads against the oracle port, with the parsed qualities
         op = O.params(True, have_quality_file=1, **flags)
         op.ignore_score_len = isl

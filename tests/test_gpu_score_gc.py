@@ -169,13 +169,15 @@ def check_against_oracle(gm, ctx, gene, ogene, reads, qual, gc, flags, with_qual
     return flagged
 
 
-# the oracle port's -s scores with a quality file differ from the device's (and from the quality-file route) for some ORFs,
-# an existing disagreement of the port: -s is held to the oracle without one
-ORACLE_CASES = [({}, False), ({}, True), ({"allow_indels": 1}, False), ({"allow_indels": 1}, True), ({"allow_subs": 1}, False)]
+ORACLE_CASES = [({}, False), ({}, True), ({"allow_indels": 1}, False), ({"allow_indels": 1}, True), ({"allow_subs": 1}, False),
+                ({"allow_subs": 1}, True)]
+ORACLE_IDS = ["plain", "plain-qual", "indels", "indels-qual", "subs", "subs-qual"]
+ROUTE_CASES = [({}, False), ({"allow_indels": 1}, True), ({"allow_subs": 1}, False), ({"allow_subs": 1}, True)]
+ROUTE_IDS = ["plain", "indels-qual", "subs", "subs-qual"]
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("flags,with_qual", ORACLE_CASES, ids=["plain", "plain-qual", "indels", "indels-qual", "subs"])
+@pytest.mark.parametrize("flags,with_qual", ORACLE_CASES, ids=ORACLE_IDS)
 @pytest.mark.parametrize("per_read_isl", [True, False], ids=["isl", "no-isl"])
 def test_distinct_gc_golden(gm, ctx, gene, ogene, golden, flags, with_qual, per_read_isl):
     reads, qual = golden
@@ -184,7 +186,7 @@ def test_distinct_gc_golden(gm, ctx, gene, ogene, golden, flags, with_qual, per_
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("flags,with_qual", ORACLE_CASES, ids=["plain", "plain-qual", "indels", "indels-qual", "subs"])
+@pytest.mark.parametrize("flags,with_qual", ORACLE_CASES, ids=ORACLE_IDS)
 def test_distinct_gc_seeded(gm, ctx, gene, ogene, flags, with_qual):
     reads, qual = seeded_reads(4000, 100, 21)
     check_against_oracle(gm, ctx, gene, ogene, reads, qual, distinct_gc(len(reads), 5), flags, with_qual, True, n_api=300)
@@ -192,8 +194,7 @@ def test_distinct_gc_seeded(gm, ctx, gene, ogene, flags, with_qual):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("var,val", ROUTES, ids=[f"{k}={v}" for k, v in ROUTES])
-@pytest.mark.parametrize("flags,with_qual", [({}, False), ({"allow_indels": 1}, True), ({"allow_subs": 1}, False)],
-                         ids=["plain", "indels-qual", "subs"])
+@pytest.mark.parametrize("flags,with_qual", ROUTE_CASES, ids=ROUTE_IDS)
 def test_routes(gm, ctx, gene, ogene, golden, monkeypatch, var, val, flags, with_qual):
     reads, qual = golden
     monkeypatch.setenv(var, val)
@@ -212,8 +213,7 @@ def test_k2_mode_one():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("flags,with_qual", [({}, False), ({"allow_indels": 1}, True), ({"allow_subs": 1}, False)],
-                         ids=["plain", "indels-qual", "subs"])
+@pytest.mark.parametrize("flags,with_qual", ROUTE_CASES, ids=ROUTE_IDS)
 def test_reduction_after_call(gm, ctx, gene, golden, flags, with_qual):
     """reduce_starts_mg after the batched call equals the reduction after per-read calls of the existing API"""
     reads, qual = golden
@@ -302,6 +302,6 @@ if __name__ == "__main__" and sys.argv[1:] == ["k2mode"]:
     reads, qual = golden_reads()
     og = O.lib().orc_icm_read(os.path.join(G, "NC_000915.icm").encode())
     gn = g.ICM.Read(c, os.path.join(G, "NC_000915.icm"))
-    for flags, with_qual in [({"allow_indels": 1}, True), ({"allow_subs": 1}, False)]:
+    for flags, with_qual in [({"allow_indels": 1}, True), ({"allow_subs": 1}, False), ({"allow_subs": 1}, True)]:
         check_against_oracle(g, c, gn, og, reads[:200], qual[:200], distinct_gc(200, 9), flags, with_qual, True, n_api=50)
     print("k2 mode 1 ok")

@@ -4,6 +4,7 @@ sample reads.  A logic check that needs no GPU; the same functions run inside th
 tests/test_gpu_parity.py holds them to the same lists."""
 import gzip
 import os
+import re
 import shutil
 import subprocess
 
@@ -38,7 +39,29 @@ def harness():
                                   (999, 0, 0, 2, 100), (999, 0, 0, 2, 99), (999, 0, 0, 2, 98), (600, 0, 0, 2, 77),
                                   (300, 0, 0, 2, 13)])
 def test_flat_enumeration_equals_oracle_on_the_host(harness, args):
-    n, ai, asub, imax, trunc = args
-    r = subprocess.run([EXE, os.path.join(ROOT, "tests", "golden", "NC_000915.icm"), harness, str(n), str(ai), str(asub),
-                        str(imax), str(trunc)], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and r.stdout.strip().splitlines()[-1].startswith("OK:"), r.stdout[-3000:] + r.stderr[-2000:]
+    run(harness, *args)
+
+
+def run(harness, *args):
+    r = subprocess.run([EXE, os.path.join(ROOT, "tests", "golden", "NC_000915.icm"), harness] + [str(a) for a in args],
+                       capture_output=True, text=True, timeout=600)
+    last = r.stdout.strip().splitlines()[-1] if r.stdout.strip() else ""
+    assert r.returncode == 0 and last.startswith("OK:"), r.stdout[-3000:] + r.stderr[-2000:]
+    return {k: int(v) for k, v in re.findall(r"(qualities 0|>= 163|\+inf|-inf): (\d+)", last)}
+
+
+# seeded Phred values as from a quality file, half of them at the table edges (0, 17-20, 162, 163, 255): the oracle gets
+# them as read, the flat passes the plane glimmer-mg builds (Clean_Quality_454 under -i only) and Pass_Stop_Penalty per root
+# (reads, allow_indels, allow_subs, indel_max, truncate_len, quality seed)
+@pytest.mark.parametrize("args", [(400, 0, 1, 2, 0, 11), (300, 1, 0, 2, 0, 12), (300, 1, 1, 2, 0, 13), (400, 1, 0, 1, 0, 14),
+                                  (400, 0, 0, 2, 0, 15), (200, 1, 1, 2, 76, 16), (999, 0, 1, 2, 100, 17)])
+def test_flat_enumeration_with_quality_file_equals_oracle_on_the_host(harness, args):
+    n, ai, asub = args[:3]
+    seen = run(harness, *args)
+    assert seen[">= 163"] > 0
+    if ai:  # cleaned: no zero survives, so no stop probability of 0
+        assert seen["qualities 0"] == 0 and seen["+inf"] == 0
+    else:
+        assert seen["qualities 0"] > 0
+    if asub and not ai:  # a 0 on a stop base: p_stop = 0, an infinite substitution penalty reaches the start scores
+        assert seen["+inf"] > 0
