@@ -2,13 +2,17 @@
 //
 //   K1  k1_planes          per-position six-frame ICM tree walks            (Score_All_Frames glimmer-mg.cc:1468,
 //                                                                            ICM_t::Frame_Score icm.cc:485)
-//   K2  k2_prefix          per-(strand, reading-frame class) prefix sums of gene - indep log-odds, previous /
-//                          next in-frame stop tables, 454 quality synthesis, FP64 exactness certificate
-//                                                                           (Cumulative_Frame_Score glimmer-mg.cc:561,
+//   K2  k2_prefix_lanes    per-(strand, reading-frame class) prefix sums of gene - indep log-odds, previous /
+//                          next in-frame stop tables, 454 quality synthesis, FP64 exactness certificate (glimmer-mg
+//                          -i / -s)                                         (Cumulative_Frame_Score glimmer-mg.cc:561,
 //                                                                            Save_Prev_Stops :675, Set_Quality_454 :1865)
-//   K3  k3_mg_starts       per-ORF start enumeration incl. indel / substitution branches
-//                                                                           (Score_Orf_Starts :1693, Score_Indels :1513)
-//       k3_g3_starts       whole-genome variant on extracted ORF strings    (Score_Orfs glimmer3.cc:1275)
+//       k2_g3_codon_cum    codon-boundary sums of the glimmer3 path
+//   K3  k_mgf_*            per-ORF start enumeration incl. indel / substitution branches, level by level (flat form)
+//       k3_mg_starts       the same with one thread per ORF         (Score_Orf_Starts :1693, Score_Indels :1513)
+//       k3_mg_plain_lanes, k3_mg_plain
+//                          K2 + K3 fused for plain glimmer-mg (no error branches)
+//       k3_g3_count, k3_g3_heads, k3_g3_emit, k3_g3_ordered
+//                          glimmer3's start enumeration                     (Score_Orfs glimmer3.cc:1275)
 //   plus the device ORF finder (Find_Orfs glimmer_base.cc:638) and the scalar operator surface
 //   (Score_String / Cumulative_Score / Frame_Score icm.cc:864/354/485).
 //
@@ -474,8 +478,7 @@ static int launch_k1(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqset* s, float** p
   if (gmg_scratch(ctx, SCR_PLANES, (size_t)6 * (s->total + 32) * sizeof(float), &planes)) return 1;
   *planes_out = (float*)planes;
   if (s->total == 0) return 0;
-  static const int k1_mode = getenv("GMG_K1_MODE") ? atoi(getenv("GMG_K1_MODE")) : 0;  // 0 bucketed, 1 generic
-  if (gene->fast.valid && gene->W <= 14 && k1_mode == 0) {
+  if (gene->fast.valid && gene->W <= 14) {
     if (!s->n_base_valid) {
       unsigned long long nb[4];
       GMG_CUDA(cudaMemcpyAsync(nb, s->d_gc + 2, sizeof nb, cudaMemcpyDeviceToHost, ctx->stream));
@@ -498,50 +501,29 @@ static int launch_k1(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqset* s, float** p
       bl += (unsigned)s->n_base[b];
     }
     const size_t smem = (size_t)(4 + 64 + 1024) * 4 + (size_t)gene->fast.np * sizeof(float);
-    // (contexts per thread and trip, threads per CTA).  Long sequences use (6, 384): six walks in flight per thread
-    // hide the shared-memory latency with a third of the warps and the loop overhead is paid once per six walks
-    // (72 us per 5 Mbp against 77.8 us for (2, 1024); (4, 512) and (3, 768) also 72-73 us, (8, 256) 76 us), and the
-    // 768 threads per SM leave room for the side-stream kernels of gmg_score_orfs_g3 to run beside K1 (0.242 ms per
-    // step against 0.255 ms with (4, 512)).  GMG_K1_U / GMG_K1_NT select the other variants.
-    // Short reads keep (2, 1024): a trip takes the tested path when ANY of its kU x 32 windows per warp is partial,
-    // and reads have W-1 partial windows at either end (reads100: 0.70 ms against 0.76 ms with four per thread).
-    static const int ku_env = getenv("GMG_K1_U") ? atoi(getenv("GMG_K1_U")) : 0;
-    static const int knt_env = getenv("GMG_K1_NT") ? atoi(getenv("GMG_K1_NT")) : 0;
+    // Six walks in flight per thread, 384 threads per CTA: the six hide the shared-memory latency with a third of the
+    // warps and pay the loop overhead once per six walks, and the 768 threads per SM leave room for the side-stream
+    // kernels of gmg_score_orfs_g3 to run beside K1 (the other shapes measured took as long or longer, DESIGN.md 3.1).
+    // Read sets walk every window as full (no partial-window test in the hot loop) and k1_partial_fix redoes the
+    // 2 (W-1) x 3 partial entries of every sequence; on long sequences the test costs less than that second launch
+    // (5 Mbp contig: 71.6 against 78.9 us), so they keep the tested loop.  GMG_K1_FIX=0 (test hook): read sets too.
     const bool long_seqs = s->total / (s->n > 0 ? s->n : 1) >= 4096;
-    const int ku = ku_env ? ku_env : (long_seqs ? 6 : 2);
-    const int knt = knt_env ? knt_env : (long_seqs ? 384 : 1024);
+    const char* fix_env = getenv("GMG_K1_FIX");
+    const bool fix = !long_seqs && !(fix_env && atoi(fix_env) == 0);
     long long need = (acc + 4095) / 4096;
     long long cap = (long long)ctx->sm_count * 2;
     int grid = (int)(need < cap ? need : cap);
     if (gmg_prof_begin(ctx, GMG_PROF_K1)) return 1;
-#define GMG_K1_LAUNCH(U, T)                                                                                             \
-  do {                                                                                                                  \
-    GMG_CUDA(cudaFuncSetAttribute(k1_planes_bucketed<U, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));     \
-    k1_planes_bucketed<U, T><<<grid, T, smem, ctx->stream>>>(gene->fast, s->d_ctxf, s->d_ctxr, (unsigned)s->total, segs,  \
-                                                            (float*)planes);                                            \
-  } while (0)
-    // read sets: every window walked as full (no partial-window test, no slow path in the hot loop), the 2 (W-1) x 3
-    // partial entries of every sequence redone by k1_partial_fix.  GMG_K1_FIX=0 disables, =1 extends it to long sequences
-    // (measured on the 5 Mbp contig: the test costs 7 % of K1's instructions, the second launch as much: 78.9 against
-    // 71.6 us, so long sequences keep the tested kernel).
-    const int fix_env = getenv("GMG_K1_FIX") ? atoi(getenv("GMG_K1_FIX")) : 2;
-    const bool fix = fix_env && !(fix_env == 2 && long_seqs) && !ku_env;
+    const auto k1 = fix ? k1_planes_bucketed<6, 384, true> : k1_planes_bucketed<6, 384, false>;
+    GMG_CUDA(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k1<<<grid, 384, smem, ctx->stream>>>(gene->fast, s->d_ctxf, s->d_ctxr, (unsigned)s->total, segs, (float*)planes);
     if (fix) {
-      GMG_CUDA(cudaFuncSetAttribute(k1_planes_bucketed<6, 384, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k1_planes_bucketed<6, 384, true><<<grid, 384, smem, ctx->stream>>>(gene->fast, s->d_ctxf, s->d_ctxr,
-                                                                         (unsigned)s->total, segs, (float*)planes);
       const int64_t items = s->n * 2 * (gene->W - 1);
       int64_t fg = (items + 255) / 256, fcap = (int64_t)ctx->sm_count * 16;
       k1_partial_fix<<<(unsigned)(fg < fcap ? fg : fcap), 256, 0, ctx->stream>>>(
           gene->fast, s->d_words, s->d_off, s->n, s->d_bktidx, s->d_ctxf, s->d_ctxr, s->total, (float*)planes);
       ctx->launches++;
-    } else if (ku == 1) GMG_K1_LAUNCH(1, 1024);
-    else if (ku == 2) GMG_K1_LAUNCH(2, 1024);
-    else if (ku == 3 && knt == 768) GMG_K1_LAUNCH(3, 768);
-    else if (ku == 8 && knt == 256) GMG_K1_LAUNCH(8, 256);
-    else if (ku == 4) GMG_K1_LAUNCH(4, 512);
-    else GMG_K1_LAUNCH(6, 384);
-#undef GMG_K1_LAUNCH
+    }
     gmg_prof_end(ctx, GMG_PROF_K1);
     ctx->launches++;
     GMG_CUDA(cudaGetLastError());
@@ -1980,193 +1962,16 @@ __global__ void __launch_bounds__(128) k3_g3_ordered(DevIcm gene, DevIcm indep, 
 }
 
 // ------------------------------------------------------------------------------------------------
-// K2 (glimmer-mg): per-sequence prefix sums, stop tables, quality synthesis, exactness certificate.
-// One warp per sequence.
-
-// lowest set bit exponent of a finite non-zero double (x is an integer multiple of 2^ret)
-__device__ __forceinline__ int low_bit_exp(double x) {
-  long long b = __double_as_longlong(x);
-  int e = (int)((b >> 52) & 0x7FF);
-  unsigned long long mant = (unsigned long long)b & 0xFFFFFFFFFFFFFull;
-  if (e == 0) return -1074 + (mant ? __ffsll((long long)mant) - 1 : 0);
-  mant |= 1ull << 52;
-  return e - 1075 + (__ffsll((long long)mant) - 1);
-}
-
-template <bool kPS>
-__global__ void __launch_bounds__(128) k2_prefix(DevIcm indep_, IndepSeqs X, const uint64_t* __restrict__ words,
-                                                 const int64_t* __restrict__ off, int64_t n_seq, int64_t total,
-                                                 const float* __restrict__ planes, const uint32_t* __restrict__ bktidx,
-                                                 CodonSets cs, DevParams P,
-                                                 const uint8_t* __restrict__ qual_in, double* __restrict__ cum,
-                                                 int32_t* __restrict__ fwd_prev, int32_t* __restrict__ rev_next,
-                                                 uint8_t* __restrict__ qual, uint8_t* __restrict__ cert) {
-  const int64_t s = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (s >= n_seq) return;
-  DevIcm own;  // kPS: the sequence's own model; the single-model form reads the kernel parameter
-  if constexpr (kPS) own = indep_of(indep_, X, s);
-  const DevIcm& indep = kPS ? own : indep_;
-  const int64_t a = off[s];
-  const int L = (int)(off[s + 1] - a);
-  if (L == 0) {
-    if (lane == 0) cert[s] = 1;
-    return;
-  }
-  int gmin = 4096;
-  double asum = 0.0;
-
-  // ---- left-to-right: reverse-strand prefix sums, previous forward stops, quality ----
-  {
-    double carry[3] = {0.0, 0.0, 0.0};
-    int last_stop[3] = {0, 1, -1};  // Save_Prev_Stops init (glimmer-mg.cc:684)
-    for (int base = 0; base < L; base += 32) {
-      const int q = base + lane;
-      const bool in = q < L;
-      double x[3] = {0.0, 0.0, 0.0};
-      if (in) {
-        const size_t pi = gmg_plane_index(words, bktidx, a + q);
-#pragma unroll
-        for (int c = 0; c < 3; c++) {
-          const int f = mod3(1 + q - c);
-          const float gval = planes[(size_t)(3 + f) * total + pi];
-          const float nval = icm_rev(indep, words, a + q, q, 0, f);
-          x[c] = (double)gval - (double)nval;
-          if (x[c] != 0.0) gmin = min(gmin, low_bit_exp(x[c]));
-          asum += fabs(x[c]);
-        }
-      }
-#pragma unroll
-      for (int c = 0; c < 3; c++) {
-        double v = x[c];
-        for (int d = 1; d < 32; d <<= 1) {
-          double t = __shfl_up_sync(0xffffffffu, v, d);
-          if (lane >= d) v += t;
-        }
-        v += carry[c];
-        if (in) cum[(size_t)(3 + c) * total + a + q] = v;
-        carry[c] = __shfl_sync(0xffffffffu, v, 31);
-      }
-      // previous forward stop per frame class q % 3 (index of the stop's last base)
-      int st = -0x40000000;
-      if (in && q >= 2 && ((cs.stop_mask >> codon_fwd_ending_at(words, a, q)) & 1)) st = q;
-      int v = st;
-      for (int d = 3; d < 32; d *= 2) {  // class-restricted max-scan: same class = multiples of 3 apart
-        int t = __shfl_up_sync(0xffffffffu, v, d);
-        if (lane >= d) v = max(v, t);
-      }
-      const int cl = q % 3;
-      int prevv = max(v, cl == 0 ? last_stop[0] : (cl == 1 ? last_stop[1] : last_stop[2]));
-      // carries must only replace the init values when a real stop was seen
-      if (v < 0) prevv = (cl == 0 ? last_stop[0] : (cl == 1 ? last_stop[1] : last_stop[2]));
-      if (in) fwd_prev[a + q] = prevv;
-      // new carries: value at the last lane of each class in this chunk
-#pragma unroll
-      for (int c = 0; c < 3; c++) {
-        // highest lane l with (base + l) % 3 == c and base + l < L
-        int top = min(31, L - 1 - base);
-        int l = top - mod3(base + top - c);
-        int nv = __shfl_sync(0xffffffffu, prevv, l < 0 ? 0 : l);
-        if (l >= 0) last_stop[c] = nv;
-      }
-      // Without a quality file, Set_Quality_454 (glimmer-mg.cc:1865-1906): last base of a homopolymer run of length r
-      // gets 31 - 5*min(r,5), every other base 31.  With one, the file's values (already clamped to 0..255), cleaned by
-      // Clean_Quality_454 (:519-546) under -i only, as main() does (:385-392): under -s alone they reach
-      // Pass_Stop_Penalty as read.
-      if (in && qual) {
-        const int b = gmg_base_at(words, a + q);
-        const bool last_of_run = (q == L - 1) || (gmg_base_at(words, a + q + 1) != b);
-        int qv;
-        if (qual_in) {
-          qv = qual_in[a + q];
-          if (P.allow_indels) {
-            if (qv <= 0) qv = 1;
-            if (!last_of_run && qv < P.indel_q_thresh + 1) qv = P.indel_q_thresh + 1;
-          }
-        } else if (!last_of_run) {
-          qv = 31;
-        } else {
-          int r = 1;
-          while (r < 5 && q - r >= 0 && gmg_base_at(words, a + q - r) == b) r++;
-          qv = 31 - 5 * r;
-        }
-        qual[a + q] = (uint8_t)qv;
-      }
-    }
-  }
-  // ---- right-to-left: forward-strand suffix sums, next reverse stops ----
-  {
-    double carry[3] = {0.0, 0.0, 0.0};
-    // Save_Prev_Stops reverse init (glimmer-mg.cc:706-708) per class r = (L-1-q) % 3: {L-1, L-2, L}
-    int next_stop[3] = {L - 1, L - 2, L};
-    for (int base = 0; base < L; base += 32) {
-      const int q = L - 1 - (base + lane);  // lane 0 = rightmost
-      const bool in = q >= 0;
-      double x[3] = {0.0, 0.0, 0.0};
-      if (in) {
-        const size_t pi = gmg_plane_index(words, bktidx, a + q);
-#pragma unroll
-        for (int c = 0; c < 3; c++) {
-          const int f = mod3(c - q);
-          const float gval = planes[(size_t)f * total + pi];
-          const float nval = icm_fwd(indep, words, a + q, q, L, f);
-          x[c] = (double)gval - (double)nval;
-          if (x[c] != 0.0) gmin = min(gmin, low_bit_exp(x[c]));
-          asum += fabs(x[c]);
-        }
-      }
-#pragma unroll
-      for (int c = 0; c < 3; c++) {
-        double v = x[c];
-        for (int d = 1; d < 32; d <<= 1) {
-          double t = __shfl_up_sync(0xffffffffu, v, d);
-          if (lane >= d) v += t;
-        }
-        v += carry[c];
-        if (in) cum[(size_t)c * total + a + q] = v;
-        carry[c] = __shfl_sync(0xffffffffu, v, 31);
-      }
-      int st = 0x40000000;
-      if (in && q <= L - 3 && ((cs.stop_mask >> codon_rev_starting_at(words, a, q)) & 1)) st = q;
-      int v = st;
-      for (int d = 3; d < 32; d *= 2) {
-        int t = __shfl_up_sync(0xffffffffu, v, d);
-        if (lane >= d) v = min(v, t);
-      }
-      const int r = (base + lane) % 3;  // (L-1-q) % 3
-      const int init = (r == 0 ? next_stop[0] : (r == 1 ? next_stop[1] : next_stop[2]));
-      // a stop at or right of q inside this chunk is always nearer than the carried one
-      const int nextv = (v >= 0x40000000) ? init : v;
-      if (in) rev_next[a + q] = nextv;
-#pragma unroll
-      for (int c = 0; c < 3; c++) {
-        int top = min(31, L - 1 - base);  // highest valid lane
-        int l = top - mod3(base + top - c);
-        int nv = __shfl_sync(0xffffffffu, nextv, l < 0 ? 0 : l);
-        if (l >= 0) next_stop[c] = nv;
-      }
-    }
-  }
-  // ---- certificate: every partial sum of every plane is exactly representable ----
-  for (int d = 16; d > 0; d >>= 1) {
-    gmin = min(gmin, __shfl_xor_sync(0xffffffffu, gmin, d));
-    asum += __shfl_xor_sync(0xffffffffu, asum, d);
-  }
-  if (lane == 0) {
-    // all terms are multiples of 2^gmin and |any partial sum| <= asum: exact iff asum < 2^(gmin+52)
-    // (one binade of margin for the rounding of asum itself)
-    bool ok = (gmin == 4096) || (asum < ldexp(1.0, gmin + 52));
-    cert[s] = ok ? 1 : 0;
-  }
-}
-
-// K2, lane-serial form (the default): one warp per sequence, every lane owns FOUR consecutive positions of a
-// 128-position tile whose start is aligned to 4 bases of the batch, so that a lane's four results of one array
-// are one aligned 32-byte run (two 16-byte stores for doubles, one for the int32 stop tables, one 4-byte store
-// for qualities) and its four plane indices share one block lookup.  Sums run serially inside the lane; one warp
-// scan per class joins the 32 lane totals -- 6 FP64 scans per 128 positions instead of 24 -- and the
-// independent model is the 384-entry full-window table (lut3) in shared memory except at the two end positions.
-// Any association gives the reference's bits under the read's certificate (same statement as above).
+// K2 (glimmer-mg -i / -s): per-sequence prefix sums, stop tables, quality synthesis, exactness certificate.
+// One warp per sequence, every lane owns FOUR consecutive positions of a 128-position tile whose start is aligned to 4
+// bases of the batch, so that a lane's four results of one array are one aligned 32-byte run (two 16-byte stores for
+// doubles, one for the int32 stop tables, one 4-byte store for qualities) and its four plane indices share one block
+// lookup.  Sums run serially inside the lane; one warp scan per class joins the 32 lane totals -- 6 FP64 scans per 128
+// positions instead of the 24 of one position per lane -- and the independent model is the 384-entry full-window table
+// (lut3) in shared memory except at the two end positions.
+// Any association gives the reference's bits under the read's certificate: every term is a multiple of 2^g (g from the
+// smallest float exponent among the read's terms), so while the sum of magnitudes stays below 2^(g+52) no partial sum
+// can round.
 #define K2_R 4
 // c + i for c in 0..2, i in 0..3, reduced mod 3 without a division
 __device__ __forceinline__ int k2_add3(int c, int i) {
@@ -2283,11 +2088,15 @@ __global__ void __launch_bounds__(128) k2_prefix_lanes(DevIcm indep_, IndepSeqs 
             const int cd = ((raw_rev & 3) << 4) | (raw_rev & 12) | (raw_rev >> 4);
             if ((cs.stop_mask >> cd) & 1) stp[i] = q;
           }
+          // Without a quality file, Set_Quality_454 (glimmer-mg.cc:1865-1906): last base of a homopolymer run of length
+          // r gets 31 - 5*min(r,5), every other base 31.  With one, the file's values (already clamped to 0..255),
+          // cleaned by Clean_Quality_454 (:519-546) under -i only, as main() does (:385-392): under -s alone they reach
+          // Pass_Stop_Penalty as read.
           if (qual) {
             const int b = (int)bs;
             const bool last_of_run = (q == L - 1) || ((int)((win >> (2 * (i + 5))) & 3) != b);
             int qv;
-            if (qual_in) {  // the file's values; Clean_Quality_454 under -i only (see k2_prefix)
+            if (qual_in) {
               qv = qual_in[a + q];
               if (P.allow_indels) {
                 if (qv <= 0) qv = 1;
@@ -3182,11 +2991,11 @@ __device__ __forceinline__ double mgl_codon_sum(const DevIcm& indep, const float
 }
 
 // G = lanes per ORF, K = chunks of G codons: an instance takes the ORFs with need_lo < need <= 3 * G * K scored bases (and
-// j_lo >= 3).  <32, 4>: one ORF per warp up to 384 bases; <16, 4>: TWO per warp up to 192; <8, 6>: FOUR per warp up to 144.
+// j_lo >= 3).  Two instances: <16, 4>, TWO ORFs per warp up to 192 bases, and <32, 4>, one ORF per warp up to 384.
 // The kernel is bound by the latency of a warp's dependent rounds (6 us per ORF with one ORF per warp, 40 % issue
 // utilisation at 32 warps per SM): more ORFs in flight per warp at the same register count is what raises the throughput
-// on short reads (0.61 -> 0.49 ms per 31 Mbp with two; four: 0.50 -- the lane's serial share grows and its prefix
-// registers spill).
+// on short reads (0.61 -> 0.49 ms per 31 Mbp with two; four per warp gave 0.50 -- the lane's serial share grows and its
+// prefix registers spill).
 template <int G, int K, bool kPS>
 __global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep_, const float* __restrict__ planes,
                                                          const uint32_t* __restrict__ bktidx, MgfBatch B, DevParams P, Which4 which,
@@ -3348,59 +3157,6 @@ __global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep_, const
     }
   }
   __syncwarp();  // the serial rows are free for the warp's next ORFs
-  }
-}
-
-// The same fused pass with ONE THREAD per ORF (an alternative, GMG_PLAIN_SERIAL=1): the ORF's records are laid out first
-// (positions, codons, flags from the codon bitmaps), then the thread walks the ORF string once, accumulating
-// gene - indep serially in the reference's own order (glimmer-mg.cc:577-586) and dropping each running sum into the
-// record that asks for it.  No scan, no certificate -- the order IS the reference's.  Measured slower than the warp form
-// on 100 bp reads (0.76 against 0.63 ms per 31 Mbp): kept as the simplest exact statement of the pass and for A/B runs.
-template <bool kPS>
-__global__ void __launch_bounds__(128) k3_mg_plain_serial(DevIcm indep_, IndepSeqs X, const float* __restrict__ planes,
-                                                          const uint32_t* __restrict__ bktidx, MgfBatch B, DevParams P_,
-                                                          CodonSets cs, const gmg_orf* __restrict__ orfs,
-                                                          const int32_t* __restrict__ orf_seq, int64_t n_orfs,
-                                                          const int64_t* __restrict__ start_off, gmg_start* __restrict__ starts) {
-  __shared__ float s_lut_sh[384];
-  if (!kPS && indep_.lut3 != NULL)
-    for (int i = threadIdx.x; i < 384; i += blockDim.x) s_lut_sh[i] = indep_.lut3[i];
-  __syncthreads();
-  const int64_t o = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (o >= n_orfs) return;
-  const int64_t so = start_off[o];
-  const int cnt = (int)(start_off[o + 1] - so);
-  if (cnt == 0) return;
-  const MgfSeq S = mgf_seq_of(B, orf_seq[o]);
-  // per-sequence models (gmg_score_orfs_mg_gc): the sequence's own table (read through L1) and ignore length
-  DevIcm own;  // kPS: the sequence's own model; the single-model form reads the kernel parameter
-  if constexpr (kPS) own = indep_of(indep_, X, orf_seq[o]);
-  const DevIcm& indep = kPS ? own : indep_;
-  const float* const s_lut = kPS ? indep.lut3 : s_lut_sh;
-  const DevParams P = kPS ? mgf_params_of(P_, X, orf_seq[o]) : P_;
-  const gmg_orf orf = orfs[o];
-  const bool fwd = orf.frame > 0;
-  const int hi = fwd ? orf.stop_position - 1 : orf.stop_position + 3 + orf.orf_len;
-  const int lo = fwd ? hi - orf.orf_len : orf.stop_position + 3;
-  MgfOwn f;
-  mgf_own_open(B, S, P, fwd, lo, hi, 0, f);
-  gmg_start* out = starts + so;
-  const int ep[2] = {0, 0}, et[2] = {0, 0};
-  DevParams Pn = P;
-  Pn.ignore_score_len = INT_MAX;  // the boost is applied when the score is known
-  mgf_own_write_with(B, S, Pn, cs, f, fwd, 0.0, 0, 0, ep, et, out, [](int) { return (int64_t)0; }, [](int) { return 0.0; });
-  // records are in descending j; walk j upwards and serve them from the last one
-  int r = cnt - 1;
-  double run = 0.0;
-  for (int j = 0; r >= 0; j++) {
-    float g, n;
-    mgp_term(indep, s_lut, planes, bktidx, B, S, fwd, (1 + j) % 3, fwd ? hi - 1 - j : lo - 1 + j, &g, &n);
-    run = run + ((double)g - (double)n);  // score[j]
-    while (r >= 0 && out[r].j - 2 == j + 1) {  // a start at j + 1 takes score[j] (glimmer-mg.cc:1826)
-      const double sc = (run - 0.0) + 0.0;
-      out[r].score = (out[r].j > P.ignore_score_len && 0.0 > sc) ? 0.0 : sc;
-      r--;
-    }
   }
 }
 
@@ -3869,8 +3625,7 @@ extern "C" int gmg_score_orfs_g3(gmg_ctx* ctx, const gmg_icm* gene, const gmg_ic
   float* planes = NULL;
   void* d_planes;
   if (gmg_scratch(ctx, SCR_PLANES, (size_t)6 * (s->total + 32) * sizeof(float), &d_planes)) return 1;  // before the fork
-  static const int no_side = getenv("GMG_G3_NO_SIDE") ? atoi(getenv("GMG_G3_NO_SIDE")) : 0;  // diagnostic: one stream
-  cudaStream_t side = no_side ? ctx->stream : ctx->side;
+  cudaStream_t side = ctx->side;
   GMG_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
   GMG_CUDA(cudaStreamWaitEvent(side, ctx->ev_fork, 0));
   GMG_CUDA(cudaMemsetAsync(counts + s->n_orfs, 0, 2 * sizeof(int64_t), side));
@@ -3932,31 +3687,10 @@ extern "C" int gmg_score_orfs_g3(gmg_ctx* ctx, const gmg_icm* gene, const gmg_ic
   return 0;
 }
 
-// gmg_score_orfs_mg (kPS = false: one independent model) and gmg_score_orfs_mg_gc (kPS: the model and ignore length of
-// every sequence from X); the kernels take the same switch, so the single-model call compiles to the work it always did
+// Plain glimmer-mg (no error branches): K2 and K3 fused into one pass per ORF over the K1 planes
 template <bool kPS>
-static int score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& indep, const IndepSeqs& X, gmg_seqset* s,
-                         const gmg_params* p, int64_t* n_starts) {
-  CodonSets cs;
-  DevParams dp;
-  if (make_codon_sets(p, &cs, &dp)) return 1;
-  GMG_CHECK(!(p->have_quality_file && !s->d_qual), "have_quality_file set but the seqset has no quality values");
-  s->n_starts = 0;
-  s->uncertified = 0;
-  s->uncert_pending = NULL;
-  s->n_red = s->n_red_fallback = 0;
-  s->d_red = NULL;
-  if (n_starts) *n_starts = 0;
-  if (s->n_orfs == 0) return 0;
-  GMG_CHECK(s->n_orfs < 0x7fffffffll && s->total < 0xffffffffll, "gmg_score_orfs_mg: batch too large (%lld ORFs): split it",
-            (long long)s->n_orfs);
-  if (ensure_codon_bits(ctx, s, cs)) return 1;  // start-codon bitmaps: the own starts of every call
-  // flat form (0) when calls can branch (-i / -s); without error branches the fused per-ORF scan (2) -- or, for very
-  // long sequences and caller-supplied ORF tables, K2 + one thread per ORF (1).  GMG_K3MG_MODE forces a form (tests).
-  const int k3mg_env = getenv("GMG_K3MG_MODE") ? atoi(getenv("GMG_K3MG_MODE")) : -1;
-  const bool branching = p->allow_indels || p->allow_subs;
-  const bool fused_ok = !branching && !s->orfs_external && s->max_len <= 3 * (MGP_SLOTS - 1);
-  const int k3mg_mode = k3mg_env >= 0 && !(k3mg_env == 2 && !fused_ok) ? k3mg_env : (branching ? 0 : (fused_ok ? 2 : 1));
+static int score_orfs_mg_plain(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& indep, const IndepSeqs& X, gmg_seqset* s,
+                               const gmg_params* p, const CodonSets& cs, const DevParams& dp, int64_t* n_starts) {
   MgfBatch B;
   memset(&B, 0, sizeof B);
   B.words = s->d_words;
@@ -3964,102 +3698,85 @@ static int score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& indep,
   B.total = s->total;
   B.cb = s->d_cbits;
   B.nwc = s->nwc;
-  int64_t* counts = NULL;
-  PlainDesc* geom = NULL;
-  if (k3mg_mode == 2) {
-    // The record counts only need the codon bitmaps: they are taken, scanned and their total sent to pinned memory BEFORE
-    // the walks are launched, so the host sizes the output while K1 runs and the emission kernel follows K1 without a gap
-    // (the stream used to drain between the count and the emission: a host round trip inside every step).
-    if (gmg_seqset_ensure_buckets(ctx, s)) return 1;  // here, not inside K1: one host synchronisation serves both
-    void* d_counts;
-    if (gmg_scratch(ctx, SCR_FLAGS, (size_t)(s->n_orfs + 2) * sizeof(int64_t), &d_counts)) return 1;
-    counts = (int64_t*)d_counts;
-    GMG_CUDA(cudaMemsetAsync(counts + s->n_orfs, 0, 2 * sizeof(int64_t), ctx->stream));
-    if (gmg_prof_begin(ctx, GMG_PROF_K3)) return 1;
-    void* d_geom;
-    if (gmg_scratch(ctx, SCR_MISC, (size_t)(s->n_orfs + 1) * sizeof(PlainDesc), &d_geom)) return 1;
-    geom = (PlainDesc*)d_geom;
-    k3_mg_plain_count<<<(unsigned)((s->n_orfs + 127) / 128), 128, 0, ctx->stream>>>(B, dp, s->d_orfs, s->d_orf_seq, s->n_orfs, counts,
-                                                                                   geom);
-    gmg_prof_end(ctx, GMG_PROF_K3);
-    ctx->launches++;
-    if (exclusive_sum_i64(ctx, counts, s->d_start_off, s->n_orfs + 1)) return 1;
-    ctx->h_scalars[6] = 0;
-    GMG_CUDA(cudaMemcpyAsync(&ctx->h_scalars[6], s->d_start_off + s->n_orfs, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    GMG_CUDA(cudaEventRecord(ctx->ev_scalars, ctx->stream));
-  }
+  // The record counts only need the codon bitmaps: they are taken, scanned and their total sent to pinned memory BEFORE
+  // the walks are launched, so the host sizes the output while K1 runs and the emission kernel follows K1 without a gap
+  // (the stream used to drain between the count and the emission: a host round trip inside every step).
+  if (gmg_seqset_ensure_buckets(ctx, s)) return 1;  // here, not inside K1: one host synchronisation serves both
+  void* d_counts;
+  if (gmg_scratch(ctx, SCR_FLAGS, (size_t)(s->n_orfs + 2) * sizeof(int64_t), &d_counts)) return 1;
+  int64_t* counts = (int64_t*)d_counts;
+  GMG_CUDA(cudaMemsetAsync(counts + s->n_orfs, 0, 2 * sizeof(int64_t), ctx->stream));
+  if (gmg_prof_begin(ctx, GMG_PROF_K3)) return 1;
+  void* d_geom;
+  if (gmg_scratch(ctx, SCR_MISC, (size_t)(s->n_orfs + 1) * sizeof(PlainDesc), &d_geom)) return 1;
+  PlainDesc* geom = (PlainDesc*)d_geom;
+  k3_mg_plain_count<<<(unsigned)((s->n_orfs + 127) / 128), 128, 0, ctx->stream>>>(B, dp, s->d_orfs, s->d_orf_seq, s->n_orfs, counts,
+                                                                                 geom);
+  gmg_prof_end(ctx, GMG_PROF_K3);
+  ctx->launches++;
+  if (exclusive_sum_i64(ctx, counts, s->d_start_off, s->n_orfs + 1)) return 1;
+  ctx->h_scalars[6] = 0;
+  GMG_CUDA(cudaMemcpyAsync(&ctx->h_scalars[6], s->d_start_off + s->n_orfs, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+  GMG_CUDA(cudaEventRecord(ctx->ev_scalars, ctx->stream));
   float* planes;
   if (launch_k1(ctx, gene, s, &planes)) return 1;
-  if (k3mg_mode == 2) {
-    // exactness is certified per ORF inside the kernel; the test hook withdraws every certificate
-    const int exact_len = (getenv("GMG_MG_FORCE_UNCERT") && atoi(getenv("GMG_MG_FORCE_UNCERT")) > 0) ? -1 : INT_MAX;
-    GMG_CUDA(cudaEventSynchronize(ctx->ev_scalars));
-    const int64_t total_starts = ctx->h_scalars[6];
-    if (ensure_start_capacity(s, total_starts)) return 1;
-    // A/B: one thread per ORF with serial sums (GMG_PLAIN_SERIAL=1; measured 0.76 ms per 31 Mbp against 0.63 ms for the
-    // warp-per-ORF scan below, which is the default)
-    const int plain_serial = getenv("GMG_PLAIN_SERIAL") ? atoi(getenv("GMG_PLAIN_SERIAL")) : 0;
-    if (total_starts > 0 && plain_serial && exact_len >= 0) {
-      if (gmg_prof_begin(ctx, GMG_PROF_K3)) return 1;
-      k3_mg_plain_serial<kPS><<<(unsigned)((s->n_orfs + 127) / 128), 128, 0, ctx->stream>>>(
-          indep, X, planes, s->d_bktidx, B, dp, cs, s->d_orfs, s->d_orf_seq, s->n_orfs, s->d_start_off, s->d_starts);
-      gmg_prof_end(ctx, GMG_PROF_K3);
-      ctx->launches++;
-      GMG_CUDA(cudaGetLastError());
-    } else if (total_starts > 0) {
-      // one codon per lane for ORFs of up to 384 scored bases (two ORFs per warp up to 192); the warp-per-ORF
-      // scan for whatever is left.  GMG_PLAIN_LANES=0: all of them through the latter, =1: one ORF per warp throughout,
-      // =2 (default): two per warp up to 192 bases, =3: four per warp up to 144 bases (measured on 100 bp reads: 0.61 /
-      // 0.49 / 0.50 ms per 31 Mbp for 1 / 2 / 3; A/B runs, tests).
-      const int plain_lanes = getenv("GMG_PLAIN_LANES") ? atoi(getenv("GMG_PLAIN_LANES")) : 2;
-      if (gmg_prof_begin(ctx, GMG_PROF_K3)) return 1;
-      if (plain_lanes) {
-        Which4 which;
-        memset(&which, 0, sizeof which);
-        for (int cd = 0; cd < 64; cd++)
-          which.w[cd >> 4] |= (unsigned long long)(cs.which[cd] < 15 ? cs.which[cd] : 15) << (4 * (cd & 15));
-        // two ORFs per warp up to 192 scored bases (every ORF of a 100 bp read set), one up to 384; optionally four up to 144
-        const int64_t lanes_cap = (int64_t)ctx->sm_count * 8;  // 8 CTAs per SM resident
-        unsigned long long* d_nord = (unsigned long long*)(counts + s->n_orfs + 1);
-        int done_to = -1;  // ORFs with need <= done_to are taken by an instance launched so far
-        if (plain_lanes >= 3) {
-          const int64_t need_ctas = (s->n_orfs * 8 + 127) / 128;
-          k3_mg_plain_lanes<8, 6, kPS><<<(unsigned)(need_ctas < lanes_cap ? need_ctas : lanes_cap), 128, 0, ctx->stream>>>(
-              indep, planes, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to, X);
-          ctx->launches++;
-          done_to = 3 * 8 * 6;
-        }
-        if (plain_lanes >= 2 && s->max_len > done_to) {
-          const int64_t need_ctas = (s->n_orfs * 16 + 127) / 128;
-          k3_mg_plain_lanes<16, 4, kPS><<<(unsigned)(need_ctas < lanes_cap ? need_ctas : lanes_cap), 128, 0, ctx->stream>>>(
-              indep, planes, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to, X);
-          ctx->launches++;
-          done_to = 3 * 16 * 4;
-        }
-        if (s->max_len > done_to) {
-          const int64_t need_ctas = (s->n_orfs * 32 + 127) / 128;
-          k3_mg_plain_lanes<32, 4, kPS><<<(unsigned)(need_ctas < lanes_cap ? need_ctas : lanes_cap), 128, 0, ctx->stream>>>(
-              indep, planes, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to, X);
-          ctx->launches++;
-        }
-      }
-      // every ORF taken above?  (need <= orf_len <= max_len; j_lo >= 3 whenever min_gene_len >= 6)
-      const bool all_taken = plain_lanes && s->max_len <= 96 * 4 && p->min_gene_len >= 6;
-      if (!all_taken) {
-        const int slots = (int)(s->max_len / 3 + 4);
-        k3_mg_plain<kPS><<<(unsigned)((s->n_orfs * 32 + 127) / 128), 128, (size_t)4 * slots * sizeof(double), ctx->stream>>>(
-            indep, X, planes, s->d_bktidx, B, dp, cs, s->d_orfs, s->d_orf_seq, s->n_orfs, s->d_start_off, s->d_starts, exact_len,
-            (unsigned long long*)(counts + s->n_orfs + 1), slots, plain_lanes);
+  // exactness is certified per ORF inside the kernel; the test hook withdraws every certificate
+  const int exact_len = (getenv("GMG_MG_FORCE_UNCERT") && atoi(getenv("GMG_MG_FORCE_UNCERT")) > 0) ? -1 : INT_MAX;
+  GMG_CUDA(cudaEventSynchronize(ctx->ev_scalars));
+  const int64_t total_starts = ctx->h_scalars[6];
+  if (ensure_start_capacity(s, total_starts)) return 1;
+  if (total_starts > 0) {
+    // one codon per lane for ORFs of up to 384 scored bases: two ORFs per warp up to 192 (every ORF of a 100 bp read set),
+    // one beyond; the warp-per-ORF scan for whatever is left.  Test hooks: GMG_PLAIN_LANES=0 sends every ORF through the
+    // latter, =1 gives one ORF per warp throughout.
+    const int lanes_env = getenv("GMG_PLAIN_LANES") ? atoi(getenv("GMG_PLAIN_LANES")) : 2;
+    const int plain_lanes = lanes_env == 0 || lanes_env == 1 ? lanes_env : 2;
+    if (gmg_prof_begin(ctx, GMG_PROF_K3)) return 1;
+    if (plain_lanes) {
+      Which4 which;
+      memset(&which, 0, sizeof which);
+      for (int cd = 0; cd < 64; cd++)
+        which.w[cd >> 4] |= (unsigned long long)(cs.which[cd] < 15 ? cs.which[cd] : 15) << (4 * (cd & 15));
+      const int64_t lanes_cap = (int64_t)ctx->sm_count * 8;  // 8 CTAs per SM resident
+      unsigned long long* d_nord = (unsigned long long*)(counts + s->n_orfs + 1);
+      int done_to = -1;  // ORFs with need <= done_to are taken by an instance launched so far
+      // one instance, G lanes per ORF: the ORFs with done_to < need <= 3 * G * 4
+      auto launch_lanes = [&](auto kernel, int G) {
+        const int64_t need_ctas = (s->n_orfs * G + 127) / 128;
+        kernel<<<(unsigned)(need_ctas < lanes_cap ? need_ctas : lanes_cap), 128, 0, ctx->stream>>>(
+            indep, planes, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to, X);
         ctx->launches++;
-      }
-      gmg_prof_end(ctx, GMG_PROF_K3);
-      GMG_CUDA(cudaGetLastError());
+        done_to = 3 * G * 4;
+      };
+      if (plain_lanes == 2) launch_lanes(k3_mg_plain_lanes<16, 4, kPS>, 16);
+      if (s->max_len > done_to) launch_lanes(k3_mg_plain_lanes<32, 4, kPS>, 32);
     }
-    s->n_starts = total_starts;
-    s->uncert_pending = (unsigned long long*)(counts + s->n_orfs + 1);  // ORFs summed in serial order; read on demand
-    if (n_starts) *n_starts = total_starts;
-    return 0;
+    // every ORF taken above?  (need <= orf_len <= max_len; j_lo >= 3 whenever min_gene_len >= 6)
+    const bool all_taken = plain_lanes && s->max_len <= 96 * 4 && p->min_gene_len >= 6;
+    if (!all_taken) {
+      const int slots = (int)(s->max_len / 3 + 4);
+      k3_mg_plain<kPS><<<(unsigned)((s->n_orfs * 32 + 127) / 128), 128, (size_t)4 * slots * sizeof(double), ctx->stream>>>(
+          indep, X, planes, s->d_bktidx, B, dp, cs, s->d_orfs, s->d_orf_seq, s->n_orfs, s->d_start_off, s->d_starts, exact_len,
+          (unsigned long long*)(counts + s->n_orfs + 1), slots, plain_lanes);
+      ctx->launches++;
+    }
+    gmg_prof_end(ctx, GMG_PROF_K3);
+    GMG_CUDA(cudaGetLastError());
   }
+  s->n_starts = total_starts;
+  s->uncert_pending = (unsigned long long*)(counts + s->n_orfs + 1);  // ORFs summed in serial order; read on demand
+  if (n_starts) *n_starts = total_starts;
+  return 0;
+}
+
+// K2 (prefix sums, stop tables, qualities, certificates), then K3: the flat enumeration (k3mg_mode 0) or one thread
+// per ORF (1)
+template <bool kPS>
+static int score_orfs_mg_k2k3(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& indep, const IndepSeqs& X, gmg_seqset* s,
+                              const gmg_params* p, const CodonSets& cs, const DevParams& dp, int k3mg_mode,
+                              int64_t* n_starts) {
+  float* planes;
+  if (launch_k1(ctx, gene, s, &planes)) return 1;
   // K2
   void *d_cum, *d_tab, *d_qual, *d_cert;
   if (gmg_scratch(ctx, SCR_CUM, (size_t)6 * s->total * sizeof(double), &d_cum)) return 1;
@@ -4090,15 +3807,9 @@ static int score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& indep,
   const bool need_qual = p->allow_indels || p->have_quality_file;
   unsigned g2 = (unsigned)((s->n * 32 + 127) / 128);
   if (gmg_prof_begin(ctx, GMG_PROF_K2)) return 1;
-  static const int k2_mode = getenv("GMG_K2_MODE") ? atoi(getenv("GMG_K2_MODE")) : 0;  // 0 lane-serial tiles, 1 one position per lane
-  if (k2_mode == 0)
-    k2_prefix_lanes<kPS><<<g2, 128, 0, ctx->stream>>>(indep, X, s->d_words, s->d_off, s->n, s->total, planes, s->d_bktidx, cs,
-                                                 dp, p->have_quality_file ? s->d_qual : NULL, (double*)d_cum, fwd_prev,
-                                                 rev_next, need_qual ? (uint8_t*)d_qual : NULL, cert);
-  else
-    k2_prefix<kPS><<<g2, 128, 0, ctx->stream>>>(indep, X, s->d_words, s->d_off, s->n, s->total, planes, s->d_bktidx, cs, dp,
-                                           p->have_quality_file ? s->d_qual : NULL, (double*)d_cum, fwd_prev, rev_next,
-                                           need_qual ? (uint8_t*)d_qual : NULL, cert);
+  k2_prefix_lanes<kPS><<<g2, 128, 0, ctx->stream>>>(indep, X, s->d_words, s->d_off, s->n, s->total, planes, s->d_bktidx, cs,
+                                                   dp, p->have_quality_file ? s->d_qual : NULL, (double*)d_cum, fwd_prev,
+                                                   rev_next, need_qual ? (uint8_t*)d_qual : NULL, cert);
   gmg_prof_end(ctx, GMG_PROF_K2);
   ctx->launches++;
   GMG_CUDA(cudaGetLastError());
@@ -4112,6 +3823,7 @@ static int score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& indep,
   }
 
   // ---- K3 ----
+  MgfBatch B;
   memset(&B, 0, sizeof B);
   B.words = s->d_words;
   B.off = s->d_off;
@@ -4126,7 +3838,7 @@ static int score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& indep,
   B.tables = d_tables;
   void* d_counts;
   if (gmg_scratch(ctx, SCR_FLAGS, (size_t)(s->n_orfs + 2) * sizeof(int64_t), &d_counts)) return 1;
-  counts = (int64_t*)d_counts;
+  int64_t* counts = (int64_t*)d_counts;
   GMG_CUDA(cudaMemsetAsync(counts, 0, (size_t)(s->n_orfs + 2) * sizeof(int64_t), ctx->stream));
   const unsigned g3 = (unsigned)((s->n_orfs + 127) / 128);
   const uint32_t no = (uint32_t)s->n_orfs;
@@ -4285,6 +3997,35 @@ static int score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& indep,
   s->n_starts = total_starts;
   if (n_starts) *n_starts = total_starts;
   return 0;
+}
+
+// gmg_score_orfs_mg (kPS = false: one independent model) and gmg_score_orfs_mg_gc (kPS: the model and ignore length of
+// every sequence from X); the kernels take the same switch, so the single-model call compiles to the work it always did
+template <bool kPS>
+static int score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& indep, const IndepSeqs& X, gmg_seqset* s,
+                         const gmg_params* p, int64_t* n_starts) {
+  CodonSets cs;
+  DevParams dp;
+  if (make_codon_sets(p, &cs, &dp)) return 1;
+  GMG_CHECK(!(p->have_quality_file && !s->d_qual), "have_quality_file set but the seqset has no quality values");
+  s->n_starts = 0;
+  s->uncertified = 0;
+  s->uncert_pending = NULL;
+  s->n_red = s->n_red_fallback = 0;
+  s->d_red = NULL;
+  if (n_starts) *n_starts = 0;
+  if (s->n_orfs == 0) return 0;
+  GMG_CHECK(s->n_orfs < 0x7fffffffll && s->total < 0xffffffffll, "gmg_score_orfs_mg: batch too large (%lld ORFs): split it",
+            (long long)s->n_orfs);
+  if (ensure_codon_bits(ctx, s, cs)) return 1;  // start-codon bitmaps: the own starts of every call
+  // flat form (0) when calls can branch (-i / -s); without error branches the fused per-ORF scan (2) -- or, for very
+  // long sequences and caller-supplied ORF tables, K2 + one thread per ORF (1).  GMG_K3MG_MODE forces a form (tests).
+  const int k3mg_env = getenv("GMG_K3MG_MODE") ? atoi(getenv("GMG_K3MG_MODE")) : -1;
+  const bool branching = p->allow_indels || p->allow_subs;
+  const bool fused_ok = !branching && !s->orfs_external && s->max_len <= 3 * (MGP_SLOTS - 1);
+  const int k3mg_mode = k3mg_env >= 0 && !(k3mg_env == 2 && !fused_ok) ? k3mg_env : (branching ? 0 : (fused_ok ? 2 : 1));
+  if (k3mg_mode == 2) return score_orfs_mg_plain<kPS>(ctx, gene, indep, X, s, p, cs, dp, n_starts);
+  return score_orfs_mg_k2k3<kPS>(ctx, gene, indep, X, s, p, cs, dp, k3mg_mode, n_starts);
 }
 
 extern "C" int gmg_score_orfs_mg(gmg_ctx* ctx, const gmg_icm* gene, const gmg_icm* indep, gmg_seqset* s,

@@ -298,13 +298,12 @@ def test_score_all_frames_bit_exact(gm, ctx, reads, monkeypatch):
         want = O.score_all_frames(og, oi, O.filter_lower(s0))
         assert got.shape == want.shape
         assert (_bits(got) == _bits(want)).all()
-    # the other routes for partial windows: tested in the walk loop (0), fix-up kernel also for long sequences (1)
-    for mode in ("0", "1"):
-        monkeypatch.setenv("GMG_K1_FIX", mode)
-        fs2 = gm.SeqSet(ctx, seqs=seqs).score_all_frames(gene, indep)
-        monkeypatch.delenv("GMG_K1_FIX")
-        for a, b in zip(fs, fs2):
-            assert (_bits(a) == _bits(b)).all(), mode
+    # the other route for partial windows on read sets: tested in the walk loop, as for long sequences
+    monkeypatch.setenv("GMG_K1_FIX", "0")
+    fs2 = gm.SeqSet(ctx, seqs=seqs).score_all_frames(gene, indep)
+    monkeypatch.delenv("GMG_K1_FIX")
+    for a, b in zip(fs, fs2):
+        assert (_bits(a) == _bits(b)).all()
     # golden Frame_Scores of the unmodified reference (first 25 reads)
     recs = parse_dump(os.path.join(G, "mg_plain_120.dump.gz"))
     gc = _gc_oracle([s for _, s in reads[:120]])
@@ -537,11 +536,7 @@ def test_mg_plain_fused_scan_matches_thread_path_and_oracle(gm, ctx, reads, monk
 
     want = run()  # fused, one codon per lane, two ORFs per warp up to 192 scored bases (parallel scan under the per-ORF certificate)
     assert want[2] == 0
-    monkeypatch.setenv("GMG_PLAIN_SERIAL", "1")
-    got = run()   # fused, one thread per ORF (serial sums in the reference's order)
-    assert got[:2] == want[:2] and got[2] == 0
-    monkeypatch.delenv("GMG_PLAIN_SERIAL")
-    for mode in ("0", "1", "3"):  # a scan per 32 bases (ORFs beyond 384 scored bases) / one codon per lane: one / up to four ORFs per warp
+    for mode in ("0", "1"):  # a scan per 32 bases (ORFs beyond 384 scored bases) / one codon per lane, one ORF per warp
         monkeypatch.setenv("GMG_PLAIN_LANES", mode)
         got = run()
         assert got[:2] == want[:2] and got[2] == 0, mode

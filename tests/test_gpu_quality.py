@@ -10,8 +10,6 @@ starts with a run of the same base, stops at the first and last bases of a read 
 limit), empty and very short reads.  Every test asserts that its edge case occurred."""
 import math
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -19,7 +17,6 @@ import pytest
 import oracle_lib as O
 
 G = O.GOLDEN
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GENE = os.path.join(G, "NC_000915.icm")
 EDGE_Q = np.array([0, 1, 2, 17, 18, 19, 20, 40, 93, 162, 163, 255])
 FILE_BIG = 999999  # what the quality file holds where the host array holds 255 (the device clamps it to 255)
@@ -273,14 +270,6 @@ def test_routes_match_oracle(gm, ctx, gene, inputs, monkeypatch, var, val, call,
 
 
 @pytest.mark.gpu
-def test_k2_mode_one():
-    """GMG_K2_MODE (one position per lane) is read once per process: run the check in a process of its own"""
-    r = subprocess.run([sys.executable, os.path.abspath(__file__), "k2mode"], cwd=ROOT, capture_output=True, text=True,
-                       env=dict(os.environ, GMG_K2_MODE="1"))
-    assert r.returncode == 0 and "k2 mode 1 ok" in r.stdout, r.stdout[-3000:] + r.stderr[-3000:]
-
-
-@pytest.mark.gpu
 @pytest.mark.parametrize("mode", ["subs", "indels-subs"])
 def test_reduction(gm, ctx, gene, inputs, mode):
     """reduce_starts_mg on start lists with infinite scores: exact ties must come back as status 2"""
@@ -327,16 +316,3 @@ def test_threshold_255_rejected(gm, ctx, gene, inputs):
     assert n > 1000
     O.lib().orc_icm_free(oi)
     O.lib().orc_icm_free(og)
-
-
-if __name__ == "__main__" and sys.argv[1:] == ["k2mode"]:
-    sys.path.insert(0, ROOT)
-    import glimmer_mg_b200 as g
-    c = g.Context(0)
-    gn = g.ICM.Read(c, GENE)
-    inp = make_inputs()
-    for mode, source, call in [("subs", "file", "mg"), ("subs", "fastq", "gc"), ("indels", "file", "mg"),
-                               ("indels-subs", "host", "gc"), ("indels-max1", "file", "mg")]:
-        _, got = device(g, c, gn, inp, mode, 1, source, call)
-        assert_same(got, oracle(g, inp, mode, 1, source, call), f"GMG_K2_MODE=1 {mode} {source} {call}")
-    print("k2 mode 1 ok")

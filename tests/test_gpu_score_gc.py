@@ -2,8 +2,6 @@
 builds Build_Indep_WO_Stops from every read's own GC fraction.  The batched call must give, read by read, the bits of the
 existing call on that read alone with that model (and the read's own Ignore_Score_Len), and of the oracle port."""
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -11,11 +9,9 @@ import pytest
 import oracle_lib as O
 
 G = O.GOLDEN
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 MODES = [{}, {"allow_indels": 1}, {"allow_subs": 1}]
 ROUTES = [("GMG_K3MG_MODE", "0"), ("GMG_K3MG_MODE", "1"), ("GMG_PLAIN_LANES", "0"), ("GMG_PLAIN_LANES", "1"),
-          ("GMG_PLAIN_LANES", "3"), ("GMG_PLAIN_SERIAL", "1"), ("GMG_MG_FORCE_UNCERT", "1"), ("GMG_MG_FORCE_UNCERT", "3"),
-          ("GMG_INDEP_FORCE_HOST", "1")]
+          ("GMG_MG_FORCE_UNCERT", "1"), ("GMG_MG_FORCE_UNCERT", "3"), ("GMG_INDEP_FORCE_HOST", "1")]
 
 
 def seeded_reads(n, length, seed):
@@ -194,22 +190,16 @@ def test_distinct_gc_seeded(gm, ctx, gene, ogene, flags, with_qual):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("var,val", ROUTES, ids=[f"{k}={v}" for k, v in ROUTES])
-@pytest.mark.parametrize("flags,with_qual", ROUTE_CASES, ids=ROUTE_IDS)
+@pytest.mark.parametrize("flags,with_qual", ORACLE_CASES, ids=ORACLE_IDS)
 def test_routes(gm, ctx, gene, ogene, golden, monkeypatch, var, val, flags, with_qual):
+    """every route in every mode, with and without a quality file (-i without one: the qualities K2 synthesises open
+    the gates)"""
     reads, qual = golden
     monkeypatch.setenv(var, val)
     flagged = check_against_oracle(gm, ctx, gene, ogene, reads[:200], qual[:200], distinct_gc(200, 9), flags, with_qual, True)
     print(f"{var}={val}: {flagged} model entries recomputed on the host")
     if var == "GMG_INDEP_FORCE_HOST":
         assert flagged > 0
-
-
-@pytest.mark.gpu
-def test_k2_mode_one():
-    """GMG_K2_MODE is read once per process: run the check in a process of its own"""
-    r = subprocess.run([sys.executable, os.path.abspath(__file__), "k2mode"], cwd=ROOT, capture_output=True, text=True,
-                       env=dict(os.environ, GMG_K2_MODE="1"))
-    assert r.returncode == 0, r.stdout + r.stderr
 
 
 @pytest.mark.gpu
@@ -293,15 +283,3 @@ def test_rejected(gm, ctx, gene, golden, bad):
     p.c.ignore_score_len = 500
     assert n == ss.score_orfs_mg(gene, gm.ICM.Build_Indep_WO_Stops(ctx, 0.4), p)
     assert ss.get_starts()[0].tobytes() == got.tobytes()
-
-
-if __name__ == "__main__" and sys.argv[1:] == ["k2mode"]:
-    sys.path.insert(0, ROOT)
-    import glimmer_mg_b200 as g
-    c = g.Context(0)
-    reads, qual = golden_reads()
-    og = O.lib().orc_icm_read(os.path.join(G, "NC_000915.icm").encode())
-    gn = g.ICM.Read(c, os.path.join(G, "NC_000915.icm"))
-    for flags, with_qual in [({"allow_indels": 1}, True), ({"allow_subs": 1}, False), ({"allow_subs": 1}, True)]:
-        check_against_oracle(g, c, gn, og, reads[:200], qual[:200], distinct_gc(200, 9), flags, with_qual, True, n_api=50)
-    print("k2 mode 1 ok")
