@@ -16,7 +16,7 @@
 #define GMG_CTX_PAD 16384
 #define GMG_PAD_WORDS 8   // 64-bit words of zero padding before/after the packed bases
 #define GMG_NPROF 8
-#define GMG_NSCRATCH 20
+#define GMG_NSCRATCH 21
 #define GMG_PROF_RING 64
 
 void gmg_set_error(const char* fmt, ...);
@@ -189,7 +189,9 @@ enum { SCR_PLANES = 0, SCR_CUM = 1, SCR_TMP = 2, SCR_TMP2 = 3, SCR_FLAGS = 4, SC
        SCR_MISC = 15,
        // gmg_score_orfs_mg_gc: per-GC model records, the call's inputs (GC values, sequence -> record, ignore lengths),
        // the flagged-model list and the host's corrections
-       SCR_INDEP = 16, SCR_INDEP_IN = 17, SCR_INDEP_AUX = 18, SCR_INDEP_FIX = 19 };
+       SCR_INDEP = 16, SCR_INDEP_IN = 17, SCR_INDEP_AUX = 18, SCR_INDEP_FIX = 19,
+       // plain glimmer-mg on read sets: the partial-window gene values of every sequence (k1_partial_side)
+       SCR_SIDE = 20 };
 int gmg_scratch(gmg_ctx* ctx, int slot, size_t bytes, void** out);
 // ctx->h_stage holds at least `bytes` (grown to max(bytes, want)); its contents are not kept when it grows
 int gmg_host_stage(gmg_ctx* ctx, size_t bytes, size_t want);
@@ -241,6 +243,23 @@ __device__ __forceinline__ uint32_t gmg_plane_index(const uint64_t* __restrict__
   const uint64_t x = w ^ (0x5555555555555555ull * b);
   const uint64_t eq = ~(x | (x >> 1)) & 0x5555555555555555ull & ((1ull << (2 * i)) - 1ull);
   return __ldg(bktidx + ((p >> 5) << 2) + b) + (uint32_t)__popcll(eq);
+}
+
+// The walk-ready contexts of position p = 32 blk + i (the format of gmg_seqset::d_ctxf / d_ctxr) from the packed words of
+// blocks blk - 1, blk, blk + 1 (zero padding either side of the batch); q / e = distance of p to the first / last base of
+// its sequence.  k_bucket_finish stores them for K1, k1_partial_side forms them again for the partial windows of read sets.
+__device__ __forceinline__ void gmg_window_ctx(uint64_t wm, uint64_t w, uint64_t wp, int i, int64_t q, int64_t e,
+                                               uint32_t* cf, uint32_t* cr) {
+  // forward: bases p .. p+15, order reversed (base p in the top pair)
+  uint32_t f = (uint32_t)(i == 0 ? w : ((w >> (2 * i)) | (wp << (64 - 2 * i))));
+  f = __brev(f);
+  f = ((f >> 1) & 0x55555555u) | ((f & 0x55555555u) << 1);
+  // reverse: complement of bases p-15 .. p (base p-15 in the low pair)
+  const uint32_t r = ~(uint32_t)(i >= 15 ? (w >> (2 * (i - 15))) : ((wm >> (64 - 2 * (15 - i))) | (w << (2 * (15 - i)))));
+  // the low four bits (the two bases farthest from p; windows of up to 14 bases never see them) hold the distance to the
+  // end / start of the sequence, clipped to 15: which window positions exist
+  *cf = (f & ~15u) | (uint32_t)(e < 15 ? e : 15);
+  *cr = (r & ~15u) | (uint32_t)(q < 15 ? q : 15);
 }
 
 // reverse the order of the low W bases of v (base i <-> base W-1-i)

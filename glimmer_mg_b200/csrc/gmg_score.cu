@@ -305,19 +305,40 @@ __device__ __forceinline__ bool k1_step2_tested(uint32_t w, uint32_t c, unsigned
 
 // Partial windows, separately: the W-1 first positions of a sequence have a partial reverse-strand window and the W-1
 // last ones a partial forward window (icm.cc:807-842).  In bucket order nearly every warp of the bucketed kernel would
-// meet one and fall to its tested path, so for read sets that kernel walks EVERY window as if it were full and this
-// kernel then overwrites the 2 (W-1) x 3 partial entries of every sequence.  One thread per (sequence, end, offset): the
-// entry's walk-ready context is read back from the context array, its three walks (one per period) go through the same
-// merged words as the main kernel -- read from global memory, 13 KB that stay in L1 -- and stop at the first node that
-// branches on an unavailable position.
+// meet one and fall to its tested path, so for read sets that kernel walks EVERY window as if it were full and one of the
+// two kernels below then walks the 2 (W-1) x 3 partial entries of every sequence again.  Their walks (one per period) go
+// through the same merged words as the main kernel -- read from global memory, 13 KB that stay in L1 -- and stop at the
+// first node that branches on an unavailable position.
+//
+// The gene value of period f of the walk-ready context c (d_ctxf / d_ctxr format) whose predicted base is pb.
+__device__ __forceinline__ float k1_partial_walk(const DevIcmFast& gm, uint32_t c, unsigned pb, int f) {
+  constexpr int NWORDS = 4 + 64 + 1024;
+  constexpr uint32_t OFF7 = (16384 - 1) / 3;
+  const int W = gm.W;
+  const int lim = max(W - 1 - (int)(c & 15u), 0);  // first available window position
+  const unsigned lsh = 30 - 2 * lim;               // a node may be descended iff its shift <= this
+  const uint32_t cw = c >> (32 - 2 * W);
+  const uint32_t* __restrict__ mw = gm.mw + (size_t)f * NWORDS;
+  const unsigned s0 = f == 0 ? gm.s0[0] : (f == 1 ? gm.s0[1] : gm.s0[2]);
+  const bool stop0 = (f == 0 ? gm.stop0[0] : (f == 1 ? gm.stop0[1] : gm.stop0[2])) != 0;
+  uint32_t res = 0;
+  if (!(stop0 || s0 > lsh)) {
+    uint32_t i = (cw << s0) >> 30;
+    if (!k1_step2_tested(__ldg(mw + i), cw, lsh, 1, &i, &res))
+      if (!k1_step2_tested(__ldg(mw + 4 + i), cw, lsh, 21, &i, &res))
+        if (!k1_step2_tested(__ldg(mw + 68 + i), cw, lsh, 341, &i, &res)) res = OFF7 + i;
+  }
+  return __ldg(gm.bleaf + (size_t)(f * 4 + (int)pb) * gm.np + res);
+}
+
+// In place, for every consumer of complete planes: one thread per (sequence, end, offset), the entry's context read back
+// from the context array, the three values stored into the planes at the position's plane index.
 __global__ void __launch_bounds__(256) k1_partial_fix(DevIcmFast gm, const uint64_t* __restrict__ words,
                                                       const int64_t* __restrict__ off, int64_t n_seq,
                                                       const uint32_t* __restrict__ bktidx,
                                                       const uint32_t* __restrict__ ctxf, const uint32_t* __restrict__ ctxr,
                                                       int64_t total, float* __restrict__ planes) {
-  constexpr int NWORDS = 4 + 64 + 1024;
-  constexpr uint32_t OFF7 = (16384 - 1) / 3;
-  const int W = gm.W, per = 2 * (W - 1), wsh = 32 - 2 * W;
+  const int W = gm.W, per = 2 * (W - 1);
   const int64_t items = n_seq * per;
   for (int64_t it = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; it < items; it += (int64_t)gridDim.x * blockDim.x) {
     const int64_t sq = it / per;
@@ -335,30 +356,44 @@ __global__ void __launch_bounds__(256) k1_partial_fix(DevIcmFast gm, const uint6
     const uint32_t c = __ldg((rev ? ctxr : ctxf) + pi);
     if ((int)(c & 15u) >= W - 1) continue;  // a full window after all
     const unsigned own = (unsigned)gmg_base_at(words, p), pb = rev ? 3u - own : own;
-    const int lim = W - 1 - (int)(c & 15u);  // first available window position (>= 1 here)
-    const unsigned lsh = 30 - 2 * lim;      // a node may be descended iff its shift <= this
-    const uint32_t cw = c >> wsh;
 #pragma unroll
-    for (int f = 0; f < 3; f++) {
-      const uint32_t* __restrict__ mw = gm.mw + (size_t)f * NWORDS;
-      const unsigned s0 = f == 0 ? gm.s0[0] : (f == 1 ? gm.s0[1] : gm.s0[2]);
-      const bool stop0 = (f == 0 ? gm.stop0[0] : (f == 1 ? gm.stop0[1] : gm.stop0[2])) != 0;
-      uint32_t res = 0;
-      if (!(stop0 || s0 > lsh)) {
-        uint32_t i = (cw << s0) >> 30;
-        if (!k1_step2_tested(__ldg(mw + i), cw, lsh, 1, &i, &res))
-          if (!k1_step2_tested(__ldg(mw + 4 + i), cw, lsh, 21, &i, &res))
-            if (!k1_step2_tested(__ldg(mw + 68 + i), cw, lsh, 341, &i, &res)) res = OFF7 + i;
-      }
-      planes[(size_t)(rev ? 3 + f : f) * total + pi] = __ldg(gm.bleaf + (size_t)(f * 4 + (int)pb) * gm.np + res);
-    }
+    for (int f = 0; f < 3; f++) planes[(size_t)(rev ? 3 + f : f) * total + pi] = k1_partial_walk(gm, c, pb, f);
   }
 }
 
-// kAllFull: the main loop walks EVERY window as a full one (no test, no slow path); k1_partial_fix then redoes the entries
-// whose window is partial.  (Tried and measured slower, 0.85 against 0.62 ms per 31 Mbp of 100 bp reads: a second phase
-// inside this kernel that scans a bitmap of the partial plane indices and walks them from the shared-memory tables --
-// with 24 warps per SM its dependent bitmap -> context loads are pure latency, and the extra registers slow the main loop.)
+// Into a dense table, for the plain glimmer-mg pass (the only consumer on its path, see mgp_gene): side[sq][k][f] for
+// k < W-1 the reverse-strand value at q = k, for k >= W-1 the forward-strand value at q = L-1-(k-(W-1)); every entry
+// whose position exists is written.  One thread per (sequence, end, offset) as above, but the context is formed from the
+// sequence's packed words (consecutive threads read the same few words) and the bounds it already holds, and the stores
+// are dense: no bucket-index or context gather and no read-modify-write of plane sectors that have left L2.
+__global__ void __launch_bounds__(256) k1_partial_side(DevIcmFast gm, const uint64_t* __restrict__ words,
+                                                       const int64_t* __restrict__ off, int64_t n_seq,
+                                                       float* __restrict__ side) {
+  const int W = gm.W, per = 2 * (W - 1);
+  const int64_t items = n_seq * per;
+  for (int64_t it = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; it < items; it += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t sq = it / per;
+    const int k = (int)(it - sq * per);
+    const int64_t a = __ldg(off + sq);
+    const int L = (int)(__ldg(off + sq + 1) - a);
+    const bool rev = k < W - 1;
+    const int q = rev ? k : L - 1 - (k - (W - 1));
+    if (q < 0 || q >= L) continue;
+    const int64_t p = a + q, blk = p >> 5;
+    const uint64_t w = __ldg(words + blk);
+    uint32_t cf, cr;
+    gmg_window_ctx(__ldg(words + blk - 1), w, __ldg(words + blk + 1), (int)(p & 31), q, L - 1 - q, &cf, &cr);
+    const unsigned own = (unsigned)(w >> (2 * (p & 31))) & 3u, pb = rev ? 3u - own : own;
+#pragma unroll
+    for (int f = 0; f < 3; f++) side[it * 3 + f] = k1_partial_walk(gm, rev ? cr : cf, pb, f);
+  }
+}
+
+// kAllFull: the main loop walks EVERY window as a full one (no test, no slow path); k1_partial_fix or k1_partial_side
+// then walks the entries whose window is partial.  (Tried and measured slower, 0.85 against 0.62 ms per 31 Mbp of 100 bp
+// reads: a second phase inside this kernel that scans a bitmap of the partial plane indices and walks them from the
+// shared-memory tables -- with 24 warps per SM its dependent bitmap -> context loads are pure latency, and the extra
+// registers slow the main loop.)
 template <int kU, int NT = 1024, bool kAllFull = false>
 __global__ void __launch_bounds__(NT, 2) k1_planes_bucketed(DevIcmFast gm, const uint32_t* __restrict__ ctxf,
                                                               const uint32_t* __restrict__ ctxr, unsigned total,
@@ -470,13 +505,16 @@ __global__ void __launch_bounds__(NT, 2) k1_planes_bucketed(DevIcmFast gm, const
   }
 }
 
-static int launch_k1(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqset* s, float** planes_out) {
+// side_out: NULL -- the planes come out complete; else the caller reads partial-window values from *side_out where it is
+// not NULL (k1_partial_side's table, in the context's SCR_SIDE scratch) and the planes hold full-window walks there.
+static int launch_k1(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqset* s, float** planes_out, float** side_out) {
   GMG_CHECK(gene->P == 3, "six-frame scoring needs a periodicity-3 gene model (got %d)", gene->P);
   if (gmg_icm_ready(gene)) return 1;
   if (gmg_seqset_ensure_buckets(ctx, s)) return 1;
   void* planes = NULL;
   if (gmg_scratch(ctx, SCR_PLANES, (size_t)6 * (s->total + 32) * sizeof(float), &planes)) return 1;
   *planes_out = (float*)planes;
+  if (side_out) *side_out = NULL;
   if (s->total == 0) return 0;
   if (gene->fast.valid && gene->W <= 14) {
     if (!s->n_base_valid) {
@@ -504,9 +542,10 @@ static int launch_k1(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqset* s, float** p
     // Six walks in flight per thread, 384 threads per CTA: the six hide the shared-memory latency with a third of the
     // warps and pay the loop overhead once per six walks, and the 768 threads per SM leave room for the side-stream
     // kernels of gmg_score_orfs_g3 to run beside K1 (the other shapes measured took as long or longer, DESIGN.md 3.1).
-    // Read sets walk every window as full (no partial-window test in the hot loop) and k1_partial_fix redoes the
-    // 2 (W-1) x 3 partial entries of every sequence; on long sequences the test costs less than that second launch
-    // (5 Mbp contig: 71.6 against 78.9 us), so they keep the tested loop.  GMG_K1_FIX=0 (test hook): read sets too.
+    // Read sets walk every window as full (no partial-window test in the hot loop) and a second kernel walks the
+    // 2 (W-1) x 3 partial entries of every sequence: into a dense table for a caller that takes one (k1_partial_side), in
+    // place otherwise (k1_partial_fix).  On long sequences the test costs less than that second launch (5 Mbp contig: 71.6
+    // against 78.9 us), so they keep the tested loop.  GMG_K1_FIX=0 (test hook): read sets too.
     const bool long_seqs = s->total / (s->n > 0 ? s->n : 1) >= 4096;
     const char* fix_env = getenv("GMG_K1_FIX");
     const bool fix = !long_seqs && !(fix_env && atoi(fix_env) == 0);
@@ -520,8 +559,16 @@ static int launch_k1(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqset* s, float** p
     if (fix) {
       const int64_t items = s->n * 2 * (gene->W - 1);
       int64_t fg = (items + 255) / 256, fcap = (int64_t)ctx->sm_count * 16;
-      k1_partial_fix<<<(unsigned)(fg < fcap ? fg : fcap), 256, 0, ctx->stream>>>(
-          gene->fast, s->d_words, s->d_off, s->n, s->d_bktidx, s->d_ctxf, s->d_ctxr, s->total, (float*)planes);
+      const unsigned fgrid = (unsigned)(fg < fcap ? fg : fcap);
+      if (side_out) {
+        void* side = NULL;
+        if (gmg_scratch(ctx, SCR_SIDE, (size_t)items * 3 * sizeof(float), &side)) return 1;
+        *side_out = (float*)side;
+        k1_partial_side<<<fgrid, 256, 0, ctx->stream>>>(gene->fast, s->d_words, s->d_off, s->n, (float*)side);
+      } else {
+        k1_partial_fix<<<fgrid, 256, 0, ctx->stream>>>(gene->fast, s->d_words, s->d_off, s->n, s->d_bktidx, s->d_ctxf,
+                                                       s->d_ctxr, s->total, (float*)planes);
+      }
       ctx->launches++;
     }
     gmg_prof_end(ctx, GMG_PROF_K1);
@@ -548,7 +595,7 @@ static int launch_k1(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqset* s, float** p
 extern "C" int gmg_k1_score_planes(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqset* s) {
   GMG_CHECK(ctx && gene && s, "gmg_k1_score_planes: NULL argument");
   float* planes;
-  return launch_k1(ctx, gene, s, &planes);
+  return launch_k1(ctx, gene, s, &planes, NULL);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -582,7 +629,7 @@ extern "C" int gmg_score_all_frames(gmg_ctx* ctx, const gmg_icm* gene, const gmg
   GMG_CHECK(indep->P == 3, "independent model must have periodicity 3");
   if (gmg_icm_ready(indep)) return 1;
   float* planes;
-  if (launch_k1(ctx, gene, s, &planes)) return 1;
+  if (launch_k1(ctx, gene, s, &planes, NULL)) return 1;
   if (s->total == 0) return 0;
   double* d_fs = out;
   if (!out_on_device) {
@@ -2779,11 +2826,34 @@ static int exclusive_sum_u32(gmg_ctx* ctx, const uint32_t* d_in, uint32_t* d_out
 // FP64 addition can round; longer ORFs are accumulated by one lane in the reference's serial order.
 #define MGP_SLOTS 512  // codon-boundary prefixes per warp: sequences up to 3 * (MGP_SLOTS - 1) bases
 
+// Plain glimmer-mg on read sets: the partial-window table of k1_partial_side, [n_seq][2 (w - 1)][3], and the gene model's
+// window; t == NULL when the K1 planes are complete.
+struct PlainSide {
+  const float* t;
+  int w;
+};
+
+// The gene-model value of period f at position q of sequence S (index sq) on one strand.  With a partial-window table the
+// planes hold full-window walks where the strand's window is partial -- the W-1 first positions of the reverse strand,
+// the W-1 last of the forward strand -- and the value comes from the table there; from the planes everywhere else, at
+// plane index pidx() (evaluated only then).  (Measured on reads100: a select of the two addresses, one load for every
+// lane, makes k3_mg_plain_lanes spill and costs 0.55 ms against 0.53 for this branch.)
+template <class PlaneIdx>
+__device__ __forceinline__ float mgp_gene(const float* __restrict__ planes, const PlainSide& ps, const MgfBatch& B, const MgfSeq& S,
+                                          int32_t sq, bool fwd, int f, int q, PlaneIdx pidx) {
+  if (ps.t != NULL) {
+    const int wm1 = ps.w - 1;
+    const int k = fwd ? wm1 + (S.L - 1 - q) : q;  // the table's offset of (q, strand)
+    if (k < (fwd ? 2 * wm1 : wm1)) return __ldg(ps.t + ((size_t)sq * (size_t)(2 * wm1) + (size_t)k) * 3 + f);
+  }
+  return __ldg(planes + (size_t)(fwd ? f : 3 + f) * (size_t)B.total + pidx());
+}
+
 __device__ __forceinline__ void mgp_term(const DevIcm& indep, const float* __restrict__ s_lut, const float* __restrict__ planes,
-                                         const uint32_t* __restrict__ bktidx, const MgfBatch& B, const MgfSeq& S, bool fwd, int f,
-                                         int q, float* g_out, float* n_out) {
+                                         const PlainSide& ps, const uint32_t* __restrict__ bktidx, const MgfBatch& B, const MgfSeq& S,
+                                         int32_t sq, bool fwd, int f, int q, float* g_out, float* n_out) {
   const int64_t p = S.a + q;
-  *g_out = __ldg(planes + (size_t)(fwd ? f : 3 + f) * (size_t)B.total + gmg_plane_index(B.words, bktidx, p));
+  *g_out = mgp_gene(planes, ps, B, S, sq, fwd, f, q, [&]() { return gmg_plane_index(B.words, bktidx, p); });
   float n;
   if (indep.lut3 != NULL) {
     if (fwd) {
@@ -2838,7 +2908,7 @@ __global__ void __launch_bounds__(128) k3_mg_plain_count(MgfBatch B, DevParams P
 }
 
 template <bool kPS>
-__global__ void __launch_bounds__(128) k3_mg_plain(DevIcm indep_, IndepSeqs X, const float* __restrict__ planes,
+__global__ void __launch_bounds__(128) k3_mg_plain(DevIcm indep_, IndepSeqs X, const float* __restrict__ planes, PlainSide ps,
                                                    const uint32_t* __restrict__ bktidx, MgfBatch B, DevParams P_, CodonSets cs,
                                                    const gmg_orf* __restrict__ orfs, const int32_t* __restrict__ orf_seq,
                                                    int64_t n_orfs, const int64_t* __restrict__ start_off,
@@ -2855,7 +2925,8 @@ __global__ void __launch_bounds__(128) k3_mg_plain(DevIcm indep_, IndepSeqs X, c
   if (o >= n_orfs) return;  // warp-uniform
   const int64_t so = start_off[o];
   if (start_off[o + 1] == so) return;
-  const MgfSeq S = mgf_seq_of(B, orf_seq[o]);
+  const int32_t sq = orf_seq[o];
+  const MgfSeq S = mgf_seq_of(B, sq);
   // per-sequence models (gmg_score_orfs_mg_gc): the sequence's own table (read through L1) and ignore length
   DevIcm own;  // kPS: the sequence's own model; the single-model form reads the kernel parameter
   if constexpr (kPS) own = indep_of(indep_, X, orf_seq[o]);
@@ -2884,7 +2955,7 @@ __global__ void __launch_bounds__(128) k3_mg_plain(DevIcm indep_, IndepSeqs X, c
     double x = 0.0;
     if (j < need) {
       float g, n;
-      mgp_term(indep, s_lut, planes, bktidx, B, S, fwd, (1 + j) % 3, fwd ? hi - 1 - j : lo - 1 + j, &g, &n);
+      mgp_term(indep, s_lut, planes, ps, bktidx, B, S, sq, fwd, (1 + j) % 3, fwd ? hi - 1 - j : lo - 1 + j, &g, &n);
       k2_cert_term(g, umin, asum);
       k2_cert_term(n, umin, asum);
       x = (double)g - (double)n;
@@ -2913,7 +2984,7 @@ __global__ void __launch_bounds__(128) k3_mg_plain(DevIcm indep_, IndepSeqs X, c
       double run = 0.0;
       for (int j = 0; j < need; j++) {
         float g, n;
-        mgp_term(indep, s_lut, planes, bktidx, B, S, fwd, (1 + j) % 3, fwd ? hi - 1 - j : lo - 1 + j, &g, &n);
+        mgp_term(indep, s_lut, planes, ps, bktidx, B, S, sq, fwd, (1 + j) % 3, fwd ? hi - 1 - j : lo - 1 + j, &g, &n);
         run = run + ((double)g - (double)n);
         if ((j + 1) % 3 == 0) pref[(j + 1) / 3] = run;
       }
@@ -2952,9 +3023,9 @@ __device__ __forceinline__ int which4_of(const Which4& t, int cd) {
 // gene - indep of the three consecutive sequence positions q0, q0 + 1, q0 + 2 (one codon), summed in ascending order of
 // q, with the certificate inputs of the six floats.  per(i) = model period of position q0 + i.  One 64-bit window of the
 // packed bases serves the three independent-model codes and the three own bases; W == 3 independent models only.
-__device__ __forceinline__ double mgl_codon_sum(const DevIcm& indep, const float* __restrict__ planes,
-                                                const uint32_t* __restrict__ bktidx, const MgfBatch& B, const MgfSeq& S, bool fwd,
-                                                int q0, unsigned& umin, float& asum) {
+__device__ __forceinline__ double mgl_codon_sum(const DevIcm& indep, const float* __restrict__ planes, const PlainSide& ps,
+                                                const uint32_t* __restrict__ bktidx, const MgfBatch& B, const MgfSeq& S, int32_t sq,
+                                                bool fwd, int q0, unsigned& umin, float& asum) {
   const int64_t p0 = S.a + q0;
   const uint64_t v = gmg_extract32(B.words, p0 - 2);  // base q0 - 2 + m at bits 2 m
   const uint32_t pu = (uint32_t)p0;                   // batches hold fewer than 2^32 bases
@@ -2966,13 +3037,14 @@ __device__ __forceinline__ double mgl_codon_sum(const DevIcm& indep, const float
   for (int i = 0; i < 3; i++) {
     const int q = q0 + i;
     const int f = fwd ? (3 - i) % 3 : (1 + i) % 3;
-    const uint32_t p = pu + (uint32_t)i, blk = p >> 5, ib = p & 31u;
-    const uint64_t w = blk == blk0 ? w0 : w2;
-    const unsigned b = (unsigned)(v >> (2 * (i + 2))) & 3u;
-    const uint64_t y = w ^ (0x5555555555555555ull * b);
-    const uint64_t eq = ~(y | (y >> 1)) & 0x5555555555555555ull & ((1ull << (2 * ib)) - 1ull);
-    const uint32_t idx = __ldg(bktidx + (blk << 2) + b) + (uint32_t)__popcll(eq);
-    const float g = __ldg(planes + (size_t)(fwd ? f : 3 + f) * (size_t)B.total + idx);
+    const float g = mgp_gene(planes, ps, B, S, sq, fwd, f, q, [&]() {
+      const uint32_t p = pu + (uint32_t)i, blk = p >> 5, ib = p & 31u;
+      const uint64_t w = blk == blk0 ? w0 : w2;
+      const unsigned b = (unsigned)(v >> (2 * (i + 2))) & 3u;
+      const uint64_t y = w ^ (0x5555555555555555ull * b);
+      const uint64_t eq = ~(y | (y >> 1)) & 0x5555555555555555ull & ((1ull << (2 * ib)) - 1ull);
+      return __ldg(bktidx + (blk << 2) + b) + (uint32_t)__popcll(eq);
+    });
     float n;
     if (fwd) {
       const int raw = (int)(v >> (2 * (i + 2))) & 63;  // bases q, q+1, q+2
@@ -2997,7 +3069,7 @@ __device__ __forceinline__ double mgl_codon_sum(const DevIcm& indep, const float
 // on short reads (0.61 -> 0.49 ms per 31 Mbp with two; four per warp gave 0.50 -- the lane's serial share grows and its
 // prefix registers spill).
 template <int G, int K, bool kPS>
-__global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep_, const float* __restrict__ planes,
+__global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep_, const float* __restrict__ planes, PlainSide ps,
                                                          const uint32_t* __restrict__ bktidx, MgfBatch B, DevParams P, Which4 which,
                                                          int64_t n_orfs, const int64_t* __restrict__ start_off,
                                                          gmg_start* __restrict__ starts, int exact_len,
@@ -3017,21 +3089,25 @@ __global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep_, const
   int64_t o = (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * HPW + grp;
   int64_t nx_so = 0, nx_so1 = 0;
   uint4 nx_d0 = make_uint4(0u, 0u, 0u, 0u), nx_d1 = make_uint4(0u, 0u, 0u, 0u);
+  int32_t nx_sq = 0;  // the ORF's sequence: its row of the partial-window table, its model (kPS)
   if (o < n_orfs) {
     nx_so = __ldg(start_off + o);
     nx_so1 = __ldg(start_off + o + 1);
     nx_d0 = __ldg(reinterpret_cast<const uint4*>(desc + o));
     nx_d1 = __ldg(reinterpret_cast<const uint4*>(desc + o) + 1);
+    nx_sq = __ldg(X.orf_seq + o);
   }
   for (; o - grp < n_orfs; o += stride) {  // warp-uniform: o - grp is the warp's first ORF of this round
   const int64_t so = nx_so, so1 = nx_so1;
   const uint4 d0 = nx_d0, d1 = nx_d1;
+  const int32_t xs = nx_sq;
   const bool have = o < n_orfs;
   if (o + stride < n_orfs) {
     nx_so = __ldg(start_off + o + stride);
     nx_so1 = __ldg(start_off + o + stride + 1);
     nx_d0 = __ldg(reinterpret_cast<const uint4*>(desc + o + stride));
     nx_d1 = __ldg(reinterpret_cast<const uint4*>(desc + o + stride) + 1);
+    nx_sq = __ldg(X.orf_seq + o + stride);
   }
   MgfSeq S;
   S.a = (int64_t)d0.x;
@@ -3052,7 +3128,6 @@ __global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep_, const
   // this group's ORF is worked on here iff it has records and its length is this instance's
   const bool act = have && so1 != so && f.j_lo >= 3 && need > need_lo && need <= 3 * G * K;
   // per-sequence models (gmg_score_orfs_mg_gc): the ORF's own table and ignore length
-  const int32_t xs = kPS && have ? __ldg(X.orf_seq + o) : 0;
   DevIcm own;  // kPS: the sequence's own model; the single-model form reads the kernel parameter
   if constexpr (kPS) own = indep_of(indep_, X, xs);
   const DevIcm& indep = kPS ? own : indep_;
@@ -3081,13 +3156,13 @@ __global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep_, const
       double x = 0.0;
       if (c < ncod) {
         if (indep.lut3 != NULL) {  // j = 3 c .. 3 c + 2: positions hi-1-3c-2 .. hi-1-3c (forward), lo-1+3c .. +2 (reverse)
-          x = mgl_codon_sum(indep, planes, bktidx, B, S, fwd, fwd ? hi - 3 - 3 * c : lo - 1 + 3 * c, umin, asum);
+          x = mgl_codon_sum(indep, planes, ps, bktidx, B, S, xs, fwd, fwd ? hi - 3 - 3 * c : lo - 1 + 3 * c, umin, asum);
         } else {
 #pragma unroll
           for (int t = 0; t < 3; t++) {
             const int j = 3 * c + t;
             float g, n;
-            mgp_term(indep, s_lut, planes, bktidx, B, S, fwd, (1 + t) % 3, fwd ? hi - 1 - j : lo - 1 + j, &g, &n);
+            mgp_term(indep, s_lut, planes, ps, bktidx, B, S, xs, fwd, (1 + t) % 3, fwd ? hi - 1 - j : lo - 1 + j, &g, &n);
             k2_cert_term(g, umin, asum);
             k2_cert_term(n, umin, asum);
             x = x + ((double)g - (double)n);
@@ -3117,7 +3192,7 @@ __global__ void __launch_bounds__(128, 8) k3_mg_plain_lanes(DevIcm indep_, const
     double run = 0.0;
     for (int j = 0; j < need; j++) {
       float g, n;
-      mgp_term(indep, s_lut, planes, bktidx, B, S, fwd, (1 + j) % 3, fwd ? hi - 1 - j : lo - 1 + j, &g, &n);
+      mgp_term(indep, s_lut, planes, ps, bktidx, B, S, xs, fwd, (1 + j) % 3, fwd ? hi - 1 - j : lo - 1 + j, &g, &n);
       run = run + ((double)g - (double)n);
       if ((j + 1) % 3 == 0) s_serial[wid][grp][j / 3] = run;
     }
@@ -3528,7 +3603,7 @@ extern "C" int gmg_all_frame_scores(gmg_ctx* ctx, const gmg_icm* gene, gmg_seqse
               "outside its %lld bp sequence", (long long)i, h_lo[i], h_lo[i] + h_len[i], (long long)L);
   }
   float* planes;
-  if (launch_k1(ctx, gene, s, &planes)) return 1;
+  if (launch_k1(ctx, gene, s, &planes, NULL)) return 1;
   void* d_it;
   if (gmg_scratch(ctx, SCR_MISC, (size_t)n * (3 * sizeof(int32_t) + 6 * sizeof(double)) + 64, &d_it)) return 1;
   double* d_out = (double*)d_it;
@@ -3651,7 +3726,7 @@ extern "C" int gmg_score_orfs_g3(gmg_ctx* ctx, const gmg_icm* gene, const gmg_ic
   }
   GMG_CUDA(cudaEventRecord(ctx->ev_join, side));
 
-  if (launch_k1(ctx, gene, s, &planes)) return 1;
+  if (launch_k1(ctx, gene, s, &planes, NULL)) return 1;
   if (exact) {  // K2 (glimmer3 path): codon-boundary cumulative sums, tile by tile
     if (gmg_prof_begin(ctx, GMG_PROF_K2)) return 1;
     k2_g3_codon_cum<<<(unsigned)ntiles, G3_TS, 0, ctx->stream>>>(indep->dev.lut3, s->d_words, s->total, planes,
@@ -3719,7 +3794,13 @@ static int score_orfs_mg_plain(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& 
   GMG_CUDA(cudaMemcpyAsync(&ctx->h_scalars[6], s->d_start_off + s->n_orfs, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
   GMG_CUDA(cudaEventRecord(ctx->ev_scalars, ctx->stream));
   float* planes;
-  if (launch_k1(ctx, gene, s, &planes)) return 1;
+  float* side;
+  if (launch_k1(ctx, gene, s, &planes, &side)) return 1;
+  PlainSide ps;
+  ps.t = side;
+  ps.w = gene->W;
+  IndepSeqs Xo = X;  // the emission kernels find every ORF's sequence here, with either kind of independent model
+  Xo.orf_seq = s->d_orf_seq;
   // exactness is certified per ORF inside the kernel; the test hook withdraws every certificate
   const int exact_len = (getenv("GMG_MG_FORCE_UNCERT") && atoi(getenv("GMG_MG_FORCE_UNCERT")) > 0) ? -1 : INT_MAX;
   GMG_CUDA(cudaEventSynchronize(ctx->ev_scalars));
@@ -3744,7 +3825,7 @@ static int score_orfs_mg_plain(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& 
       auto launch_lanes = [&](auto kernel, int G) {
         const int64_t need_ctas = (s->n_orfs * G + 127) / 128;
         kernel<<<(unsigned)(need_ctas < lanes_cap ? need_ctas : lanes_cap), 128, 0, ctx->stream>>>(
-            indep, planes, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to, X);
+            indep, planes, ps, s->d_bktidx, B, dp, which, s->n_orfs, s->d_start_off, s->d_starts, exact_len, d_nord, geom, done_to, Xo);
         ctx->launches++;
         done_to = 3 * G * 4;
       };
@@ -3756,7 +3837,7 @@ static int score_orfs_mg_plain(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& 
     if (!all_taken) {
       const int slots = (int)(s->max_len / 3 + 4);
       k3_mg_plain<kPS><<<(unsigned)((s->n_orfs * 32 + 127) / 128), 128, (size_t)4 * slots * sizeof(double), ctx->stream>>>(
-          indep, X, planes, s->d_bktidx, B, dp, cs, s->d_orfs, s->d_orf_seq, s->n_orfs, s->d_start_off, s->d_starts, exact_len,
+          indep, X, planes, ps, s->d_bktidx, B, dp, cs, s->d_orfs, s->d_orf_seq, s->n_orfs, s->d_start_off, s->d_starts, exact_len,
           (unsigned long long*)(counts + s->n_orfs + 1), slots, plain_lanes);
       ctx->launches++;
     }
@@ -3776,7 +3857,7 @@ static int score_orfs_mg_k2k3(gmg_ctx* ctx, const gmg_icm* gene, const DevIcm& i
                               const gmg_params* p, const CodonSets& cs, const DevParams& dp, int k3mg_mode,
                               int64_t* n_starts) {
   float* planes;
-  if (launch_k1(ctx, gene, s, &planes)) return 1;
+  if (launch_k1(ctx, gene, s, &planes, NULL)) return 1;
   // K2
   void *d_cum, *d_tab, *d_qual, *d_cert;
   if (gmg_scratch(ctx, SCR_CUM, (size_t)6 * s->total * sizeof(double), &d_cum)) return 1;

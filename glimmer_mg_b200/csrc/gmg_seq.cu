@@ -213,14 +213,6 @@ __global__ void __launch_bounds__(256) k_bucket_finish(const uint64_t* __restric
     const uint64_t eq = ~(x | (x >> 1)) & 0x5555555555555555ull & ((1ull << (2 * i)) - 1ull);
     const unsigned first = b == 0 ? pre.x : (b == 1 ? pre.y : (b == 2 ? pre.z : pre.w));
     const unsigned idx = first + (unsigned)__popcll(eq);
-    // forward: bases p .. p+15, order reversed (base p in the top pair)
-    uint32_t f = (uint32_t)(i == 0 ? w : ((w >> (2 * i)) | (wp << (64 - 2 * i))));
-    f = __brev(f);
-    f = ((f >> 1) & 0x55555555u) | ((f & 0x55555555u) << 1);
-    // reverse: complement of bases p-15 .. p (base p-15 in the low pair)
-    const uint32_t r = ~(uint32_t)(i >= 15 ? (w >> (2 * (i - 15))) : ((wm >> (64 - 2 * (15 - i))) | (w << (2 * (15 - i)))));
-    // the low four bits (the two bases farthest from p; windows of up to 14 bases never see them) hold the distance
-    // to the end / start of the sequence, clipped to 15: which window positions exist
     int64_t a, nx;
     if (staged) {
       int kb = s_blk[bt];
@@ -233,9 +225,10 @@ __global__ void __launch_bounds__(256) k_bucket_finish(const uint64_t* __restric
       while (p >= nx) nx = __ldg(off + (++sq) + 1);
       a = __ldg(off + sq);
     }
-    const int64_t q = p - a, e = nx - 1 - p;
-    ctxf[idx] = (f & ~15u) | (uint32_t)(e < 15 ? e : 15);
-    ctxr[idx] = (r & ~15u) | (uint32_t)(q < 15 ? q : 15);
+    uint32_t cf, cr;
+    gmg_window_ctx(wm, w, wp, i, p - a, nx - 1 - p, &cf, &cr);
+    ctxf[idx] = cf;
+    ctxr[idx] = cr;
   }
 }
 
